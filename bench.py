@@ -15,6 +15,9 @@ rows per GPU and the cross-GPU synchronisation inside the kernel).
 value    : interactions/s with the epoch's batches already resident in HBM, device-timed (CUDA events around every
            step, L2 flushed between steps by writing a 512 MB buffer, outside the events), max over ranks.  One
            cooperative launch per step (wr_bprmf_step).
+--dump-outputs DIR: after the timed steps, the loss of the last timed step and the user / item embedding tables it left
+           (what a caller of train_step receives) are written as DIR/<name>.npy in float32.  The corpus, the initial
+           tables and the batches are seeded, so two builds run with the same arguments can be compared array by array.
 e2e      : the same through the reference-facing API with HOST batches -- model.train_step_host -> wr_bprmf_ctx_step:
            every step's ids start in ORDINARY (pageable) host memory, are collated into the context's pinned ring, pulled
            over PCIe by the resident training kernel, and the batch loss comes back through mapped host memory; the call
@@ -32,6 +35,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -42,7 +46,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 B, D, LR, L2 = 2048, 64, 1e-3, 1e-6
-CACHE = os.environ.get('WR_CACHE', '/tmp/wr_cache')
+CACHE = os.environ.get('WR_CACHE', os.path.join(tempfile.gettempdir(), 'wr_cache_%d' % os.getuid()))   # one per user
 TRAFFIC_FILE = os.path.join(ROOT, 'profiles', 'r02_kernel_traffic.json')   # ncu --set full: dram bytes per launch, by kernel + shape
 
 
@@ -76,6 +80,13 @@ def emit(line):
         sys.stdout.write(data.decode()); sys.stdout.flush()
     else:
         os.write(_STDOUT_FD, data)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array of `arrays` (name -> tensor) as <out_dir>/<name>.npy in float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), np.asarray(a.detach().cpu().numpy(), dtype=np.float32))
 
 
 def peaks():
@@ -260,6 +271,9 @@ def run_ours(a, rank, world, local_rank):
             step(a.warmup + s, ev[s])
         barrier()
         wall = time.perf_counter() - wall0
+        if a.dump_outputs:                                     # before the untimed steps below
+            last = {'loss': losses[a.warmup + a.steps - 1:].cpu(), 'user_embeddings': t.users(t.P).cpu(),
+                    'item_embeddings': t.items(t.P).cpu()}
         if wall < 1.5:                                         # keep the sampler alive long enough to see clocks
             t_end = time.perf_counter() + 1.5 - wall
             while time.perf_counter() < t_end:
@@ -385,6 +399,8 @@ def run_ours(a, rank, world, local_rank):
             except Exception as e:  # noqa: BLE001
                 line['extra']['torch_eager_b200'] = {'error': repr(e)}
     if rank == 0:
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, last)
         emit(line)
     if world > 1:
         import torch.distributed as dist
@@ -438,6 +454,9 @@ def run_ours_sharded(a, rank, world, local_rank):
             step(a.warmup + s, ev[s])
         barrier()
         wall = time.perf_counter() - wall0
+        if a.dump_outputs:                                     # before the untimed steps below; every rank takes part
+            gu, gi = st.gather_full()
+            last = {'loss': losses[a.warmup + a.steps - 1:].cpu(), 'user_embeddings': gu.cpu(), 'item_embeddings': gi.cpu()}
         extra_steps = int(max(0.0, 1.5 - wall) / 2e-4) if wall < 1.5 else 0
         t_extra = torch.tensor([extra_steps], device=dev)
         dist.all_reduce(t_extra, op=dist.ReduceOp.MAX)         # every rank runs the same number of steps
@@ -524,6 +543,8 @@ def run_ours_sharded(a, rank, world, local_rank):
     if not a.no_extras:
         line['extra'].update(extras_sharded(peers, dev, hbm_peak, flush))
     if rank == 0:
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, last)
         emit(line)
     peers.close()
     dist.destroy_process_group()
@@ -718,6 +739,8 @@ def run_reference(a, rank):
     for k in range(a.steps):
         d, loss = cpu_steps(U, I, cols, per_step, start=a.warmup * 5 + k * per_step)
         dt += d
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {'loss': torch.tensor([loss]), 'user_embeddings': U, 'item_embeddings': I})
     value = a.steps * per_step * B / dt
     sample = '%d batches of B=%d per step, model-only (batches pre-assembled), oracle port of the reference' % (per_step, B)
     emit({
@@ -999,6 +1022,8 @@ def main():
     ap.add_argument('--impl', type=str, default='ours', choices=['ours', 'reference'])
     ap.add_argument('--cpu-budget', type=float, default=12.0, dest='cpu_budget')
     ap.add_argument('--no-extras', action='store_true', dest='no_extras')
+    ap.add_argument('--dump-outputs', metavar='DIR', dest='dump_outputs', default=None,
+                    help='write the loss and the embedding tables of the last timed step as DIR/<name>.npy (float32)')
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3)
     rank, world = int(os.environ.get('RANK', 0)), int(os.environ.get('WORLD_SIZE', 1))

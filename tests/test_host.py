@@ -21,7 +21,11 @@ from whisprrec_b200.models.general.LightGCN import LightGCN, build_norm_adj_csr
 from whisprrec_b200.utils import utils
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DATA = '/root/reference/data/'
+# a checkout of the unmodified reference (HeyWeCome/WhisprRec, with data/ml-100k): the interchange tests run its code
+REFERENCE = os.environ.get('WHISPRREC_REFERENCE', '')
+REF_SRC, REF_DATA = os.path.join(REFERENCE, 'src'), os.path.join(REFERENCE, 'data') + os.sep
+needs_reference = pytest.mark.skipif(not REFERENCE or not os.path.exists(os.path.join(REF_SRC, 'models', 'general', 'BPRMF.py')),
+                                     reason='needs a checkout of the unmodified reference (set WHISPRREC_REFERENCE)')
 
 
 def test_library_exports_every_declared_symbol():
@@ -192,12 +196,38 @@ def test_history_csr_matches_oracle():
         assert set(hi[hp[u]:hp[u + 1]]) == corpus.train_clicked_set[u] | corpus.residual_clicked_set[u]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_DATA, 'ml-100k', 'ml-100k.inter')),
-                    reason='reference data only exists in the authoring container')
-def test_reader_reproduces_reference_split():
+def test_reader_reproduces_reference_split(tmp_path):
+    """The reader's filter, id remap and seeded 80/10/10 split reproduce the reference's ml-100k split
+    (tests/golden/ml100k_corpus.npz).  The input `.inter` is rebuilt from that split: its rows go back to file order by
+    inverting the two seeded shuffles, and raw ids are a seeded permutation of the codes, so only a remap by first
+    appearance gives the codes back.  Kept rows are rated 3 to 5 (3 is the floor).  Users left with fewer than 20 rows are
+    padded with ratings 1 and 2, which the reader counts for the user filter and then drops.  One more user has 19
+    above-floor rows and must be filtered out."""
+    from sklearn.model_selection import train_test_split
     c = load('ml100k_corpus.npz')
-    args = model_args(BPRMF, path=REF_DATA, dataset='ml-100k')
-    corpus = BaseReader(args)
+    parts = [np.stack([c[ph + '_user'], c[ph + '_item']], 1).astype(np.int64) for ph in ('train', 'dev', 'test')]
+    n = sum(len(p) for p in parts)
+    train_at, rest_at = train_test_split(np.arange(n), train_size=0.8, random_state=42, shuffle=True)
+    dev_at, test_at = train_test_split(rest_at, train_size=0.5, random_state=42, shuffle=True)
+    rows = np.empty((n, 2), dtype=np.int64)
+    for at, p in zip((train_at, dev_at, test_at), parts):
+        rows[at] = p
+    cnt = np.bincount(rows[:, 0])
+    short = np.nonzero(cnt < 20)[0]
+    assert len(short) > 0
+    pad = np.repeat(short, 20 - cnt[short])
+    rng = np.random.RandomState(5)
+    user_token = rng.permutation(int(c['n_users'])) + 1
+    item_token = rng.permutation(int(c['n_items'])) + 1
+    users = np.concatenate([user_token[rows[:, 0]], user_token[pad], np.full(19, 5000)])
+    items = np.concatenate([item_token[rows[:, 1]], np.full(len(pad) + 19, item_token[0])])
+    rating = np.concatenate([rng.randint(3, 6, n), rng.randint(1, 3, len(pad)), np.full(19, 5)])
+    assert (rating[:n] == 3).any() and (rating[n:n + len(pad)] == 2).any()
+    inter = pd.DataFrame({'user_id:token': users, 'item_id:token': items, 'rating:float': rating,
+                          'timestamp:float': 874_724_710 + np.arange(len(users))})
+    os.makedirs(tmp_path / 'ml-100k')
+    inter.to_csv(tmp_path / 'ml-100k' / 'ml-100k.inter', sep='\t', index=False)
+    corpus = BaseReader(model_args(BPRMF, path=str(tmp_path), dataset='ml-100k'))
     assert int(corpus.n_users) == int(c['n_users']) == 943 and int(corpus.n_items) == int(c['n_items']) == 1574
     for ph in ('train', 'dev', 'test'):
         assert (corpus.data_df[ph]['user_id'].to_numpy() == c[ph + '_user']).all()
@@ -255,15 +285,17 @@ def test_spmm_plan_slices_tile_the_long_rows_exactly():
     assert _lib.SpmmPlan(rowptr, 64, 'cpu', threshold=10_000).ref() is None      # nothing to split
 
 
-def test_bench_reference_arm_prints_one_contract_line():
-    """`bench.py --impl reference` (the CPU arm the driver runs beside ours): exactly one JSON line on stdout with the
-    contract keys, nothing else there."""
+def test_bench_reference_arm_prints_one_contract_line(tmp_path):
+    """`bench.py --impl reference` (the CPU arm of the benchmark): exactly one JSON line on stdout with the contract
+    keys, nothing else there; --dump-outputs writes the last step's loss and tables as float32 .npy files."""
     import json
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dump = tmp_path / 'outputs'
     r = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--impl', 'reference', '--steps', '1',
-                        '--warmup', '3'], capture_output=True, text=True, timeout=900, cwd=root)
+                        '--warmup', '3', '--dump-outputs', str(dump)], capture_output=True, text=True, timeout=900,
+                       cwd=root)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, r.stdout[-2000:]
@@ -273,6 +305,20 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert d['cpu_baseline']['kind'] == 'port' and d['cpu_baseline']['cores'] >= 1
     assert d['e2e'] == {'value': d['value'], 'unit': d['unit'], 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}
     assert 'workload' in d['config']
+    out = {f: np.load(dump / f) for f in os.listdir(dump)}
+    assert sorted(out) == ['item_embeddings.npy', 'loss.npy', 'user_embeddings.npy']
+    assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in out.values())
+    assert out['loss.npy'].shape == (1,) and out['user_embeddings.npy'].shape == (6040, 64)
+    assert out['item_embeddings.npy'].shape == (3706, 64)
+    # the tables after the timed steps, not the seeded initial ones; Adam moves a parameter by about lr per step
+    import bench
+    from whisprrec_b200.utils import synthetic
+    U0, I0, _ = bench.cpu_problem(synthetic.ml1m_shaped_corpus(cache_dir=os.path.join(bench.CACHE, 'ref')))
+    n_steps = 3 * 5 + 1 * 100                          # warmup * 5 + steps * 100 batches (run_reference)
+    for got, init in ((out['user_embeddings.npy'], U0.numpy()), (out['item_embeddings.npy'], I0.numpy())):
+        moved = np.abs(got - init).max()
+        assert 0.1 * bench.LR < moved <= 2 * bench.LR * n_steps, moved
+    assert 0.0 < out['loss.npy'][0] < np.log(2.0)      # BPR starts at log 2 on these near-zero tables and falls
 
 
 @pytest.mark.parametrize('n,k', [(10, 3), (10, 10), (21, 6), (22, 6), (100, 90), (1000, 5), (100000, 7), (200000, 180000),
@@ -370,8 +416,18 @@ def test_corpus_cache_is_written_under_the_reference_class_path(tmp_path):
     assert back.train_clicked_set == corpus.train_clicked_set and back.residual_clicked_set == corpus.residual_clicked_set
     for ph in ('train', 'dev', 'test'):
         assert back.data_df[ph].equals(corpus.data_df[ph])
+    # a cache the reference wrote lacks `_csr_cache`, the one attribute only this package sets: the CSR views the
+    # kernels consume are rebuilt on demand from the splits
+    ref_like = BaseReader.__new__(BaseReader)
+    ref_like.__dict__.update({k: v for k, v in corpus.__dict__.items() if k != '_csr_cache'})
+    wr_main.save_corpus(ref_like, pkl)
+    back = wr_main.load_corpus(pkl)
+    assert type(back) is BaseReader and '_csr_cache' not in back.__dict__
+    for view in ('train_csr', 'history_csr'):
+        for a, b in zip(getattr(back, view)(), getattr(corpus, view)()):
+            assert a.dtype == b.dtype and (a == b).all(), view
 
-    class Theirs(object):                     # what the reference does: its own class, object.__new__ + __dict__
+    class Theirs(object):                    # what the reference does: its own class, object.__new__ + __dict__
         pass
 
     class U(pickle.Unpickler):
@@ -384,8 +440,7 @@ def test_corpus_cache_is_written_under_the_reference_class_path(tmp_path):
     assert type(theirs) is Theirs and theirs.n_items == corpus.n_items and len(theirs.data_df['train']) == len(corpus.data_df['train'])
 
 
-@pytest.mark.skipif(not os.path.exists('/root/reference/src/models/general/BPRMF.py'),
-                    reason='needs the reference checkout (authoring container only)')
+@needs_reference
 def test_our_corpus_cache_loads_in_the_reference(tmp_path):
     """The same file through the reference's own code path: `pickle.load` in a process that has the reference's `src/` on
     its path (main.py:57-59) yields the reference's BaseReader with our ids and splits."""
@@ -398,7 +453,7 @@ def test_our_corpus_cache_loads_in_the_reference(tmp_path):
     code = f"""
 import sys, pickle, numpy as np
 np.float_ = np.float64
-sys.path.insert(0, '/root/reference/src')
+sys.path.insert(0, {REF_SRC!r})
 from helpers.BaseReader import BaseReader
 with open("{pkl}", "rb") as f:
     c = pickle.load(f)
@@ -411,8 +466,7 @@ print(c.n_users, c.n_items, len(c.data_df['train']), len(c.train_clicked_set))
                                 str(len(corpus.train_clicked_set))]
 
 
-@pytest.mark.skipif(not os.path.exists('/root/reference/src/models/general/BPRMF.py'),
-                    reason='needs the reference checkout (authoring container only)')
+@needs_reference
 def test_checkpoints_interchange_with_the_reference(tmp_path):
     """SURVEY.md section 8 f-4: a `.pt` written by the reference's BaseModel.save_model loads into ours and the other way
     round -- same state_dict keys, shapes, dtype (reference models/BaseModel.py:48-59)."""
@@ -426,7 +480,7 @@ def test_checkpoints_interchange_with_the_reference(tmp_path):
     script = f'''
 import sys, types, numpy as np, torch
 np.float_ = np.float64
-sys.path.insert(0, "/root/reference/src")
+sys.path.insert(0, {REF_SRC!r})
 from models.general.BPRMF import BPRMF
 args = types.SimpleNamespace(device=torch.device("cpu"), model_path="", buffer=1, num_neg=1, test_all=1, embedding_size=64)
 corpus = types.SimpleNamespace(n_users={int(corpus.n_users)}, n_items={int(corpus.n_items)})
@@ -446,8 +500,7 @@ print("REF_SUM", float(m.user_embeddings.weight.double().sum()), float(m.item_em
     assert float(ours.item_embeddings.weight.double().sum()) == i_sum
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_DATA, 'ml-100k', 'ml-100k.inter')),
-                    reason='needs the reference checkout (authoring container only)')
+@needs_reference
 def test_reference_corpus_cache_loads_as_our_reader(tmp_path):
     """SURVEY.md section 8 f-4: a `BaseReader.pkl` cached by the reference (main.py:54-63) is picked up by `--regenerate 0`
     here: it unpickles as this package's reader and yields the same splits and CSR views."""
@@ -458,9 +511,9 @@ def test_reference_corpus_cache_loads_as_our_reader(tmp_path):
     script = f'''
 import sys, types, pickle, numpy as np
 np.float_ = np.float64
-sys.path.insert(0, "/root/reference/src")
+sys.path.insert(0, {REF_SRC!r})
 from helpers.BaseReader import BaseReader
-args = types.SimpleNamespace(sep="\\t", path="{REF_DATA}", dataset="ml-100k", sample="random")
+args = types.SimpleNamespace(sep="\\t", path={REF_DATA!r}, dataset="ml-100k", sample="random")
 with open("{pkl}", "wb") as f:
     pickle.dump(BaseReader(args), f)
 '''
