@@ -285,12 +285,12 @@ int wr_csr_spmm(const int64_t *rowptr, const int32_t *col, const float *val, int
  * scores_out: optional dense fp32 [R, n_items] copy of S, unmasked -- what full_predict returns; NULL on the
  *             fast path (the point of the fusion is not to write it).
  * precision 0: fp32 FMA chains over d = 0..D-1 for every score (target included), so comparisons are
- * consistent.  precision 1: bf16 operands on the tcgen05 tensor cores (TMA-fed, TMEM accumulators), fp32
- * accumulation; D in {64, 128}; ranks and, if asked for, the top-k lists come out of the same epilogue; needs
+ * consistent; D in {16, 32, 64, 128, 256}.  precision 1: bf16 operands on the tcgen05 tensor cores (TMA-fed, TMEM accumulators), fp32
+ * accumulation; D in {64, 128, 256}; ranks and, if asked for, the top-k lists come out of the same epilogue; needs
  * `scratch`; looser parity (operands are rounded to bf16, the target's own column is excluded from the count
  * explicitly).  precision 2: precision 0's RANKS, bit for bit, at tensor-core speed (k must be 0): every fp32 operand
  * is split into two bf16 terms and the tensor cores accumulate hi.hi + hi.lo + lo.hi (K = 3 D); a score farther than
- * eps_r = c_D ||a_r|| max_j ||b_j|| from the row's target (c_64 = 1.5e-4, c_128 = 2e-4: twice the worst-case sum of
+ * eps_r = c_D ||a_r|| max_j ||b_j|| from the row's target (c_64 = 1.5e-4, c_128 = 2e-4, c_256 = 3.1e-4: twice the worst-case sum of
  * the split residual 3.1 2^-16, the fp32 accumulation of 3 D products and the FMA chain's own rounding) decides the
  * comparison as precision 0 would, the pairs inside the band (~0.1 %) are re-scored with precision 0's FMA chain.
  * If the candidate list overflows (degenerate tables) WR_STATUS_EVAL_OVERFLOW is raised: rerun with precision 0.
@@ -302,7 +302,7 @@ int wr_eval_rank_topk(const float *Uemb, const float *Iemb, const int64_t *user,
 
 /* Bytes of 1024-byte-aligned device scratch wr_eval_rank_topk needs for `precision` (0 for precision 0): the bf16
  * copies of the gathered user rows and of the item table that the TMA descriptors point at (three bf16 terms per
- * element for precision 2, plus its candidate list). */
+ * element for precision 2 -- two for the user rows at D = 256 -- plus its candidate list). */
 size_t wr_eval_scratch_bytes(int64_t R, int64_t n_items, int D, int precision);
 
 /* wr_metrics: BaseRunner.evaluate_method (BaseRunner.py:76-88) from the ranks; float64 means.
@@ -559,6 +559,7 @@ int wr_csr_spmm_sharded(const int64_t *rowptr, const int32_t *col, const float *
  *                   if this shard owns it, else -1
  *   rank[r] = 1 + #{local j not in hist : score > target[r]}   =>   global rank = 1 + sum over shards (rank - 1)
  *   topk_idx: LOCAL indices (global item = local * world + shard).
+ * D and precision as for wr_eval_rank_topk: D in {16, 32, 64, 128, 256} for precision 0, {64, 128, 256} for 1 and 2.
  */
 int wr_eval_rank_topk_shard(const float *Urows, const float *Iemb, const int64_t *user, const int64_t *pos_local,
                             int64_t R, int64_t n_users, int64_t n_items_local, int D, const int64_t *hist_ptr,

@@ -502,8 +502,8 @@ def csr_spmm(rowptr, col, val, X, Y=None, add=None, zero_add=False, acc_in=None,
 
 
 def exact_tc_supported(D, k=0, scores=False):
-    """precision 2 (precision 0's ranks on the tensor cores) covers D in {64, 128}, ranks only."""
-    return D in (64, 128) and k == 0 and not scores
+    """precision 2 (precision 0's ranks on the tensor cores) covers D in {64, 128, 256}, ranks only."""
+    return D in (64, 128, 256) and k == 0 and not scores
 
 
 def eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k=0, precision=0, scores=False):
@@ -550,7 +550,7 @@ def _eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k, precision,
 
 
 METRIC_CUTOFFS_PER_CALL = 8       # wr_metrics takes up to 8 cut-offs per launch
-EVAL_DIMS = (16, 32, 64, 128)     # embedding sizes the full-ranking evaluation kernels are instantiated for
+EVAL_DIMS = (16, 32, 64, 128, 256)     # embedding sizes the full-ranking evaluation kernels are instantiated for
 
 
 def metrics(rank, ks, ws):

@@ -40,17 +40,31 @@ __device__ __forceinline__ void cp_async_wait() {
 
 // Thread (ty, tx) of the 16x16 grid owns rows ty+16i and columns tx+16j (i, j < 4): with a row pitch of D+4
 // floats the 128-bit shared loads of a quarter warp then fall into 8 distinct 4-bank groups (no conflicts).
+// Top-k at D = 256 would need 233,984 B of shared memory with a separate staging buffer S, over the 232,448 B a CTA
+// may have: there S takes the B buffer the FMA loop has just consumed (one more barrier per tile).
+template <int D, bool TOPK>
+struct EvalSmem {
+    static constexpr int LD = D + 4;
+    static constexpr bool S_IN_B = TOPK && D >= 256;
+    static constexpr size_t S_BYTES = TOPK && !S_IN_B ? (size_t)EV_TR * (EV_TI + 1) * 4 : 0;
+    static constexpr size_t BYTES = (size_t)(EV_TR * LD + 2 * EV_TI * LD) * 4 + 2 * EV_TR * 2 * 4 + EV_TR * 4 + S_BYTES +
+                                    (TOPK ? (size_t)EV_TR * EV_KMAX * 8 : 0);
+    static_assert(!S_IN_B || EV_TR * (EV_TI + 1) <= EV_TI * LD, "S fits in one B buffer");
+    static_assert(BYTES <= 227 * 1024, "shared memory budget");
+};
+
 template <int D, bool TOPK>
 __global__ void __launch_bounds__(256) eval_rank_kernel(EvalParams p) {
-    constexpr int LD = D + 4;
+    using SM = EvalSmem<D, TOPK>;
+    constexpr int LD = SM::LD;
     constexpr int D4 = D / 4;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float *As = reinterpret_cast<float *>(smem_raw);            // [EV_TR][LD]
     float *Bs = As + EV_TR * LD;                                 // [2][EV_TI][LD]
     uint32_t *mask = reinterpret_cast<uint32_t *>(Bs + 2 * EV_TI * LD);  // [2][EV_TR][2]
     float *st_s = reinterpret_cast<float *>(mask + 2 * EV_TR * 2);       // [EV_TR]
-    float *S = st_s + EV_TR;                                     // [EV_TR][EV_TI+1]     (TOPK only)
-    float *tkv = S + EV_TR * (EV_TI + 1);                        // [EV_TR][EV_KMAX]     (TOPK only)
+    float *S = st_s + EV_TR;                                     // [EV_TR][EV_TI+1]     (TOPK only; S_IN_B: per tile)
+    float *tkv = S + SM::S_BYTES / 4;                            // [EV_TR][EV_KMAX]     (TOPK only)
     int32_t *tki = reinterpret_cast<int32_t *>(tkv + EV_TR * EV_KMAX);
 
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4, lane = tid & 31, warp = tid >> 5;
@@ -179,6 +193,10 @@ __global__ void __launch_bounds__(256) eval_rank_kernel(EvalParams p) {
                     acc[i][j] = fmaf(a[i].w, b[j].w, acc[i][j]);
                 }
         }
+        if (SM::S_IN_B) {
+            __syncthreads();                                     // every thread is done reading Bt
+            S = Bs + buf * EV_TI * LD;
+        }
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
             const int rl = ty + 16 * i;
@@ -305,9 +323,7 @@ __global__ void __launch_bounds__(256) metrics_kernel(const int32_t *__restrict_
 
 template <int D, bool TOPK>
 static int launch_eval(EvalParams &p, cudaStream_t st, int row_tiles) {
-    constexpr int LD = D + 4;
-    size_t smem = (size_t)(EV_TR * LD + 2 * EV_TI * LD) * 4 + 2 * EV_TR * 2 * 4 + EV_TR * 4;
-    if (TOPK) smem += (size_t)EV_TR * (EV_TI + 1) * 4 + (size_t)EV_TR * EV_KMAX * 8;
+    const size_t smem = EvalSmem<D, TOPK>::BYTES;
     cudaError_t e = cudaFuncSetAttribute(eval_rank_kernel<D, TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem);
     if (e != cudaSuccess) return (int)e;
@@ -372,6 +388,7 @@ static int eval_rank_topk_impl(const float *Uemb, const float *Iemb, const int64
         case 32: WR_EVAL_CALL(32); break;
         case 64: WR_EVAL_CALL(64); break;
         case 128: WR_EVAL_CALL(128); break;
+        case 256: WR_EVAL_CALL(256); break;
         default: return WR_E_DIM;
     }
 #undef WR_EVAL_CALL

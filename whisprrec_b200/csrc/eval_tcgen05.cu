@@ -14,7 +14,8 @@
 // precision 1: operands are rounded to bf16 once per evaluation (pack kernels below); the target score is the fp32 FMA
 // chain over the same bf16-rounded operands.  Parity with the fp32 path is therefore "looser": see tests.
 // precision 2 ("exact"): every fp32 operand is split into two bf16 terms, a = hi + lo, and the tensor cores accumulate
-// hi.hi + hi.lo + lo.hi (K = 3 D: A' = [hi | hi | lo], B' = [hi | lo | hi]).  The result is within
+// hi.hi + hi.lo + lo.hi (K = 3 D: A' = [hi | hi | lo], B' = [hi | lo | hi]; at D = 256 only [hi | lo] of A' is stored and
+// resident, the MMAs of the middle K third read its hi blocks again).  The result is within
 // eps_r = c_D * ||a_r|| * max_j ||b_j|| of the fp32 FMA chain precision 0 computes (bound below), so a score farther than
 // eps_r from the row's target decides the comparison as precision 0 would; the few pairs inside the band go to a
 // candidate list and are re-scored with exactly precision 0's FMA chain (eval_recheck_kernel).  Ranks are therefore
@@ -231,12 +232,13 @@ __global__ void __launch_bounds__(256) pack_items_split_kernel(const float *__re
     if (lane == 0 && mx > 0.f) atomicMax(bmax_bits, __float_as_uint(mx));
 }
 
-// one warp per eval row: A'[r] = [hi | hi | lo]; target[r] = precision 0's FMA chain over the UNROUNDED fp32 rows;
-// anorm[r] = ||a_r||_2.  rows_gathered != 0: U holds one row per eval row (item-shard mode) and target is an input.
+// one warp per eval row: A'[r] = [hi | hi | lo] ([hi | lo] if a_hilo); target[r] = precision 0's FMA chain over the
+// UNROUNDED fp32 rows; anorm[r] = ||a_r||_2.  rows_gathered != 0: U holds one row per eval row (item-shard mode) and
+// target is an input.
 __global__ void __launch_bounds__(256) pack_users_split_kernel(const float *__restrict__ U, const float *__restrict__ I,
                                                                 const int64_t *user, const int64_t *pos, int64_t R,
                                                                 int64_t n_users, int64_t n_items, int D, int rows_gathered,
-                                                                __nv_bfloat16 *A, float *target, float *anorm,
+                                                                int a_hilo, __nv_bfloat16 *A, float *target, float *anorm,
                                                                 uint8_t *row_ok, WrWorkspace *ws) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -251,10 +253,14 @@ __global__ void __launch_bounds__(256) pack_users_split_kernel(const float *__re
             const float x = ok ? a[d] : 0.f;
             __nv_bfloat16 hi, lo;
             split_bf16(x, hi, lo);
-            __nv_bfloat16 *o = A + r * 3 * D;
+            __nv_bfloat16 *o = A + r * (a_hilo ? 2 : 3) * D;
             o[d] = hi;
-            o[D + d] = hi;
-            o[2 * D + d] = lo;
+            if (a_hilo) {
+                o[D + d] = lo;
+            } else {
+                o[D + d] = hi;
+                o[2 * D + d] = lo;
+            }
             ss = fmaf(x, x, ss);
         }
         ss = warp_sum(ss);
@@ -308,8 +314,16 @@ constexpr int TC_THREADS = (4 + TC_EPI_WARPS) * 32;
 
 // K = contraction length in bf16 elements (D for precision 1, 3 D for precision 2).  A (128 x K) is loaded once per CTA;
 // B travels through a ring of stages of SKB 64-element K blocks (32 KB each) of one 256-item tile: a whole tile per
-// stage for precision 1 (one barrier round per tile: 5 % faster at D = 128 than block-wise staging), one K block per
-// stage for precision 2, whose tiles (96 / 192 KB) would not fit twice.
+// stage for precision 1 (one barrier round per tile: 5 % faster at D = 128 than block-wise staging) as long as two such
+// stages fit, else half a tile (D = 256: two 64 KB stages beside the 64 KB of A); one K block per stage for precision 2,
+// whose tiles (96 / 192 / 384 KB) would not fit twice.
+// Precision 2 at D = 256: A' = [hi | hi | lo] would take 192 KB and leave no room for a ring, so only [hi | lo] (128 KB)
+// is resident (A_HILO) and the MMAs of K blocks KB/3 .. 2 KB/3 - 1 read the hi blocks again; two 32 KB B stages fit.
+__host__ __device__ constexpr bool exact_a_hilo(int D) { return D >= 256; }
+// K blocks per B stage: the whole tile if two stages of it fit in room_kblocks, else the largest power-of-two share
+__host__ __device__ constexpr int tc_stage_kblocks(int kb, int room_kblocks) {
+    return kb > 1 && room_kblocks < 2 * kb ? tc_stage_kblocks(kb / 2, room_kblocks) : kb;
+}
 constexpr int TC_CAND_BUF = 64;                        // candidate entries buffered per epilogue warp (precision 2)
 // MT = 128-row A tiles per CTA.  MT = 1 (default): 128 rows x 256-item tiles; MT = 2 (WR_TC_VARIANT=12): 256 rows x
 // 128-item tiles -- the same 32,768 scores and the same 512 TMEM columns per tile, but every B byte that leaves L2 feeds
@@ -317,18 +331,20 @@ constexpr int TC_CAND_BUF = 64;                        // candidate entries buff
 // holds the kernel at 36 % tensor-pipe activity at D = 64: it is not -- 43.3 ms against 43.2 ms at D = 64, 60.2 against
 // 59.6 at D = 128 (profiles/r02_eval_variants.txt).  ncu: 0.745 instructions issued per cycle per SM sub-partition, ALU
 // pipe 65 % busy: the epilogue's ~4.5 issue slots per score (2 for the count, the rest mask / cursor / loop overhead per
-// 32-column chunk) are the limiter at D = 64.
+// 32-column chunk) are the limiter at D = 64.  At D = 256 MT = 2 still fits (128 KB of A, two 32 KB half-tile stages).
 template <int K, int EXACT, int MT>
 struct TcCfg {
     static constexpr int BM = TC_BM * MT;                  // rows per CTA
     static constexpr int BN = MT == 2 ? 128 : TC_BN;       // items per tile
     static constexpr int KB = K / 64;                      // 64-element (128 B) K blocks
-    static constexpr int SKB = EXACT ? 1 : KB;             // K blocks per stage
+    static constexpr bool A_HILO = EXACT && exact_a_hilo(K / 3);
+    static constexpr int A_KB = A_HILO ? 2 * KB / 3 : KB;  // resident K blocks of A
     static constexpr int KBLOCK_BYTES = BN * 128;
-    static constexpr int STAGE_BYTES = SKB * KBLOCK_BYTES;
-    static constexpr int A_BYTES = BM * K * 2;
+    static constexpr int A_BYTES = BM * A_KB * 128;
     static constexpr int TAIL = 256 /*barriers*/ + 4 * TC_BM * 4 /*counts*/ + (EXACT ? TC_EPI_WARPS * TC_CAND_BUF * 8 : 0);
     static constexpr int ROOM = 227 * 1024 - 1024 - A_BYTES - TAIL - (MT == 1 && !EXACT ? 19 * 1024 : 0) /*top-k drain state*/;
+    static constexpr int SKB = EXACT ? 1 : tc_stage_kblocks(KB, ROOM / KBLOCK_BYTES);      // K blocks per stage
+    static constexpr int STAGE_BYTES = SKB * KBLOCK_BYTES;
     static constexpr int STAGES = ROOM / STAGE_BYTES > 6 ? 6 : ROOM / STAGE_BYTES;
     static_assert(STAGES >= 2, "the B ring needs two stages");
     static constexpr int SMEM = 1024 /*align slack*/ + A_BYTES + STAGES * STAGE_BYTES + TAIL;
@@ -432,6 +448,7 @@ __global__ void __launch_bounds__(TOPK == 2 ? TC_THREADS_DRAIN : TC_THREADS, 1)
 eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TcParams p) {
     using C = TcCfg<K, EXACT, MT>;
     static_assert(MT == 1 || TOPK == 0, "the top-k lists are laid out for 128 rows per CTA");
+    static_assert(TOPK != 1 || C::STAGES * C::STAGE_BYTES >= TC_BM * 4 * TC_KMAX * 8, "stripe lists fit in the B ring");
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     uint8_t *sA = smem;
@@ -491,9 +508,9 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             // ---------------- TMA producer ----------------
             mbar_expect_tx(a_full, C::A_BYTES);
 #pragma unroll
-            for (int kb = 0; kb < C::KB; ++kb)
+            for (int kb = 0; kb < C::A_KB; ++kb)
                 for (int mh = 0; mh < MT; ++mh)
-                    tma_load_2d(&tmA, a_full, sA + (mh * C::KB + kb) * (TC_BM * 128), kb * 64, (int)row0 + mh * TC_BM);
+                    tma_load_2d(&tmA, a_full, sA + (mh * C::A_KB + kb) * (TC_BM * 128), kb * 64, (int)row0 + mh * TC_BM);
             int it = 0;
             for (int t = t0; t < t1; ++t) {
 #pragma unroll 1
@@ -530,9 +547,11 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
                     for (int kb = 0; kb < C::SKB; ++kb) {
                         const uint64_t b0 = umma_desc_sw128(sB + stage * C::STAGE_BYTES + kb * C::KBLOCK_BYTES);
+                        // A_HILO: K blocks of the middle third (B's lo) pair with A's hi blocks, the last third with lo
+                        const int akb = C::A_HILO && kb0 + kb >= C::KB / 3 ? kb0 + kb - C::KB / 3 : kb0 + kb;
 #pragma unroll
                         for (int mh = 0; mh < MT; ++mh) {   // the two row halves share the B tile
-                            const uint64_t a0 = umma_desc_sw128(sA + (mh * C::KB + kb0 + kb) * (TC_BM * 128));
+                            const uint64_t a0 = umma_desc_sw128(sA + (mh * C::A_KB + akb) * (TC_BM * 128));
 #pragma unroll
                             for (int k = 0; k < 4; ++k)     // K = 16 bf16 = 32 B per instruction: +2 in the >>4 address field
                                 umma_bf16(d_tmem + mh * C::BN, a0 + 2 * k, b0 + 2 * k, idesc, (kb0 | kb | k) != 0);
@@ -1010,6 +1029,19 @@ static int launch_tc(const CUtensorMap &ma, const CUtensorMap &mb, TcParams &p, 
 
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// bf16 columns of the packed user rows: D (precision 1), 3 D = [hi | hi | lo] or, at D = 256, 2 D = [hi | lo] (precision 2)
+static inline int tc_a_cols(int D, bool exact) { return !exact ? D : exact_a_hilo(D) ? 2 * D : 3 * D; }
+
+// c_D of the precision-2 band: twice the worst-case sum of the dropped lo.lo term (3.1 2^-16), the fp32 accumulation of
+// 3 D products (3 D 2^-23) and precision 0's own FMA chain (D 2^-24), rounded up -- DESIGN.md section 4.3
+static inline float exact_band_c(int D) {
+    switch (D) {
+        case 64: return 1.5e-4f;        // 2 x 7.40e-5
+        case 128: return 2.0e-4f;       // 2 x 1.007e-4
+        default: return 3.1e-4f;        // D = 256: 2 x 1.542e-4
+    }
+}
+
 }  // namespace wr
 
 using namespace wr;
@@ -1031,7 +1063,8 @@ static void exact_blocking(int64_t R, int64_t n_items, int64_t *rows_per_block, 
 extern "C" size_t wr_eval_scratch_bytes(int64_t R, int64_t n_items, int D, int precision) {
     if ((precision != 1 && precision != 2) || R <= 0 || n_items <= 0 || D <= 0) return 0;
     const size_t k = precision == 2 ? 3 : 1;
-    size_t n = align_up((size_t)R * D * 2 * k, 1024) + align_up((size_t)n_items * D * 2 * k, 1024) + align_up((size_t)R, 1024) + 1024;
+    size_t n = align_up((size_t)R * tc_a_cols(D, precision == 2) * 2, 1024) + align_up((size_t)n_items * D * 2 * k, 1024) +
+               align_up((size_t)R, 1024) + 1024;
     if (precision == 2) {
         int64_t rb;
         unsigned long long cap;
@@ -1046,14 +1079,15 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
                     int64_t n_users, int64_t n_items, int D, const int64_t *hist_ptr, const int32_t *hist_idx,
                     int32_t *rank, float *target, const float *target_in, float *scores_out, int k, int32_t *topk_idx,
                     float *topk_val, void *scratch, WrWorkspace *ws, cudaStream_t st, int precision) {
-    if (D != 64 && D != 128) return WR_E_DIM;
+    if (D != 64 && D != 128 && D != 256) return WR_E_DIM;
     if (!scratch) return WR_E_NULL;
     if ((reinterpret_cast<uintptr_t>(scratch) & 1023u) != 0) return WR_E_ALIGN;
     const bool exact = precision == 2;
     const int K = exact ? 3 * D : D;
+    const int KA = tc_a_cols(D, exact);
     uint8_t *base = static_cast<uint8_t *>(scratch);
     __nv_bfloat16 *A = reinterpret_cast<__nv_bfloat16 *>(base);
-    base += align_up((size_t)R * K * 2, 1024);
+    base += align_up((size_t)R * KA * 2, 1024);
     __nv_bfloat16 *Bm = reinterpret_cast<__nv_bfloat16 *>(base);
     base += align_up((size_t)n_items * K * 2, 1024);
     uint8_t *row_ok = base;
@@ -1100,7 +1134,11 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
             fill_rank_kernel<<<(int)min((int64_t)kSMs * 4, (R + 255) / 256), 256, 0, st>>>(rank, R, 1);
             WR_CHECK_LAUNCH();
         }
-        return D == 64 ? launch_tc<64>(ma, mb, p, row_tiles, st) : launch_tc<128>(ma, mb, p, row_tiles, st);
+        switch (D) {
+            case 64: return launch_tc<64>(ma, mb, p, row_tiles, st);
+            case 128: return launch_tc<128>(ma, mb, p, row_tiles, st);
+            default: return launch_tc<256>(ma, mb, p, row_tiles, st);
+        }
     }
 
     // ---------------- precision 2 ----------------
@@ -1119,10 +1157,11 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
     pack_items_split_kernel<<<(int)min((int64_t)16 * kSMs, (n_items + 7) / 8), 256, 0, st>>>(Iemb, n_items, D, Bm, bmax_bits);
     WR_CHECK_LAUNCH();
     pack_users_split_kernel<<<(int)min((int64_t)16 * kSMs, (R + 7) / 8), 256, 0, st>>>(
-        Uemb, Iemb, user, pos, R, n_users, n_items, D, target_in ? 1 : 0, A, target, anorm, row_ok, ws);
+        Uemb, Iemb, user, pos, R, n_users, n_items, D, target_in ? 1 : 0, exact_a_hilo(D) ? 1 : 0, A, target, anorm, row_ok,
+        ws);
     WR_CHECK_LAUNCH();
     p.bmax = reinterpret_cast<const float *>(bmax_bits);
-    p.band_c = D == 64 ? 1.5e-4f : 2.0e-4f;
+    p.band_c = exact_band_c(D);
     p.cand = cand;
     p.cand_cnt = cand_cnt;
     p.cand_cap = cap;
@@ -1132,7 +1171,7 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
         TcParams q = p;
         q.user = user + r0; q.pos = pos + r0; q.R = rn; q.target = p.target + r0; q.row_ok = row_ok + r0; q.rank = rank + r0;
         q.anorm = anorm + r0;
-        rc = make_map(&ma, A + r0 * K, rn, K, TC_BM);
+        rc = make_map(&ma, A + r0 * KA, rn, KA, TC_BM);
         if (rc) return rc;
         const int row_tiles = (int)((rn + BMc - 1) / BMc);
         int splits = 1;
@@ -1147,7 +1186,11 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
         }
         e = cudaMemsetAsync(cand_cnt, 0, sizeof(unsigned long long), st);
         if (e != cudaSuccess) return (int)e;
-        rc = D == 64 ? launch_tc_v<192, 1, 0, 1, 1>(ma, mb, q, row_tiles, st) : launch_tc_v<384, 1, 0, 1, 1>(ma, mb, q, row_tiles, st);
+        switch (D) {
+            case 64: rc = launch_tc_v<192, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;
+            case 128: rc = launch_tc_v<384, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;
+            default: rc = launch_tc_v<768, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;       // A_HILO
+        }
         if (rc) return rc;
         eval_recheck_kernel<<<8 * kSMs, 256, 0, st>>>(cand, cand_cnt, cap, target_in ? Uemb + r0 * D : Uemb, q.user,
                                                        target_in ? 1 : 0, Iemb, D, q.target, q.rank);

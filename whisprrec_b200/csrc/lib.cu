@@ -8,7 +8,7 @@ extern "C" const char *wr_error_string(int code) {
         case WR_OK: return "ok";
         case WR_E_NULL: return "a required pointer is NULL";
         case WR_E_SIZE: return "negative or inconsistent size";
-        case WR_E_DIM: return "unsupported embedding size (needs D % 4 == 0; eval needs D in {16,32,64,128})";
+        case WR_E_DIM: return "unsupported embedding size (needs D % 4 == 0; eval needs D in {16,32,64,128,256})";
         case WR_E_TOPK: return "k outside [1, 32]";
         case WR_E_ALIGN: return "table pointer not 16-byte aligned";
         case WR_E_PRECISION: return "unknown or unavailable scoring precision";
