@@ -44,6 +44,8 @@ extern "C" {
 #define WR_STATUS_EVAL_OVERFLOW 4u      /* precision-2 evaluation: more score/target near-ties than the candidate list
                                            holds (degenerate tables, e.g. all rows equal); ranks are incomplete -- rerun
                                            with precision 0 */
+#define WR_STATUS_TOPK_OVERFLOW 8u      /* precision-2 top-k: a row had more list candidates than its segment holds; its
+                                           list is returned as topk_idx[r, 0] = -2 -- rerun those rows with precision 0 */
 #define WR_PEER_TIMEOUT_NS 20000000000ull
 
 int wr_version(void);
@@ -288,12 +290,18 @@ int wr_csr_spmm(const int64_t *rowptr, const int32_t *col, const float *val, int
  * consistent; D in {16, 32, 64, 128, 256}.  precision 1: bf16 operands on the tcgen05 tensor cores (TMA-fed, TMEM accumulators), fp32
  * accumulation; D in {64, 128, 256}; ranks and, if asked for, the top-k lists come out of the same epilogue; needs
  * `scratch`; looser parity (operands are rounded to bf16, the target's own column is excluded from the count
- * explicitly).  precision 2: precision 0's RANKS, bit for bit, at tensor-core speed (k must be 0): every fp32 operand
+ * explicitly).  precision 2: precision 0's RANKS, bit for bit, at tensor-core speed: every fp32 operand
  * is split into two bf16 terms and the tensor cores accumulate hi.hi + hi.lo + lo.hi (K = 3 D); a score farther than
  * eps_r = c_D ||a_r|| max_j ||b_j|| from the row's target (c_64 = 1.5e-4, c_128 = 2e-4, c_256 = 3.1e-4: twice the worst-case sum of
  * the split residual 3.1 2^-16, the fp32 accumulation of 3 D products and the FMA chain's own rounding) decides the
  * comparison as precision 0 would, the pairs inside the band (~0.1 %) are re-scored with precision 0's FMA chain.
  * If the candidate list overflows (degenerate tables) WR_STATUS_EVAL_OVERFLOW is raised: rerun with precision 0.
+ * precision 2 with k in [1, 32] (D in {64, 128, 256}, scores_out NULL): precision 0's top-k lists too -- the same ids and
+ * the same fp32 values in the same order.  The tensor-core scores pick a per-row candidate set that provably holds the
+ * exact top k (every item within 2 eps_r of the running k-th best), and eval_topk_select_kernel re-scores the candidates
+ * with precision 0's FMA chain.  `scratch` must then hold wr_eval_scratch_bytes_topk(..., k) bytes.  A row with more than
+ * 1,024 candidates is returned with topk_idx[r, 0] = -2 and WR_STATUS_TOPK_OVERFLOW raised: rerun those rows with
+ * precision 0 (wr_eval_rank_topk_shard with their target scores); their ranks are already exact.
  */
 int wr_eval_rank_topk(const float *Uemb, const float *Iemb, const int64_t *user, const int64_t *pos, int64_t R,
                       int64_t n_users, int64_t n_items, int D, const int64_t *hist_ptr, const int32_t *hist_idx,
@@ -304,6 +312,11 @@ int wr_eval_rank_topk(const float *Uemb, const float *Iemb, const int64_t *user,
  * copies of the gathered user rows and of the item table that the TMA descriptors point at (three bf16 terms per
  * element for precision 2 -- two for the user rows at D = 256 -- plus its candidate list). */
 size_t wr_eval_scratch_bytes(int64_t R, int64_t n_items, int D, int precision);
+
+/* The same for a call that also asks for top-k lists (k = 0: wr_eval_scratch_bytes).  Precision 2 adds a segment of
+ * 1,024 candidate item ids and a count per row of a row block (rows are evaluated in blocks of at most 262,144, so the
+ * segments stay <= 1 GB); precision 1 needs nothing more. */
+size_t wr_eval_scratch_bytes_topk(int64_t R, int64_t n_items, int D, int precision, int k);
 
 /* wr_metrics: BaseRunner.evaluate_method (BaseRunner.py:76-88) from the ranks; float64 means.
  *   hr[i] = mean(rank <= ks[i]);  ndcg[i] = mean((rank <= ks[i]) / log2(rank + 1))
@@ -560,6 +573,8 @@ int wr_csr_spmm_sharded(const int64_t *rowptr, const int32_t *col, const float *
  *   rank[r] = 1 + #{local j not in hist : score > target[r]}   =>   global rank = 1 + sum over shards (rank - 1)
  *   topk_idx: LOCAL indices (global item = local * world + shard).
  * D and precision as for wr_eval_rank_topk: D in {16, 32, 64, 128, 256} for precision 0, {64, 128, 256} for 1 and 2.
+ * Precision 2 with top-k works here as there (size `scratch` with wr_eval_scratch_bytes_topk over n_items_local; rows
+ * marked -2 are rerun with precision 0 on this shard).
  */
 int wr_eval_rank_topk_shard(const float *Urows, const float *Iemb, const int64_t *user, const int64_t *pos_local,
                             int64_t R, int64_t n_users, int64_t n_items_local, int D, const int64_t *hist_ptr,

@@ -54,6 +54,7 @@ SIGNATURES = {
     'wr_eval_rank_topk': (_int, [_p, _p, _p, _p, _i64, _i64, _i64, _int, _p, _p, _int, _int, _p, _p, _p, _p, _p, _p,
                                  _p, _p]),
     'wr_eval_scratch_bytes': (_sz, [_i64, _i64, _int, _int]),
+    'wr_eval_scratch_bytes_topk': (_sz, [_i64, _i64, _int, _int, _int]),
     'wr_metrics': (_int, [_p, _i64, _c.POINTER(_int), _int, _p, _p, _p]),
     'wr_gather_rows': (_int, [_p, _p, _i64, _int, _i64, _p, _p, _p]),
     'wr_scatter_add_rows': (_int, [_p, _p, _i64, _int, _i64, _p, _p, _p]),
@@ -162,6 +163,7 @@ class Workspace:
         lib = load()
         self.buf = torch.empty(lib.wr_workspace_bytes(), dtype=torch.uint8, device=device)
         check(lib.wr_workspace_init(self.buf.data_ptr(), stream_ptr()))
+        self.last_topk_fallback_rows = 0      # rows of the last precision-2 top-k call that were rerun at precision 0
 
     @property
     def ptr(self):
@@ -502,16 +504,54 @@ def csr_spmm(rowptr, col, val, X, Y=None, add=None, zero_add=False, acc_in=None,
 
 
 def exact_tc_supported(D, k=0, scores=False):
-    """precision 2 (precision 0's ranks on the tensor cores) covers D in {64, 128, 256}, ranks only."""
+    """The ranks-only predicate: precision 2 (precision 0's ranks on the tensor cores) covers D in {64, 128, 256} for
+    calls without top-k lists or a score dump.  Calls with lists: exact_tc_topk_supported."""
     return D in (64, 128, 256) and k == 0 and not scores
+
+
+def exact_tc_topk_supported(D, k, scores=False):
+    """precision 2 with top-k lists (precision 0's lists on the tensor cores): D in {64, 128, 256}, 1 <= k <= 32, no
+    score dump."""
+    return D in (64, 128, 256) and 1 <= k <= 32 and not scores
+
+
+def _exact_topk_fallback(out, U, gathered, Iemb, user, pos, n_users, hist_ptr, hist_idx, target, ws, k):
+    """Rows of a precision-2 top-k call whose candidate segment overflowed (topk_idx[r, 0] = -2): their lists again with
+    precision 0, on those rows only (item-shard mode with their targets); the ranks are exact already.  U: the user
+    table (gathered = False) or one row per eval row (gathered = True)."""
+    tki, tkv = out[-2], out[-1]
+    bad = (tki[:, 0] == -2).nonzero().flatten()
+    ws.last_topk_fallback_rows = bad.numel()
+    if bad.numel():
+        rows = U.index_select(0, bad) if gathered else gather_rows(U, user[bad].contiguous(), ws)
+        _, bi, bv = _eval_rank_topk_shard(rows.contiguous(), Iemb, user[bad].contiguous(), pos[bad].contiguous(),
+                                          n_users, hist_ptr, hist_idx, target[bad].contiguous(), ws, k, 0)
+        tki[bad] = bi
+        tkv[bad] = bv
 
 
 def eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k=0, precision=0, scores=False):
     """Returns (rank int32 [R], target fp32 [R], topk_idx int32 [R,k] | None, topk_val fp32 [R,k] | None,
     scores fp32 [R, n_items] | None).  precision: 0 fp32 FMA tiles; 1 bf16 tensor cores; 2 split-bf16 tensor cores +
     exact re-check (ranks identical to 0; if the candidate list overflows -- degenerate tables -- the call is repeated
-    with precision 0, which costs one synchronisation)."""
+    with precision 0, which costs one synchronisation).  Precision 2 with k in 1..32 gives precision 0's lists too: rows
+    whose list candidates overflow their segment are rerun alone at precision 0 (ws.last_topk_fallback_rows)."""
     R, D = user.numel(), Uemb.shape[1]
+    if precision == 2 and k > 0:
+        if not exact_tc_topk_supported(D, k, scores):
+            return _eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k, 0, scores)
+        out = _eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k, 2, False)
+        st = ws.status()
+        ws.last_topk_fallback_rows = 0
+        if st & 4:
+            out = _eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k, 0, False)
+            ws.last_topk_fallback_rows = R
+        elif st & 8:
+            _exact_topk_fallback(out[2:4], Uemb, False, Iemb, user, pos, Uemb.shape[0], hist_ptr, hist_idx, out[1], ws, k)
+        st &= ~12
+        if st:
+            ws.restore_status(st)
+        return out
     if precision == 2:
         if not exact_tc_supported(D, k, scores):
             precision = 0
@@ -535,7 +575,7 @@ def _eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k, precision,
     tki = torch.empty((R, k), dtype=I32, device=dev) if k > 0 else None
     tkv = torch.empty((R, k), dtype=F32, device=dev) if k > 0 else None
     sc = torch.empty((R, Iemb.shape[0]), dtype=F32, device=dev) if scores else None
-    nbytes = load().wr_eval_scratch_bytes(R, Iemb.shape[0], D, precision)
+    nbytes = load().wr_eval_scratch_bytes_topk(R, Iemb.shape[0], D, precision, k)
     scratch = None
     if nbytes:
         scratch = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
@@ -844,8 +884,24 @@ def rowdot(A, B, round_bf16=False):
 
 
 def eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k=0, precision=0):
-    """One item shard: returns (rank int32 [R] = 1 + local count, topk_idx LOCAL int32 [R,k] | None, topk_val | None)."""
+    """One item shard: returns (rank int32 [R] = 1 + local count, topk_idx LOCAL int32 [R,k] | None, topk_val | None).
+    Precision 2 with k as in eval_rank_topk."""
     R, D = user.numel(), Urows.shape[1]
+    if precision == 2 and k > 0:
+        if not exact_tc_topk_supported(D, k):
+            return _eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k, 0)
+        out = _eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k, 2)
+        st = ws.status()
+        ws.last_topk_fallback_rows = 0
+        if st & 4:
+            out = _eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k, 0)
+            ws.last_topk_fallback_rows = R
+        elif st & 8:
+            _exact_topk_fallback(out[1:3], Urows, True, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k)
+        st &= ~12
+        if st:
+            ws.restore_status(st)
+        return out
     if precision == 2:
         if not exact_tc_supported(D, k):
             precision = 0
@@ -867,7 +923,7 @@ def _eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_
     rank = torch.empty(R, dtype=I32, device=dev)
     tki = torch.empty((R, k), dtype=I32, device=dev) if k > 0 else None
     tkv = torch.empty((R, k), dtype=F32, device=dev) if k > 0 else None
-    nbytes = load().wr_eval_scratch_bytes(R, Iemb.shape[0], D, precision)
+    nbytes = load().wr_eval_scratch_bytes_topk(R, Iemb.shape[0], D, precision, k)
     scratch = None
     if nbytes:
         scratch = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)

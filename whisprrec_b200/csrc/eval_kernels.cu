@@ -358,7 +358,6 @@ static int eval_rank_topk_impl(const float *Uemb, const float *Iemb, const int64
     cudaStream_t st = (cudaStream_t)stream;
     const bool topk = topk_idx != nullptr;
     if (precision == 1 || precision == 2) {
-        if (precision == 2 && topk) return WR_E_TOPK;
         return wr_eval_rank_tc(Uemb, Iemb, user, pos, R, n_users, n_items, D, hist_ptr, hist_idx, rank, target,
                                target_in, scores_out, topk ? k : 0, topk_idx, topk_val, scratch, (WrWorkspace *)ws, st,
                                precision);

@@ -50,9 +50,12 @@ struct TcParams {
     unsigned long long *cand_cnt;
     unsigned long long cand_cap;
     uint32_t *status;           // WR_STATUS_EVAL_OVERFLOW when the list is full
+    int32_t *seg;               // top-k: [rows][TC_SEG_CAP] list candidates (item ids) per row
+    int32_t *seg_cnt;           // top-k: [rows] candidates appended (> TC_SEG_CAP: the segment overflowed)
 };
 
 constexpr int TC_KMAX = 32;
+constexpr int TC_SEG_CAP = 1024;        // list candidates kept per row (precision 2 with top-k)
 
 // ---------------------------------------------------------------------------------------------------------
 // PTX wrappers (sm_100a)
@@ -305,6 +308,82 @@ __global__ void __launch_bounds__(256) eval_recheck_kernel(const uint2 *__restri
     }
 }
 
+// ordering of candidates: higher value first, lower id first among equal values
+__device__ __forceinline__ bool top_worse(float v, int32_t id, float w, int32_t wid) {
+    return v < w || (v == w && id > wid);
+}
+
+// Precision 2 with top-k, one warp per row: the row's candidates (a superset of precision 0's top k, see the drain warps)
+// are re-scored with precision 0's FMA chain, one candidate per lane, and merged into a sorted list (lane = slot) by
+// (value desc, id asc), as eval_rank_kernel does.  Slots left empty are written as (-inf, -1), as precision 0 writes them.
+// A row whose segment overflowed gets topk_idx[r, 0] = -2 and WR_STATUS_TOPK_OVERFLOW: the caller reruns it.
+__global__ void __launch_bounds__(256) eval_topk_select_kernel(const int32_t *__restrict__ seg,
+                                                                const int32_t *__restrict__ seg_cnt, int64_t R,
+                                                                const float *__restrict__ U, const int64_t *user,
+                                                                int rows_gathered, const float *__restrict__ I, int D,
+                                                                int k, int32_t *topk_idx, float *topk_val, uint32_t *status) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    const uint32_t kmask = k >= 32 ? 0xffffffffu : ((1u << k) - 1u);
+    for (int64_t r = warp; r < R; r += nwarps) {
+        const int n = seg_cnt[r];
+        if (n > TC_SEG_CAP) {
+            if (lane < k) {
+                topk_val[r * k + lane] = -INFINITY;
+                topk_idx[r * k + lane] = lane == 0 ? -2 : -1;
+            }
+            if (lane == 0) atomicOr(status, WR_STATUS_TOPK_OVERFLOW);
+            continue;
+        }
+        const float *a = U + (rows_gathered ? r : user[r]) * D;
+        float tv = -INFINITY, tau = -INFINITY;          // slot value; empty slots are worse than any candidate
+        int32_t ti = INT32_MAX, taui = INT32_MAX;
+        for (int c0 = 0; c0 < n; c0 += 32) {
+            const int c = c0 + lane;
+            float s = -INFINITY;
+            int32_t id = INT32_MAX;
+            if (c < n) {
+                id = seg[r * TC_SEG_CAP + c];
+                const float *b = I + (int64_t)id * D;
+                s = 0.f;                                 // eval_kernels.cu: s = fmaf(a_d, b_d, s), d = 0 .. D-1
+                for (int d = 0; d < D; d += 4) {
+                    const float4 x = ldg4(a + d), y = ldg4(b + d);
+                    s = fmaf(x.x, y.x, s);
+                    s = fmaf(x.y, y.y, s);
+                    s = fmaf(x.z, y.z, s);
+                    s = fmaf(x.w, y.w, s);
+                }
+            }
+            uint32_t pend = __ballot_sync(0xffffffffu, c < n && top_worse(tau, taui, s, id));
+            while (pend) {
+                const int src = __ffs(pend) - 1;
+                pend &= pend - 1;
+                const float v = __shfl_sync(0xffffffffu, s, src);
+                const int32_t vid = __shfl_sync(0xffffffffu, id, src);
+                if (!top_worse(tau, taui, v, vid)) continue;
+                const int ins = __popc(__ballot_sync(0xffffffffu, !top_worse(tv, ti, v, vid)) & kmask);
+                const float up_v = __shfl_up_sync(0xffffffffu, tv, 1);
+                const int32_t up_i = __shfl_up_sync(0xffffffffu, ti, 1);
+                if (lane == ins) {
+                    tv = v;
+                    ti = vid;
+                } else if (lane > ins) {
+                    tv = up_v;
+                    ti = up_i;
+                }
+                tau = __shfl_sync(0xffffffffu, tv, k - 1);
+                taui = __shfl_sync(0xffffffffu, ti, k - 1);
+            }
+        }
+        if (lane < k) {
+            const bool empty = ti == INT32_MAX;
+            topk_val[r * k + lane] = empty ? -INFINITY : tv;
+            topk_idx[r * k + lane] = empty ? -1 : ti;
+        }
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // the scoring kernel
 // ---------------------------------------------------------------------------------------------------------
@@ -325,6 +404,11 @@ __host__ __device__ constexpr int tc_stage_kblocks(int kb, int room_kblocks) {
     return kb > 1 && room_kblocks < 2 * kb ? tc_stage_kblocks(kb / 2, room_kblocks) : kb;
 }
 constexpr int TC_CAND_BUF = 64;                        // candidate entries buffered per epilogue warp (precision 2)
+// top-k mode 2 (below): per-row rings in shared memory, drained by four extra warps
+constexpr int TC_RING = 16;                             // ring entries per row
+constexpr int TC_DRAIN_WARPS = 4;
+constexpr int TC_THREADS_DRAIN = TC_THREADS + TC_DRAIN_WARPS * 32;
+constexpr int TC_SMEM_DRAIN = TC_BM * TC_RING * 8 + TC_BM * 12 + 64;      // rings, head / tail / tau per row, counters
 // MT = 128-row A tiles per CTA.  MT = 1 (default): 128 rows x 256-item tiles; MT = 2 (WR_TC_VARIANT=12): 256 rows x
 // 128-item tiles -- the same 32,768 scores and the same 512 TMEM columns per tile, but every B byte that leaves L2 feeds
 // twice the rows.  Built to test whether the 6 TB/s of L2 reads (the item table is streamed once per 128 rows) is what
@@ -332,7 +416,10 @@ constexpr int TC_CAND_BUF = 64;                        // candidate entries buff
 // 59.6 at D = 128 (profiles/r02_eval_variants.txt).  ncu: 0.745 instructions issued per cycle per SM sub-partition, ALU
 // pipe 65 % busy: the epilogue's ~4.5 issue slots per score (2 for the count, the rest mask / cursor / loop overhead per
 // 32-column chunk) are the limiter at D = 64.  At D = 256 MT = 2 still fits (128 KB of A, two 32 KB half-tile stages).
-template <int K, int EXACT, int MT>
+// TOPK only matters for precision 2: its top-k instantiation takes the drain state out of the ring's room (D = 64: four
+// stages instead of five; D = 128 / 256 keep three / two), the ranks-only configurations are untouched.  Precision 1
+// reserves 19 KB for the drain state whether or not a call asks for lists.
+template <int K, int EXACT, int MT, int TOPK = 0>
 struct TcCfg {
     static constexpr int BM = TC_BM * MT;                  // rows per CTA
     static constexpr int BN = MT == 2 ? 128 : TC_BN;       // items per tile
@@ -342,7 +429,8 @@ struct TcCfg {
     static constexpr int KBLOCK_BYTES = BN * 128;
     static constexpr int A_BYTES = BM * A_KB * 128;
     static constexpr int TAIL = 256 /*barriers*/ + 4 * TC_BM * 4 /*counts*/ + (EXACT ? TC_EPI_WARPS * TC_CAND_BUF * 8 : 0);
-    static constexpr int ROOM = 227 * 1024 - 1024 - A_BYTES - TAIL - (MT == 1 && !EXACT ? 19 * 1024 : 0) /*top-k drain state*/;
+    static constexpr int ROOM = 227 * 1024 - 1024 - A_BYTES - TAIL - (MT == 1 && !EXACT ? 19 * 1024 : 0) /*top-k drain state*/
+                                - (EXACT && TOPK == 2 ? TC_SMEM_DRAIN : 0);
     static constexpr int SKB = EXACT ? 1 : tc_stage_kblocks(KB, ROOM / KBLOCK_BYTES);      // K blocks per stage
     static constexpr int STAGE_BYTES = SKB * KBLOCK_BYTES;
     static constexpr int STAGES = ROOM / STAGE_BYTES > 6 ? 6 : ROOM / STAGE_BYTES;
@@ -365,10 +453,6 @@ struct TopState {
     float bv[TC_TOPBUF];
     int32_t bi[TC_TOPBUF];
 };
-// ordering of candidates: higher value first, lower id first among equal values
-__device__ __forceinline__ bool top_worse(float v, int32_t id, float w, int32_t wid) {
-    return v < w || (v == w && id > wid);
-}
 __device__ __noinline__ void top_compact(TopState &t, int k, int &bcnt, float &tau, int &worst) {
     const int most = __reduce_max_sync(0xffffffffu, bcnt);
     for (int i = 0; i < most; ++i) {
@@ -402,14 +486,17 @@ __device__ __forceinline__ float fmax3(float a, float b, float c) {
     return d;
 }
 
+// Precision 2 with top-k: a score t_j can be in precision 0's top k only if t_j >= tau_final - 2 eps_r (DESIGN.md
+// section 4.3); tau only grows, so the test against the current tau keeps a superset.  eps here is c_D ||a_r|| max ||b||,
+// twice the bound on |t - s|; the 2.4e-7 |tau| term covers the rounding of the subtraction.  -inf stays -inf.
+__device__ __forceinline__ float exact_topk_floor(float tau, float eps) {
+    return tau - (2.f * eps + 2.4e-7f * fabsf(tau));
+}
+
 // Top-k mode 2: the epilogue warps only FILTER -- a score that reaches the row's current k-th best is pushed into the
 // row's ring in shared memory -- and four extra warps (one thread per row) drain the rings into per-row k-best
 // lists and publish the new threshold.  The epilogue never sorts, never compacts and never waits for another
 // epilogue warp's bookkeeping, and the threshold is per ROW (all 256 columns of a tile), not per 64-column stripe.
-constexpr int TC_RING = 16;                             // ring entries per row
-constexpr int TC_DRAIN_WARPS = 4;
-constexpr int TC_THREADS_DRAIN = TC_THREADS + TC_DRAIN_WARPS * 32;
-constexpr int TC_SMEM_DRAIN = TC_BM * TC_RING * 8 + TC_BM * 12 + 64;      // rings, head / tail / tau per row, counters
 
 __device__ __forceinline__ uint32_t lds_vol_u32(uint32_t a) {
     uint32_t v;
@@ -446,8 +533,9 @@ __device__ __forceinline__ void ring_push(const TopRings &rg, int row, float x, 
 template <int K, int VARIANT, int TOPK, int EXACT, int MT>
 __global__ void __launch_bounds__(TOPK == 2 ? TC_THREADS_DRAIN : TC_THREADS, 1)
 eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TcParams p) {
-    using C = TcCfg<K, EXACT, MT>;
+    using C = TcCfg<K, EXACT, MT, TOPK>;
     static_assert(MT == 1 || TOPK == 0, "the top-k lists are laid out for 128 rows per CTA");
+    static_assert(!EXACT || TOPK != 1, "precision 2 builds its lists with the drain warps");
     static_assert(TOPK != 1 || C::STAGES * C::STAGE_BYTES >= TC_BM * 4 * TC_KMAX * 8, "stripe lists fit in the B ring");
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -597,10 +685,12 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         float st_hi = st, st_lo = st;
         int ccount = 0;                                        // candidates buffered by this warp (warp-uniform)
         uint2 *cbuf = cand_s + (warp - 4) * TC_CAND_BUF;
+        float eps_top = 0.f;                                   // precision-2 top-k: |t - s| <= eps_top / 2 for every item
         if (EXACT && live) {
             const float eps = p.band_c * p.anorm[r] * p.bmax[0] + 2.4e-7f * fabsf(st);
             st_hi = st + eps;
             st_lo = st - eps;
+            if (TOPK == 2) eps_top = p.band_c * p.anorm[r] * p.bmax[0];
         }
         TopState top;
         const int top_trigger = p.top_trigger;      // fold the buffers once any lane holds more than this many
@@ -646,8 +736,10 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                             if ((m_top >> i) & 1u) v[i] = 0xff800000u;      // -inf; these columns are in m as well
                     }
                     // the row's threshold as the drain warps last published it (stale = lower = still correct).
-                    // ">=" lets ties through: the drainer decides them by item id
-                    const float tau_row = *reinterpret_cast<volatile float *>(rg.tau + rl);
+                    // ">=" lets ties through: the drainer decides them by item id.  Precision 2 lowers it by the
+                    // band (tau - 2 eps_r, rounded down): such scores may still be in precision 0's top k
+                    const float tau_pub = *reinterpret_cast<volatile float *>(rg.tau + rl);
+                    const float tau_row = EXACT ? exact_topk_floor(tau_pub, eps_top) : tau_pub;
 #pragma unroll
                     for (int g8 = 0; g8 < 32; g8 += 8) {
                         float mx = fmax3(__uint_as_float(v[g8]), __uint_as_float(v[g8 + 1]), __uint_as_float(v[g8 + 2]));
@@ -897,6 +989,16 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         int32_t wid = INT32_MAX;
         int wp = 0;
         uint32_t tail = 0;
+        // precision 2: the k-best list above is over the tensor-core scores; what is kept is the row's candidate
+        // segment -- every entry of the list and every score within the band of its k-th best on arrival
+        const int64_t row = row0 + r;
+        float e = 0.f;
+        int nseg = 0;
+        int32_t *segr = nullptr;
+        if (EXACT && row < p.R) {
+            e = p.band_c * p.anorm[row] * p.bmax[0];
+            segr = p.seg + row * TC_SEG_CAP;
+        }
         volatile uint32_t *vhead = rg.head + r;
         volatile int32_t *vid = rg.id + r * TC_RING;
         volatile float *vv = rg.v + r * TC_RING;
@@ -918,7 +1020,9 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 __threadfence_block();
                 ++tail;
                 *reinterpret_cast<volatile uint32_t *>(rg.tail + r) = tail;
+                bool keep = false;
                 if (top_worse(w, wid, x, id)) {         // beats the worst kept entry (ties: the lower id wins)
+                    keep = true;
                     lv[wp] = x;
                     li[wp] = id;
                     w = lv[0];
@@ -932,11 +1036,18 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                         }
                     }
                     *reinterpret_cast<volatile float *>(rg.tau + r) = w;
+                } else if (EXACT && e > 0.f && x >= exact_topk_floor(w, e)) {
+                    keep = true;                        // below the list but within 2 eps_r of its k-th best
+                }
+                if (EXACT && keep) {
+                    if (nseg < TC_SEG_CAP) segr[nseg] = id;
+                    ++nseg;
                 }
             }
         }
-        const int64_t row = row0 + r;
-        if (row < p.R) {
+        if (EXACT) {
+            if (row < p.R) p.seg_cnt[row] = nseg;
+        } else if (row < p.R) {
             for (int s = 0; s < k; ++s) {               // k selection passes: best first
                 int best = -1;
                 for (int j = 0; j < k; ++j) {
@@ -988,7 +1099,7 @@ static int make_map(CUtensorMap *map, const void *base, int64_t rows, int D /* b
 
 template <int K, int VARIANT, int TOPK, int EXACT, int MT>
 static int launch_tc_v(const CUtensorMap &ma, const CUtensorMap &mb, TcParams &p, int row_tiles, cudaStream_t st) {
-    constexpr int smem = TcCfg<K, EXACT, MT>::SMEM + (TOPK == 2 ? TC_SMEM_DRAIN : 0);
+    constexpr int smem = TcCfg<K, EXACT, MT, TOPK>::SMEM + (TOPK == 2 ? TC_SMEM_DRAIN : 0);
     constexpr int threads = TOPK == 2 ? TC_THREADS_DRAIN : TC_THREADS;
     static_assert(smem <= 227 * 1024, "shared memory budget");
     cudaError_t e = cudaFuncSetAttribute(eval_tc_rank_kernel<K, VARIANT, TOPK, EXACT, MT>,
@@ -1060,6 +1171,13 @@ static void exact_blocking(int64_t R, int64_t n_items, int64_t *rows_per_block, 
     *cand_cap = cap;
 }
 
+// precision 2 with top-k: the same blocks, at most 262,144 rows so that the candidate segments (4 KB per row) stay <= 1 GB
+static void exact_blocking_topk(int64_t R, int64_t n_items, int k, int64_t *rows_per_block, unsigned long long *cand_cap) {
+    exact_blocking(R, n_items, rows_per_block, cand_cap);
+    const int64_t most = ((int64_t)1 << 30) / ((int64_t)TC_SEG_CAP * 4);
+    if (k > 0 && *rows_per_block > most) *rows_per_block = most;
+}
+
 extern "C" size_t wr_eval_scratch_bytes(int64_t R, int64_t n_items, int D, int precision) {
     if ((precision != 1 && precision != 2) || R <= 0 || n_items <= 0 || D <= 0) return 0;
     const size_t k = precision == 2 ? 3 : 1;
@@ -1074,6 +1192,15 @@ extern "C" size_t wr_eval_scratch_bytes(int64_t R, int64_t n_items, int D, int p
     return n;
 }
 
+extern "C" size_t wr_eval_scratch_bytes_topk(int64_t R, int64_t n_items, int D, int precision, int k) {
+    const size_t n = wr_eval_scratch_bytes(R, n_items, D, precision);
+    if (precision != 2 || k <= 0 || n == 0) return n;
+    int64_t rb;
+    unsigned long long cap;
+    exact_blocking_topk(R, n_items, k, &rb, &cap);
+    return n + 1024 + align_up((size_t)rb * 4, 1024) + (size_t)rb * TC_SEG_CAP * 4;      // counts, then segments
+}
+
 // precision-1 / precision-2 body of wr_eval_rank_topk (eval_kernels.cu dispatches here)
 int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, const int64_t *pos, int64_t R,
                     int64_t n_users, int64_t n_items, int D, const int64_t *hist_ptr, const int32_t *hist_idx,
@@ -1083,6 +1210,7 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
     if (!scratch) return WR_E_NULL;
     if ((reinterpret_cast<uintptr_t>(scratch) & 1023u) != 0) return WR_E_ALIGN;
     const bool exact = precision == 2;
+    if (exact && scores_out) return WR_E_TOPK;          // no dense score dump at precision 2
     const int K = exact ? 3 * D : D;
     const int KA = tc_a_cols(D, exact);
     uint8_t *base = static_cast<uint8_t *>(scratch);
@@ -1142,7 +1270,6 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
     }
 
     // ---------------- precision 2 ----------------
-    if (topk_idx || scores_out) return WR_E_TOPK;
     float *anorm = reinterpret_cast<float *>(base);
     base += align_up((size_t)R * 4, 1024);
     uint32_t *bmax_bits = reinterpret_cast<uint32_t *>(base);
@@ -1151,7 +1278,11 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
     uint2 *cand = reinterpret_cast<uint2 *>(base);
     int64_t rb;
     unsigned long long cap;
-    exact_blocking(R, n_items, &rb, &cap);
+    exact_blocking_topk(R, n_items, topk_idx ? k : 0, &rb, &cap);
+    // top-k: per-row candidate counts and segments behind the list (wr_eval_scratch_bytes_topk)
+    const size_t seg_at = align_up((size_t)(base - static_cast<uint8_t *>(scratch)) + (size_t)cap * 8, 1024);
+    int32_t *seg_cnt = reinterpret_cast<int32_t *>(static_cast<uint8_t *>(scratch) + seg_at);
+    int32_t *seg = reinterpret_cast<int32_t *>(static_cast<uint8_t *>(scratch) + seg_at + align_up((size_t)rb * 4, 1024));
     cudaError_t e = cudaMemsetAsync(bmax_bits, 0, 64, st);
     if (e != cudaSuccess) return (int)e;
     pack_items_split_kernel<<<(int)min((int64_t)16 * kSMs, (n_items + 7) / 8), 256, 0, st>>>(Iemb, n_items, D, Bm, bmax_bits);
@@ -1171,11 +1302,17 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
         TcParams q = p;
         q.user = user + r0; q.pos = pos + r0; q.R = rn; q.target = p.target + r0; q.row_ok = row_ok + r0; q.rank = rank + r0;
         q.anorm = anorm + r0;
+        if (topk_idx) {
+            q.topk_idx = topk_idx + r0 * k;
+            q.topk_val = topk_val + r0 * k;
+            q.seg = seg;
+            q.seg_cnt = seg_cnt;
+        }
         rc = make_map(&ma, A + r0 * KA, rn, KA, TC_BM);
         if (rc) return rc;
         const int row_tiles = (int)((rn + BMc - 1) / BMc);
         int splits = 1;
-        if (row_tiles < kSMs) splits = (kSMs + row_tiles - 1) / row_tiles;
+        if (row_tiles < kSMs && !topk_idx) splits = (kSMs + row_tiles - 1) / row_tiles;     // lists: one CTA per row
         if (splits > q.n_tiles) splits = q.n_tiles;
         if (splits > 65535) splits = 65535;
         q.tiles_per_split = (q.n_tiles + splits - 1) / splits;
@@ -1186,15 +1323,29 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
         }
         e = cudaMemsetAsync(cand_cnt, 0, sizeof(unsigned long long), st);
         if (e != cudaSuccess) return (int)e;
-        switch (D) {
-            case 64: rc = launch_tc_v<192, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;
-            case 128: rc = launch_tc_v<384, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;
-            default: rc = launch_tc_v<768, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;       // A_HILO
+        if (topk_idx) {              // the ranks as below, plus the drain warps' candidate segments
+            switch (D) {
+                case 64: rc = launch_tc_v<192, 1, 2, 1, 1>(ma, mb, q, row_tiles, st); break;
+                case 128: rc = launch_tc_v<384, 1, 2, 1, 1>(ma, mb, q, row_tiles, st); break;
+                default: rc = launch_tc_v<768, 1, 2, 1, 1>(ma, mb, q, row_tiles, st); break;
+            }
+        } else {
+            switch (D) {
+                case 64: rc = launch_tc_v<192, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;
+                case 128: rc = launch_tc_v<384, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;
+                default: rc = launch_tc_v<768, 1, 0, 1, 1>(ma, mb, q, row_tiles, st); break;       // A_HILO
+            }
         }
         if (rc) return rc;
-        eval_recheck_kernel<<<8 * kSMs, 256, 0, st>>>(cand, cand_cnt, cap, target_in ? Uemb + r0 * D : Uemb, q.user,
-                                                       target_in ? 1 : 0, Iemb, D, q.target, q.rank);
+        const float *Ublk = target_in ? Uemb + r0 * D : Uemb;
+        eval_recheck_kernel<<<8 * kSMs, 256, 0, st>>>(cand, cand_cnt, cap, Ublk, q.user, target_in ? 1 : 0, Iemb, D,
+                                                       q.target, q.rank);
         WR_CHECK_LAUNCH();
+        if (topk_idx) {
+            eval_topk_select_kernel<<<(int)min((int64_t)16 * kSMs, (rn + 7) / 8), 256, 0, st>>>(
+                seg, seg_cnt, rn, Ublk, q.user, target_in ? 1 : 0, Iemb, D, k, q.topk_idx, q.topk_val, &ws->status);
+            WR_CHECK_LAUNCH();
+        }
     }
     return WR_OK;
 }

@@ -302,6 +302,16 @@ class BaseRunner(object):
                                   precision=self.eval_precision)
         return out
 
+    def recommend(self, dataset, k=None):
+        """Top-k recommendation lists for each row of `dataset`: (items int64 [n, k], scores float32 [n, k]) as host
+        NumPy arrays, best first, in the corpus's item codes.  The user's history is masked as in evaluation; rows with
+        fewer than k candidates are padded with (-1, -inf).  k defaults to max(self.topk).  At the default precision 2
+        the lists equal precision 0's.  On a sharded model every rank returns the same lists."""
+        k = max(self.topk) if k is None else int(k)
+        _, _, tki, tkv, _ = self.rank_topk(dataset, k=k)
+        dataset.model.tables.ws.raise_on_status()
+        return tki.to(torch.int64).cpu().numpy(), tkv.cpu().numpy()
+
     def evaluate(self, dataset, topks, metrics):
         """BaseRunner.py:210-216 -> {metric@k: float64}."""
         rank = self.rank_topk(dataset)[0]
