@@ -139,6 +139,12 @@ size_t wr_bprmf_epoch_scratch_bytes(int64_t N, int64_t batch);
  * [3] Adam phase done, [4] past grid barrier 2 (CTA 0), [5] descriptor seen by the poller, [6] ids staged (CTA 0),
  * [7] completion word written (streaming).  scripts/prof_resident.py prints the breakdown. */
 int wr_debug_epoch_trace(uint64_t *dev_trace, uint64_t *dev_cta_trace /* nullable: [step][CTA][4], both barriers of every CTA */);
+/* Profiling aid: with a DEVICE buffer of 8 x uint64 per CTA set here (NULL switches it off), every later one-GPU launch
+ * of the single-launch step (wr_bprmf_step on cache-sized tables, D <= 128) records %globaltimer stamps of thread 0 of every CTA:
+ * [0] entry, [1] ids landed, [2] rows landed, [3] REDs issued, [4] arrived at the grid barrier, [5] barrier passed,
+ * [6] Adam operands landed, [7] exit.  The buffer needs 8 x (CTAs of the launch) words (<= 8 x 2048).
+ * scripts/prof_step_phases.py prints the breakdown. */
+int wr_debug_step_trace(uint64_t *dev_trace);
 int wr_bprmf_epoch(float *P, float *M, float *V, float *G, const int64_t *ids, int64_t N, int64_t batch, int D,
                    int64_t n_users, int64_t n_items, float gamma, double lr, float l2, double beta1, double beta2,
                    float eps, int64_t adam_t0, float *losses, void *scratch, size_t scratch_bytes, void *ws,

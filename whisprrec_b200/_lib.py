@@ -35,6 +35,7 @@ SIGNATURES = {
                              _f32, _p, _p, _p, _p]),
     'wr_bprmf_epoch_scratch_bytes': (_sz, [_i64, _i64]),
     'wr_debug_epoch_trace': (_int, [_p, _p]),
+    'wr_debug_step_trace': (_int, [_p]),
     'wr_bprmf_epoch': (_int, [_p, _p, _p, _p, _p, _i64, _i64, _int, _i64, _i64, _f32, _f64, _f32, _f64, _f64, _f32, _i64,
                               _p, _p, _sz, _p, _p]),
     'wr_bprmf_step_host': (_int, [_p, _p, _p, _p, _p, _p, _p, _i64, _int, _i64, _i64, _f32, _f32, _f64, _f64, _f32,

@@ -26,6 +26,10 @@ struct WrWorkspace {
     uint32_t ep_fetched[16];                   // streaming: helper warps that have copied their piece of step s's ids, at
                                                // [(s - first) % 16]; cumulative per slot (helpers run < 16 steps apart)
     uint32_t ep_flag[WR_EP_MAX_GRID * 32];     // grid barrier: CTA c's arrival number at [32 c] (one 128-byte line each)
+    // ---- single-launch step (bprmf_step_kernel); never reset: both words only move forward ----
+    uint32_t st_gen;                           // grid barrier generation: launches so far
+    uint32_t st_pad[31];
+    uint32_t st_flag[WR_EP_MAX_GRID * 32];     // CTA c's arrival (generation + 1) at [32 c]
 };
 
 #define WR_CHECK_LAUNCH()                        \
@@ -164,6 +168,12 @@ __device__ __forceinline__ void adam_elem_nr(float &p, float &m, float &v, float
 __device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t *p) {
     uint32_t v;
     asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+
+__device__ __forceinline__ uint32_t ld_relaxed_gpu_u32(const uint32_t *p) {
+    uint32_t v;
+    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
     return v;
 }
 

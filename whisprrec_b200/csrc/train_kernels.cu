@@ -2,6 +2,7 @@
 // See include/whisprrec_b200.h for the reference lines each entry point replaces.
 #include <cmath>
 #include <cstring>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -409,10 +410,10 @@ __global__ void __launch_bounds__(256) scatter_add_rows_kernel(float *G, const i
 
 // ------------------------------------------------------------------------------------------------------
 // One launch for a whole BPRMF step (BaseRunner.py:196-199) when the tables are cache-sized and the step is
-// latency-bound rather than bandwidth-bound: every thread first issues the loads of its share of P / M / V
-// (they do not depend on the batch), then the grid does the BPR forward+backward (ids -> rows -> REDs into
-// G) while those loads are in flight, meets at a grid barrier (cooperative launch: all CTAs are resident),
-// and finishes with the Adam+L2 update of the elements it already holds -- G comes back as L2 hits.
+// latency-bound rather than bandwidth-bound: every warp first issues its ids, then the CTA pulls its spans of
+// P / M / V / G towards L2 (they do not depend on the batch), the grid does the BPR forward+backward (ids -> rows ->
+// REDs into G) while those streams are in flight, meets at a grid barrier (cooperative launch: all CTAs are
+// resident), and finishes with the Adam+L2 update of its spans, which come back as L2 hits.
 // ------------------------------------------------------------------------------------------------------
 // Cross-GPU synchronisation state of the single-launch step on row-sharded tables (world > 1).
 struct StepSync {
@@ -423,20 +424,73 @@ struct StepSync {
     uint32_t epoch;                 // the step number: 1, 2, 3, ... (the same on every rank)
 };
 
-template <int LPR, int VPL, class TABS>
-__global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, float4 *P, float4 *M, float4 *V, float4 *G,
+// wr_debug_step_trace: [CTA][8] %globaltimer stamps of thread 0 of every CTA, written by the TRACE instantiation only
+// (the production instantiation never names it).  Slots: 0 entry, 1 ids landed, 2 rows landed, 3 REDs issued,
+// 4 arrived (fence + arrival done), 5 barrier passed, 6 Adam operands landed, 7 exit.  Slots 1 / 2 / 6 are thread 0's
+// last batch group and last Adam iteration.
+__device__ uint64_t *g_step_trace;
+
+__device__ __forceinline__ void wait_for(int64_t x) { asm volatile("" ::"l"(x)); }
+__device__ __forceinline__ void wait_for(float4 x) { asm volatile("" ::"f"(x.x), "f"(x.y), "f"(x.z), "f"(x.w)); }
+
+// The stamp waits for `deps` (registers of loads that must have landed) before it reads the clock.
+template <bool TRACE, class... T>
+__device__ __forceinline__ void step_stamp(int slot, T... deps) {
+    if constexpr (TRACE) {
+        if (threadIdx.x == 0) {
+            (wait_for(deps), ...);
+            g_step_trace[8 * blockIdx.x + slot] = global_timer_ns();
+        }
+    }
+}
+
+// Wait until CTA `line`'s arrival word has reached `value` (wrap-safe); gives up after WR_PEER_TIMEOUT_NS so that a CTA
+// that never arrives cannot hang the GPU.
+__device__ __forceinline__ void wait_arrival(const uint32_t *line, uint32_t value, WrWorkspace *ws) {
+    uint64_t t0 = 0;
+    for (uint32_t spins = 1; (int32_t)(ld_acquire_u32(line) - value) < 0; ++spins) {
+        if ((spins & 1023u) == 0) {
+            const uint64_t now = global_timer_ns();
+            if (t0 == 0) t0 = now;
+            if (now - t0 > WR_PEER_TIMEOUT_NS) {
+                atomicOr(&ws->status, WR_STATUS_PEER_TIMEOUT);
+                break;
+            }
+        }
+    }
+}
+
+// One CTA per SM (launch_step_fused sizes blockDim so that every thread's Adam share is whole).
+template <int LPR, int VPL, class TABS, bool TRACE = false>
+__global__ void __launch_bounds__(1024, 1) bprmf_step_kernel(BprParamsT<TABS> p, float4 *P, float4 *M, float4 *V, float4 *G,
                                                              int64_t n4, AdamScalars s, const float *dev_scalars,
                                                              StepSync sy) {
     using RG = RowGroup<LPR, VPL>;
     constexpr int D = RG::D;
-    __shared__ float red[8];
+    __shared__ float red[32];
+    step_stamp<TRACE>(0);
+    // The grid barrier's generation: every CTA reads it before it arrives, CTA 0 advances it once it has passed, so
+    // arrival lines need no reset and a line left by an earlier launch (of any grid size) is simply older.
+    const uint32_t arrived = ld_relaxed_gpu_u32(&p.ws->st_gen) + 1u;
     if (dev_scalars) {
         s.step_size = __ldg(dev_scalars);
         s.bc2_sqrt = __ldg(dev_scalars + 1);
     }
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     const int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    // ---- phase 0: pull this CTA's spans of P / M / V towards L2 (one bulk prefetch per 4 KB span) ----
+    // The first batch group's ids go out before the table streams below: behind 10 MB of them in the DRAM queues they
+    // land microseconds later, and every gather waits for them.
+    const int lane = threadIdx.x & 31, sub = lane % LPR, grp = lane / LPR;
+    const int64_t warp = (int64_t)(threadIdx.x >> 5) * gridDim.x + blockIdx.x;
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    const int64_t first = warp * RG::GROUPS;
+    int64_t u = 0, i = 0, j = 0;
+    if (first + grp < p.B) {
+        u = p.user[first + grp];
+        i = p.pos[first + grp];
+        j = p.neg[first + grp];
+    }
+    // ---- phase 0: pull this CTA's spans of P / M / V / G towards L2 (one bulk prefetch per span) ----
     if (threadIdx.x < 4) {      // G too: the gradient REDs then meet lines that are already on their way
         const float4 *arr = threadIdx.x == 0 ? P : (threadIdx.x == 1 ? M : (threadIdx.x == 2 ? V : G));
         for (int64_t c = (int64_t)blockIdx.x * blockDim.x; c < n4; c += stride) {
@@ -458,21 +512,21 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
         __syncthreads();
     }
     // ---- phase 1: BPR forward + backward; consecutive interaction groups go to different CTAs ----
-    const int lane = threadIdx.x & 31, sub = lane % LPR, grp = lane / LPR;
-    const int64_t warp = (int64_t)(threadIdx.x >> 5) * gridDim.x + blockIdx.x;
-    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
     float local = 0.f;
-    for (int64_t base = warp * RG::GROUPS; base < p.B; base += nwarps * RG::GROUPS) {
+    for (int64_t base = first; base < p.B; base += nwarps * RG::GROUPS) {
         const int64_t b = base + grp;
         const bool valid = b < p.B;
-        int64_t u = 0, i = 0, j = 0;
-        if (valid) {
-            u = p.user[b];
-            i = p.pos[b];
-            j = p.neg[b];
+        if (base != first) {
+            u = i = j = 0;
+            if (valid) {
+                u = p.user[b];
+                i = p.pos[b];
+                j = p.neg[b];
+            }
         }
         const bool ok = valid && (uint64_t)u < (uint64_t)p.n_users && (uint64_t)i < (uint64_t)p.n_items &&
                         (uint64_t)j < (uint64_t)p.n_items;
+        step_stamp<TRACE>(1, j);                   // (the last of the three id loads)
         if (valid && !ok && sub == 0) atomicOr(&p.ws->status, WR_STATUS_INDEX_OUT_OF_RANGE);
         float4 ue[VPL], pe[VPL], ne[VPL];
         if (ok) {     // P is rewritten by phase 2 (and by the peers' Adam phases): coherent loads, not ld.global.nc
@@ -484,6 +538,7 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
             RG::zero(pe);
             RG::zero(ne);
         }
+        step_stamp<TRACE>(2, ne[VPL - 1]);         // (the last of the row loads)
         float sp = 0.f, sn = 0.f;
 #pragma unroll
         for (int v = 0; v < VPL; ++v) {
@@ -506,35 +561,29 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
             }
         }
     }
+    // block_sum's last __syncthreads follows every REDs of the CTA: thread 0's release below speaks for all of them
     const float bsum = block_sum(local, red);
-    if (threadIdx.x == 0) p.ws->partial[blockIdx.x] = bsum;
-    // ---- grid barrier (ticket[3] counts arrivals, ticket[4] departures; the last CTA to leave re-arms both).
-    //      Sharded: CTA 0 extends it across the GPUs -- once every local CTA has arrived (all of this GPU's REDs,
-    //      local and remote, are performed) it deposits the loss share with every peer, publishes this rank's
-    //      arrival, waits for every peer's, and only then opens the gate (ticket[5]) for the local CTAs. ----
-    __syncthreads();
+    step_stamp<TRACE>(3);
+    // ---- grid barrier: CTA c release-stores the generation + 1 into its own 128-byte line (after its REDs, and its
+    //      loss partial), thread t waits for lines t, t + blockDim, ...: no counter, no atomics.  (Small tables run
+    //      more CTAs than threads: (500 + 700) x 64 is 100 CTAs of 96.)  Sharded: only CTA 0 waits; once every
+    //      local CTA has arrived (all of this GPU's REDs, local and remote, are performed) it deposits the loss share
+    //      with every peer, publishes this rank's arrival, waits for every peer's, and only then opens the gate
+    //      (ticket[5]) for the local CTAs. ----
     if (threadIdx.x == 0) {
-        if (sy.world > 1) __threadfence_system(); else __threadfence();
-        atomicAdd(&p.ws->ticket[3], 1u);
-        if (sy.world == 1 || blockIdx.x == 0) {
-            uint64_t t0 = 0;
-            for (uint32_t spins = 1; ld_acquire_u32(&p.ws->ticket[3]) < gridDim.x; ++spins) {
-                if ((spins & 1023u) == 0) {          // a CTA that never arrives must not hang the GPU
-                    const uint64_t now = global_timer_ns();
-                    if (t0 == 0) t0 = now;
-                    if (now - t0 > WR_PEER_TIMEOUT_NS) {
-                        atomicOr(&p.ws->status, WR_STATUS_PEER_TIMEOUT);
-                        break;
-                    }
-                }
-            }
-            __threadfence();
-        }
+        p.ws->partial[blockIdx.x] = bsum;
+        if (sy.world > 1) __threadfence_system();
+        st_release_gpu(&p.ws->st_flag[32 * blockIdx.x], arrived);
+        step_stamp<TRACE>(4);
     }
-    float loss_sum = 0.f;
-    if (blockIdx.x == 0) {
+    if (sy.world == 1 || blockIdx.x == 0) {
+        for (int c = threadIdx.x; c < (int)gridDim.x; c += blockDim.x) wait_arrival(&p.ws->st_flag[32 * c], arrived, p.ws);
         __syncthreads();
+    }
+    if (blockIdx.x == 0) {
+        float loss_sum = 0.f;
         if (threadIdx.x < 32) {      // this GPU's loss share, summed in CTA order (deterministic)
+            if (threadIdx.x == 0) p.ws->st_gen = arrived;      // every CTA read the generation before it arrived
             float t = 0.f;
             for (int i = threadIdx.x; i < (int)gridDim.x; i += 32) t += __ldcg(&p.ws->partial[i]);
             loss_sum = warp_sum(t) / p.loss_div;
@@ -542,7 +591,7 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
         if (sy.world > 1) {
             // Arrival and loss share travel as ONE 8-byte word {epoch, loss bits} per peer (slots[g] read as uint64[world]):
             // no fence between a payload and its flag (a fence.sys behind a remote store is an NVLink round trip).  The
-            // word is a release: every local CTA fenced its REDs at system scope before the ticket this thread acquired.
+            // word is a release: every local CTA fenced its REDs at system scope before the line this CTA acquired.
             // One slot per sender suffices: a peer writes epoch e + 1 only after it has seen this rank's rows-final flag
             // of epoch e, which is published after the losses of epoch e were read.
             loss_sum = __shfl_sync(0xffffffffu, loss_sum, 0);
@@ -597,7 +646,8 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
             __threadfence();
         }
     }
-    __syncthreads();
+    if (sy.world > 1) __syncthreads();
+    step_stamp<TRACE>(5);
     // ---- phase 2: Adam + L2 over every element, gradient re-zeroed; two iterations of loads in flight ----
     // div_nr / sqrt_nr (<= 1 ulp from the IEEE forms): with the IEEE sequences this phase is issue-bound on cache-sized tables
     const float inv_bc2 = 1.0f / s.bc2_sqrt;
@@ -613,6 +663,7 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
             vb = V[i2];
             gb = __ldcg(G + i2);
         }
+        step_stamp<TRACE>(6, ga, gb);
         adam_elem_nr(pa.x, ma.x, va.x, ga.x, s, inv_bc2);
         adam_elem_nr(pa.y, ma.y, va.y, ga.y, s, inv_bc2);
         adam_elem_nr(pa.z, ma.z, va.z, ga.z, s, inv_bc2);
@@ -632,15 +683,14 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
             G[i2] = z;
         }
     }
-    const bool announce = sy.world > 1;
-    if (announce) __syncthreads();              // the departure below speaks for the whole CTA's stores
-    if (threadIdx.x == 0) {
-        if (announce) __threadfence();
-        const uint32_t t = atomicAdd(&p.ws->ticket[4], 1u);
-        if (t == gridDim.x - 1) {
-            p.ws->ticket[3] = 0;
-            p.ws->ticket[4] = 0;
-            if (sy.world > 1) {                 // this rank's rows of P are final: peers may gather them for step e+1
+    // Sharded: the last CTA to finish its Adam tells the peers that this rank's rows of P are final (they may gather
+    // them for step e + 1).  One GPU: nothing reads a departure, the next launch starts behind this one in stream order.
+    if (sy.world > 1) {
+        __syncthreads();                        // the departure below speaks for the whole CTA's stores
+        if (threadIdx.x == 0) {
+            __threadfence();
+            if (atomicAdd(&p.ws->ticket[4], 1u) == gridDim.x - 1) {
+                p.ws->ticket[4] = 0;
                 // ONE fence, then relaxed stores that travel side by side (a release store per peer waits for the
                 // previous peer's acknowledgement: world - 1 serialised NVLink round trips on the next step's critical path)
                 __threadfence_system();
@@ -650,6 +700,7 @@ __global__ void __launch_bounds__(256, 4) bprmf_step_kernel(BprParamsT<TABS> p, 
             }
         }
     }
+    step_stamp<TRACE>(7);
 }
 
 static inline int grid_for(int64_t work_items, int per_block, int max_blocks) {
@@ -966,7 +1017,8 @@ extern "C" int wr_adam_l2_sweep_marked(float *P, float *M, float *V, float *G, i
     return e == cudaSuccess ? WR_OK : (int)e;
 }
 
-// Largest grid of bprmf_step_kernel<...> that is resident at once on the current device (cached per instantiation).
+// Largest grid of bprmf_step_kernel<...>: one CTA per SM (up to 1,024 threads each), at most WR_EP_MAX_GRID arrival
+// lines (cached per instantiation).
 template <int LPR, int VPL, class TABS>
 static int step_max_grid(int *out) {
     static int cached = 0;
@@ -975,15 +1027,16 @@ static int step_max_grid(int *out) {
         cudaError_t e = cudaGetDevice(&dev);
         if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         if (e == cudaSuccess)
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bprmf_step_kernel<LPR, VPL, TABS>, 256, 0);
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bprmf_step_kernel<LPR, VPL, TABS>, 1024, 0);
         if (e != cudaSuccess) return (int)e;
-        cached = sms * per_sm;
-        if (cached > WR_MAX_PARTIAL_BLOCKS) cached = WR_MAX_PARTIAL_BLOCKS;
-        if (cached < 1) return (int)cudaErrorLaunchOutOfResources;
+        if (per_sm < 1) return (int)cudaErrorLaunchOutOfResources;
+        cached = sms < WR_EP_MAX_GRID ? sms : WR_EP_MAX_GRID;
     }
     *out = cached;
     return 0;
 }
+
+static bool g_step_trace_on = false;      // wr_debug_step_trace: one-GPU launches take the TRACE instantiation
 
 template <int LPR, int VPL, class TABS>
 static int launch_step_fused(BprParamsT<TABS> &bp, float *P, float *M, float *V, float *G, int64_t n4, AdamScalars &s,
@@ -991,14 +1044,18 @@ static int launch_step_fused(BprParamsT<TABS> &bp, float *P, float *M, float *V,
     int max_grid = 0;
     const int rc = step_max_grid<LPR, VPL, TABS>(&max_grid);
     if (rc) return rc;
-    // whole iterations for every CTA: the fewest passes the resident grid needs, then the smallest grid for them
-    const int64_t per_pass = (int64_t)max_grid * 256;
-    const int64_t passes = (n4 + per_pass - 1) / per_pass;
-    int grid = grid_for(n4, (int)(256 * passes), max_grid);
+    // Every thread updates `per` float4 of each array (even: the Adam loop keeps two in flight), as few as 1,024-thread
+    // CTAs on every SM allow; then the fewest threads per CTA (whole warps) and the fewest CTAs for that share.  The bench
+    // shape (155,936 float4 per array, 148 SMs): per = 2, 544 threads, 144 CTAs.
+    const int64_t per = 2 * ((n4 + 2048 * (int64_t)max_grid - 1) / (2048 * (int64_t)max_grid));
+    const int threads = (int)((n4 + max_grid * per - 1) / (max_grid * per) + 31) / 32 * 32;
+    const int grid = grid_for(n4, (int)(threads * per), max_grid);
     float4 *P4 = (float4 *)P, *M4 = (float4 *)M, *V4 = (float4 *)V, *G4 = (float4 *)G;
     void *args[] = {&bp, &P4, &M4, &V4, &G4, &n4, &s, &dev_scalars, &sy};
-    return (int)cudaLaunchCooperativeKernel((const void *)bprmf_step_kernel<LPR, VPL, TABS>, dim3(grid), dim3(256), args,
-                                            0, st);
+    const void *fn = (const void *)bprmf_step_kernel<LPR, VPL, TABS>;
+    if constexpr (std::is_same<TABS, LocalTabs>::value && VPL == 1)      // D <= 128 (D = 256 would spill with the stamps)
+        if (g_step_trace_on) fn = (const void *)bprmf_step_kernel<LPR, VPL, TABS, true>;
+    return (int)cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(threads), args, 0, st);
 }
 
 template <class TABS>
@@ -1076,6 +1133,13 @@ int wr_bprmf_step_impl(float *P, float *M, float *V, float *G, const int64_t *us
     StepSync sy{};
     sy.world = 1;
     return dispatch_step_fused(bp, D, P, M, V, G, n_elems >> 2, s, dev_scalars, sy, (cudaStream_t)stream);
+}
+
+extern "C" int wr_debug_step_trace(uint64_t *dev_trace) {
+    const cudaError_t e = cudaMemcpyToSymbol(g_step_trace, &dev_trace, sizeof(dev_trace));
+    if (e != cudaSuccess) return (int)e;
+    g_step_trace_on = dev_trace != nullptr;
+    return WR_OK;
 }
 
 extern "C" int wr_bprmf_step_sharded_supported(int64_t n_local_rows, int D) {
