@@ -33,7 +33,7 @@ extern "C" {
 #define WR_E_NULL (-1)   /* a required pointer is NULL */
 #define WR_E_SIZE (-2)   /* a negative / inconsistent size */
 #define WR_E_DIM (-3)    /* embedding size not supported (D % 4 != 0 or D > 512) */
-#define WR_E_TOPK (-4)   /* k outside [1, 32] */
+#define WR_E_TOPK (-4)   /* k outside [1, 32] ([1, 256] for the _long calls, at precision 0 or 2 only) */
 #define WR_E_ALIGN (-5)  /* a table pointer is not 16-byte aligned */
 #define WR_E_PRECISION (-6) /* unknown / unavailable scoring precision */
 
@@ -45,7 +45,9 @@ extern "C" {
                                            holds (degenerate tables, e.g. all rows equal); ranks are incomplete -- rerun
                                            with precision 0 */
 #define WR_STATUS_TOPK_OVERFLOW 8u      /* precision-2 top-k: a row had more list candidates than its segment holds; its
-                                           list is returned as topk_idx[r, 0] = -2 -- rerun those rows with precision 0 */
+                                           list is returned as topk_idx[r, 0] = -2 -- rerun those rows with precision 0.
+                                           Long lists (wr_eval_rank_topk_long): such rows were finished on the device;
+                                           their lists are exact */
 #define WR_PEER_TIMEOUT_NS 20000000000ull
 
 int wr_version(void);
@@ -595,6 +597,39 @@ int wr_rowdot(const float *A, const float *B, int64_t R, int D, int round_bf16, 
  * ids, unfilled slots -1 / -inf); out: the k best per row, best first, ties to the lower id. */
 int wr_topk_merge(const float *val, const int32_t *idx, int world, int64_t R, int k, float *out_val,
                   int32_t *out_idx, void *stream);
+
+/* ---- top-k lists with k up to 256 ---------------------------------------------------------------------------
+ * wr_eval_rank_topk_long: wr_eval_rank_topk for 1 <= k <= 256 (lists required, no score dump).  Every row gets precision
+ * 0's list: the same item ids in the same order, the same fp32 values (the d = 0 .. D-1 FMA chain), ordered by (value desc,
+ * id asc), history items masked, padded with (-1, -inf).  rank and target equal those of a k = 0 call at the same
+ * precision.  precision 0: D in {16, 32, 64, 128, 256}; precision 2: D in {64, 128, 256} (tensor cores); precision 1 and
+ * any other k: WR_E_TOPK.  The wrappers of this library use it for k > 32 only.
+ * Three passes per block of rows: a bound pass takes the k'-th best score of each of n >= S = ceil(k / 32) item ranges
+ * (k' = ceil(k / S) <= 32) -- the S-th largest of them, L, bounds the k-th best from below (precision 2: on the
+ * tensor-core scores, so the candidates are t >= L - 2 eps_r) -- a collect pass computes the ranks and appends every
+ * unmasked item at or above the bound to a 4,096-id segment per row, and a select pass re-scores the candidates with
+ * precision 0's FMA chain and sorts them.  A row with more candidates is finished on the device by a sweep over all its items:
+ * WR_STATUS_TOPK_OVERFLOW is raised and the 32-bit word at scratch[0] counts those rows; the lists are exact either way.
+ * scratch: wr_eval_scratch_bytes_topk_long bytes, 1024-byte aligned (required at both precisions).
+ */
+int wr_eval_rank_topk_long(const float *Uemb, const float *Iemb, const int64_t *user, const int64_t *pos, int64_t R,
+                           int64_t n_users, int64_t n_items, int D, const int64_t *hist_ptr, const int32_t *hist_idx,
+                           int k, int precision, int32_t *topk_idx, float *topk_val, int32_t *rank, float *target,
+                           void *scratch, void *ws, void *stream);
+
+/* wr_eval_rank_topk_long against ONE item shard, with the arguments of wr_eval_rank_topk_shard (LOCAL list ids). */
+int wr_eval_rank_topk_long_shard(const float *Urows, const float *Iemb, const int64_t *user, const int64_t *pos_local,
+                                 int64_t R, int64_t n_users, int64_t n_items_local, int D, const int64_t *hist_ptr,
+                                 const int32_t *hist_idx, int k, int precision, const float *target, int32_t *topk_idx,
+                                 float *topk_val, int32_t *rank, void *scratch, void *ws, void *stream);
+
+/* Bytes of scratch a long call needs (0 for arguments it refuses): the header, precision 2's wr_eval_scratch_bytes, and
+ * per row of a block (at most 65,536 rows, so the segments stay <= 1 GB) 16 range bounds, a count and 4,096 ids. */
+size_t wr_eval_scratch_bytes_topk_long(int64_t R, int64_t n_items, int D, int precision, int k);
+
+/* wr_topk_merge for lists of 1 <= k <= 256 entries: val / idx [world, R, k]. */
+int wr_topk_merge_long(const float *val, const int32_t *idx, int world, int64_t R, int k, float *out_val,
+                       int32_t *out_idx, void *stream);
 
 #ifdef __cplusplus
 }

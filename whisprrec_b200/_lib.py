@@ -99,6 +99,13 @@ SIGNATURES = {
                                        _p, _p, _p]),
     'wr_rowdot': (_int, [_p, _p, _i64, _int, _int, _p, _p]),
     'wr_topk_merge': (_int, [_p, _p, _int, _i64, _int, _p, _p, _p]),
+    # ---- top-k lists of up to 256 items ----
+    'wr_eval_rank_topk_long': (_int, [_p, _p, _p, _p, _i64, _i64, _i64, _int, _p, _p, _int, _int, _p, _p, _p, _p, _p,
+                                      _p, _p]),
+    'wr_eval_rank_topk_long_shard': (_int, [_p, _p, _p, _p, _i64, _i64, _i64, _int, _p, _p, _int, _int, _p, _p, _p, _p,
+                                            _p, _p, _p]),
+    'wr_eval_scratch_bytes_topk_long': (_sz, [_i64, _i64, _int, _int, _int]),
+    'wr_topk_merge_long': (_int, [_p, _p, _int, _i64, _int, _p, _p, _p]),
 }
 
 _lib = None
@@ -164,7 +171,8 @@ class Workspace:
         lib = load()
         self.buf = torch.empty(lib.wr_workspace_bytes(), dtype=torch.uint8, device=device)
         check(lib.wr_workspace_init(self.buf.data_ptr(), stream_ptr()))
-        self.last_topk_fallback_rows = 0      # rows of the last precision-2 top-k call that were rerun at precision 0
+        # rows of the last top-k call that were rerun at precision 0 (k <= 32) or finished by the row sweep (k > 32)
+        self.last_topk_fallback_rows = 0
 
     @property
     def ptr(self):
@@ -516,6 +524,84 @@ def exact_tc_topk_supported(D, k, scores=False):
     return D in (64, 128, 256) and 1 <= k <= 32 and not scores
 
 
+TOPK_KMAX = 32             # lists of wr_eval_rank_topk
+TOPK_LONG_KMAX = 256       # lists of wr_eval_rank_topk_long
+
+
+def exact_tc_topk_long_supported(D, k):
+    """precision 2 with long lists (wr_eval_rank_topk_long on the tensor cores): D in {64, 128, 256}, 1 <= k <= 256.
+    The wrappers below use that entry point for k > 32 only."""
+    return D in (64, 128, 256) and 1 <= k <= TOPK_LONG_KMAX
+
+
+def _long_precision(D, k, precision, scores):
+    """The precision a list of k > 32 items is computed at: 2 on the tensor cores where they cover D, else 0."""
+    if precision == 1:
+        raise WhisprError(f'precision 1 gives top-k lists of at most {TOPK_KMAX} items (k = {k}); use precision 0 or 2')
+    if scores:
+        raise WhisprError(f'no dense score dump with top-k lists of more than {TOPK_KMAX} items')
+    if k > TOPK_LONG_KMAX:
+        raise WhisprError(f'top-k lists hold at most {TOPK_LONG_KMAX} items (k = {k})')
+    return 2 if precision == 2 and exact_tc_topk_long_supported(D, k) else 0
+
+
+def _aligned_scratch(nbytes, dev):
+    scratch = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
+    off = (-scratch.data_ptr()) % 1024
+    return scratch[off:off + nbytes]
+
+
+def _long_call(launch, R, n_items, D, k, precision, ws):
+    """One wr_eval_rank_topk_long(_shard) call, launch(precision, scratch_ptr).  Precision 2 whose rank candidate list
+    overflowed (degenerate tables) is repeated at precision 0.  Rows finished by the device-side sweep go to
+    ws.last_topk_fallback_rows; status bits that are not the call's own are handed back."""
+    keep = 0
+    for p in ((2, 0) if precision == 2 else (0,)):
+        scratch = _aligned_scratch(load().wr_eval_scratch_bytes_topk_long(R, n_items, D, p, k), ws.buf.device)
+        out = launch(p, scratch.data_ptr())
+        st = ws.status()
+        keep |= st & ~12
+        if not (p == 2 and st & 4):
+            break
+    ws.last_topk_fallback_rows = int(scratch[:4].view(torch.int32).item())
+    if keep:
+        ws.restore_status(keep)
+    return out
+
+
+def _eval_rank_topk_long(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k, precision):
+    R, D = user.numel(), Uemb.shape[1]
+    dev = Uemb.device
+    rank = torch.empty(R, dtype=I32, device=dev)
+    target = torch.empty(R, dtype=F32, device=dev)
+    tki = torch.empty((R, k), dtype=I32, device=dev)
+    tkv = torch.empty((R, k), dtype=F32, device=dev)
+
+    def launch(p, scratch):
+        check(load().wr_eval_rank_topk_long(ptr(Uemb, F32), ptr(Iemb, F32), ptr(user, I64), ptr(pos, I64), R,
+                                            Uemb.shape[0], Iemb.shape[0], D, ptr(hist_ptr, I64), ptr(hist_idx, I32), k,
+                                            p, ptr(tki, I32), ptr(tkv, F32), ptr(rank, I32), ptr(target, F32), scratch,
+                                            ws.ptr, stream_ptr()))
+        return rank, target, tki, tkv, None
+    return _long_call(launch, R, Iemb.shape[0], D, k, precision, ws)
+
+
+def _eval_rank_topk_long_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k, precision):
+    R, D = user.numel(), Urows.shape[1]
+    dev = Urows.device
+    rank = torch.empty(R, dtype=I32, device=dev)
+    tki = torch.empty((R, k), dtype=I32, device=dev)
+    tkv = torch.empty((R, k), dtype=F32, device=dev)
+
+    def launch(p, scratch):
+        check(load().wr_eval_rank_topk_long_shard(ptr(Urows, F32), ptr(Iemb, F32), ptr(user, I64), ptr(pos_local, I64),
+                                                  R, n_users, Iemb.shape[0], D, ptr(hist_ptr, I64), ptr(hist_idx, I32),
+                                                  k, p, ptr(target, F32), ptr(tki, I32), ptr(tkv, F32), ptr(rank, I32),
+                                                  scratch, ws.ptr, stream_ptr()))
+        return rank, tki, tkv
+    return _long_call(launch, R, Iemb.shape[0], D, k, precision, ws)
+
+
 def _exact_topk_fallback(out, U, gathered, Iemb, user, pos, n_users, hist_ptr, hist_idx, target, ws, k):
     """Rows of a precision-2 top-k call whose candidate segment overflowed (topk_idx[r, 0] = -2): their lists again with
     precision 0, on those rows only (item-shard mode with their targets); the ranks are exact already.  U: the user
@@ -536,8 +622,14 @@ def eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k=0, precision
     scores fp32 [R, n_items] | None).  precision: 0 fp32 FMA tiles; 1 bf16 tensor cores; 2 split-bf16 tensor cores +
     exact re-check (ranks identical to 0; if the candidate list overflows -- degenerate tables -- the call is repeated
     with precision 0, which costs one synchronisation).  Precision 2 with k in 1..32 gives precision 0's lists too: rows
-    whose list candidates overflow their segment are rerun alone at precision 0 (ws.last_topk_fallback_rows)."""
+    whose list candidates overflow their segment are rerun alone at precision 0 (ws.last_topk_fallback_rows).
+    k in 33..256 (precision 0 or 2; 2 falls back to 0 where the tensor cores do not cover D): the same lists from
+    wr_eval_rank_topk_long; rows with more candidates than their segment holds are finished on the device
+    (ws.last_topk_fallback_rows)."""
     R, D = user.numel(), Uemb.shape[1]
+    if k > TOPK_KMAX:
+        return _eval_rank_topk_long(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k,
+                                    _long_precision(D, k, precision, scores))
     if precision == 2 and k > 0:
         if not exact_tc_topk_supported(D, k, scores):
             return _eval_rank_topk(Uemb, Iemb, user, pos, hist_ptr, hist_idx, ws, k, 0, scores)
@@ -886,8 +978,11 @@ def rowdot(A, B, round_bf16=False):
 
 def eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k=0, precision=0):
     """One item shard: returns (rank int32 [R] = 1 + local count, topk_idx LOCAL int32 [R,k] | None, topk_val | None).
-    Precision 2 with k as in eval_rank_topk."""
+    Precision 2 with k, and k up to 256, as in eval_rank_topk."""
     R, D = user.numel(), Urows.shape[1]
+    if k > TOPK_KMAX:
+        return _eval_rank_topk_long_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k,
+                                          _long_precision(D, k, precision, False))
     if precision == 2 and k > 0:
         if not exact_tc_topk_supported(D, k):
             return _eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_idx, target, ws, k, 0)
@@ -938,9 +1033,10 @@ def _eval_rank_topk_shard(Urows, Iemb, user, pos_local, n_users, hist_ptr, hist_
 
 
 def topk_merge(val, idx, k):
-    """val / idx: [world, R, k] candidates with GLOBAL item ids -> ([R, k] values, [R, k] ids)."""
+    """val / idx: [world, R, k] candidates with GLOBAL item ids -> ([R, k] values, [R, k] ids); k up to 256."""
     world, R = val.shape[0], val.shape[1]
     ov = torch.empty((R, k), dtype=F32, device=val.device)
     oi = torch.empty((R, k), dtype=I32, device=val.device)
-    check(load().wr_topk_merge(ptr(val, F32), ptr(idx, I32), world, R, k, ptr(ov, F32), ptr(oi, I32), stream_ptr()))
+    merge = load().wr_topk_merge_long if k > TOPK_KMAX else load().wr_topk_merge
+    check(merge(ptr(val, F32), ptr(idx, I32), world, R, k, ptr(ov, F32), ptr(oi, I32), stream_ptr()))
     return ov, oi

@@ -56,6 +56,76 @@ static inline int sm_count() {
 }
 #define kSMs (::wr::sm_count())
 
+// ---- top-k lists with k up to 256 (wr_eval_rank_topk_long, DESIGN.md section 4.3) ----
+constexpr int WR_LONG_KMAX = 256;
+constexpr int WR_LONG_SEG_CAP = 4096;            // candidate ids kept per row; a row with more is finished by a sweep
+constexpr int WR_LONG_RANGES = 16;               // item ranges of the bound pass: ceil(k / 32) .. 2 ceil(k / 32) - 1
+constexpr int64_t WR_LONG_BLOCK_ROWS = 65536;    // rows per block, so that the segments stay <= 1 GB
+
+// The part of a long call's scratch that both precisions use: a 1,024-byte header at offset 0 (word 0: rows the sweep
+// finished, read by the caller), then -- after precision 2's tensor-core scratch -- these per-row-block arrays.
+struct LongScratch {
+    float *bound;        // [rows][WR_LONG_RANGES] the k'-th best score of each item range
+    int32_t *seg_cnt;    // [rows] candidates appended
+    int32_t *seg;        // [rows][WR_LONG_SEG_CAP] candidate item ids
+    static size_t align(size_t x) { return (x + 1023) / 1024 * 1024; }
+    static size_t bytes(int64_t rows) {
+        return align((size_t)rows * WR_LONG_RANGES * 4) + align((size_t)rows * 4) + (size_t)rows * WR_LONG_SEG_CAP * 4;
+    }
+    LongScratch(void *base, int64_t rows) {
+        uint8_t *p = static_cast<uint8_t *>(base);
+        bound = reinterpret_cast<float *>(p);
+        seg_cnt = reinterpret_cast<int32_t *>(p + align((size_t)rows * WR_LONG_RANGES * 4));
+        seg = reinterpret_cast<int32_t *>(p + align((size_t)rows * WR_LONG_RANGES * 4) + align((size_t)rows * 4));
+    }
+};
+
+// The select pass of a long call (eval_kernels.cu): one CTA per row re-scores the row's candidates with precision 0's FMA
+// chain and sorts them by (value desc, id asc); a row whose segment overflowed is swept over every item instead.
+struct LongSelect {
+    const int32_t *seg, *seg_cnt;
+    int64_t R;                   // rows of this block
+    const float *U;              // user table (rows_gathered = 0: row r is U[user[r]]) or the block's gathered rows
+    const int64_t *user;
+    int rows_gathered;
+    const float *I;
+    int D;
+    int64_t n_items;
+    const int64_t *hist_ptr;
+    const int32_t *hist_idx;
+    int k;
+    int32_t *topk_idx;           // the block's [R][k] outputs
+    float *topk_val;
+    uint32_t *fallback;          // rows swept (header word 0 of the scratch)
+    uint32_t *status;
+};
+int long_select(const LongSelect &q, cudaStream_t st);
+
+// Item ranges of the bound pass over n_tiles tiles for a k-list: need = ceil(k / 32) or more ranges of whole tiles (the
+// last may be short), each giving the k'-th best of its items, k' = ceil(k / need) <= 32, from the k <= 32 list
+// machinery.  Returns the number of ranges (0: fewer tiles than need -- no bound, every unmasked item is a candidate) and
+// sets the tiles per range, k' and need.
+static inline int long_ranges(int n_tiles, int k, int *tiles_per_range, int *kp, int *need) {
+    *need = (k + 31) / 32;
+    *kp = (k + *need - 1) / *need;
+    if (n_tiles < *need) return 0;
+    *tiles_per_range = n_tiles / *need;
+    return (n_tiles + *tiles_per_range - 1) / *tiles_per_range;      // need .. 2 need - 1
+}
+
+// The collect pass's threshold for one row: the need-th largest of its n range bounds b.  The need ranges whose bounds
+// are at least that large each hold k' unmasked items scoring at or above their bound, so need k' >= k items reach it: a
+// lower bound on the row's k-th best.  -inf when fewer than need ranges hold k' items (or n = 0).
+__device__ __forceinline__ float long_bound(const float *b, int n, int need) {
+    float L = -INFINITY;
+    for (int c = 0; c < n; ++c) {
+        int ge = 0;
+        for (int c2 = 0; c2 < n; ++c2) ge += b[c2] >= b[c] ? 1 : 0;
+        if (ge >= need) L = fmaxf(L, b[c]);
+    }
+    return L;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

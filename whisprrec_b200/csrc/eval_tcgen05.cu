@@ -52,6 +52,8 @@ struct TcParams {
     uint32_t *status;           // WR_STATUS_EVAL_OVERFLOW when the list is full
     int32_t *seg;               // top-k: [rows][TC_SEG_CAP] list candidates (item ids) per row
     int32_t *seg_cnt;           // top-k: [rows] candidates appended (> TC_SEG_CAP: the segment overflowed)
+    float *bound;               // long lists: [rows][WR_LONG_RANGES] the k'-th best t of each item range
+    int n_bounds, bound_need;   // long lists, collect pass: ranges written by the bound pass (0: no bound), long_bound
 };
 
 constexpr int TC_KMAX = 32;
@@ -530,12 +532,17 @@ __device__ __forceinline__ void ring_push(const TopRings &rg, int row, float x, 
     }
 }
 
-template <int K, int VARIANT, int TOPK, int EXACT, int MT>
+// LONG (precision 2 with TOPK = 2 only, wr_eval_rank_topk_long): 1 = bound pass -- the drain warps keep the k'-best list
+// of this CTA's item range (blockIdx.y) and write its k'-th best t, no segment; 2 = collect pass -- the row's threshold is
+// fixed at long_bound of its range bounds and every item the epilogue pushes (t >= that bound - 2 eps_r) goes to its
+// segment.
+template <int K, int VARIANT, int TOPK, int EXACT, int MT, int LONG = 0>
 __global__ void __launch_bounds__(TOPK == 2 ? TC_THREADS_DRAIN : TC_THREADS, 1)
 eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TcParams p) {
     using C = TcCfg<K, EXACT, MT, TOPK>;
     static_assert(MT == 1 || TOPK == 0, "the top-k lists are laid out for 128 rows per CTA");
     static_assert(!EXACT || TOPK != 1, "precision 2 builds its lists with the drain warps");
+    static_assert(LONG == 0 || (EXACT && TOPK == 2), "long lists are a precision-2 drain-warp mode");
     static_assert(TOPK != 1 || C::STAGES * C::STAGE_BYTES >= TC_BM * 4 * TC_KMAX * 8, "stripe lists fit in the B ring");
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -583,7 +590,8 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         for (int i = 0; i < TC_RING; ++i) rg.id[r * TC_RING + i] = -1;
         rg.head[r] = 0;
         rg.tail[r] = 0;
-        rg.tau[r] = -INFINITY;
+        rg.tau[r] = LONG == 2 && row0 + r < p.R ? long_bound(p.bound + (row0 + r) * WR_LONG_RANGES, p.n_bounds, p.bound_need)
+                                                : -INFINITY;
         if (r == 0) *rg.epi_done = 0;
     }
     tc_fence_before();
@@ -993,11 +1001,12 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         // segment -- every entry of the list and every score within the band of its k-th best on arrival
         const int64_t row = row0 + r;
         float e = 0.f;
+        constexpr int SEG_CAP = LONG ? WR_LONG_SEG_CAP : TC_SEG_CAP;
         int nseg = 0;
         int32_t *segr = nullptr;
         if (EXACT && row < p.R) {
             e = p.band_c * p.anorm[row] * p.bmax[0];
-            segr = p.seg + row * TC_SEG_CAP;
+            if (LONG != 1) segr = p.seg + row * SEG_CAP;
         }
         volatile uint32_t *vhead = rg.head + r;
         volatile int32_t *vid = rg.id + r * TC_RING;
@@ -1020,8 +1029,8 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 __threadfence_block();
                 ++tail;
                 *reinterpret_cast<volatile uint32_t *>(rg.tail + r) = tail;
-                bool keep = false;
-                if (top_worse(w, wid, x, id)) {         // beats the worst kept entry (ties: the lower id wins)
+                bool keep = LONG == 2;                  // collect pass: every push is a candidate, tau stays put
+                if (LONG != 2 && top_worse(w, wid, x, id)) {    // beats the worst kept entry (ties: the lower id wins)
                     keep = true;
                     lv[wp] = x;
                     li[wp] = id;
@@ -1036,16 +1045,18 @@ eval_tc_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                         }
                     }
                     *reinterpret_cast<volatile float *>(rg.tau + r) = w;
-                } else if (EXACT && e > 0.f && x >= exact_topk_floor(w, e)) {
+                } else if (LONG == 0 && EXACT && e > 0.f && x >= exact_topk_floor(w, e)) {
                     keep = true;                        // below the list but within 2 eps_r of its k-th best
                 }
-                if (EXACT && keep) {
-                    if (nseg < TC_SEG_CAP) segr[nseg] = id;
+                if (EXACT && LONG != 1 && keep) {
+                    if (nseg < SEG_CAP) segr[nseg] = id;
                     ++nseg;
                 }
             }
         }
-        if (EXACT) {
+        if (LONG == 1) {
+            if (row < p.R) p.bound[row * WR_LONG_RANGES + blockIdx.y] = w;     // -inf: fewer than k' items in range
+        } else if (EXACT) {
             if (row < p.R) p.seg_cnt[row] = nseg;
         } else if (row < p.R) {
             for (int s = 0; s < k; ++s) {               // k selection passes: best first
@@ -1097,15 +1108,15 @@ static int make_map(CUtensorMap *map, const void *base, int64_t rows, int D /* b
     return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
 }
 
-template <int K, int VARIANT, int TOPK, int EXACT, int MT>
+template <int K, int VARIANT, int TOPK, int EXACT, int MT, int LONG = 0>
 static int launch_tc_v(const CUtensorMap &ma, const CUtensorMap &mb, TcParams &p, int row_tiles, cudaStream_t st) {
     constexpr int smem = TcCfg<K, EXACT, MT, TOPK>::SMEM + (TOPK == 2 ? TC_SMEM_DRAIN : 0);
     constexpr int threads = TOPK == 2 ? TC_THREADS_DRAIN : TC_THREADS;
     static_assert(smem <= 227 * 1024, "shared memory budget");
-    cudaError_t e = cudaFuncSetAttribute(eval_tc_rank_kernel<K, VARIANT, TOPK, EXACT, MT>,
+    cudaError_t e = cudaFuncSetAttribute(eval_tc_rank_kernel<K, VARIANT, TOPK, EXACT, MT, LONG>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return (int)e;
-    eval_tc_rank_kernel<K, VARIANT, TOPK, EXACT, MT><<<dim3(row_tiles, p.splits), threads, smem, st>>>(ma, mb, p);
+    eval_tc_rank_kernel<K, VARIANT, TOPK, EXACT, MT, LONG><<<dim3(row_tiles, p.splits), threads, smem, st>>>(ma, mb, p);
     return (int)cudaGetLastError();
 }
 
@@ -1178,6 +1189,14 @@ static void exact_blocking_topk(int64_t R, int64_t n_items, int k, int64_t *rows
     if (k > 0 && *rows_per_block > most) *rows_per_block = most;
 }
 
+// long lists: the same blocks, at most WR_LONG_BLOCK_ROWS rows so that the segments (16 KB per row) stay <= 1 GB
+static int64_t exact_blocking_long(int64_t R, int64_t n_items) {
+    int64_t rb;
+    unsigned long long cap;
+    exact_blocking(R, n_items, &rb, &cap);
+    return rb < WR_LONG_BLOCK_ROWS ? rb : WR_LONG_BLOCK_ROWS;
+}
+
 extern "C" size_t wr_eval_scratch_bytes(int64_t R, int64_t n_items, int D, int precision) {
     if ((precision != 1 && precision != 2) || R <= 0 || n_items <= 0 || D <= 0) return 0;
     const size_t k = precision == 2 ? 3 : 1;
@@ -1201,11 +1220,25 @@ extern "C" size_t wr_eval_scratch_bytes_topk(int64_t R, int64_t n_items, int D, 
     return n + 1024 + align_up((size_t)rb * 4, 1024) + (size_t)rb * TC_SEG_CAP * 4;      // counts, then segments
 }
 
-// precision-1 / precision-2 body of wr_eval_rank_topk (eval_kernels.cu dispatches here)
+// A long call (wr_eval_rank_topk_long) needs a 1,024-byte header; precision 2 then lays out the rank path's scratch and,
+// behind it, the per-block bounds and segments (LongScratch); precision 0 only the latter, over blocks of at most
+// WR_LONG_BLOCK_ROWS rows.
+extern "C" size_t wr_eval_scratch_bytes_topk_long(int64_t R, int64_t n_items, int D, int precision, int k) {
+    if (R <= 0 || n_items <= 0 || k < 1 || k > WR_LONG_KMAX) return 0;
+    if (precision == 0) {
+        if (D != 16 && D != 32 && D != 64 && D != 128 && D != 256) return 0;
+        return 1024 + LongScratch::bytes(R < WR_LONG_BLOCK_ROWS ? R : WR_LONG_BLOCK_ROWS);
+    }
+    if (precision != 2 || (D != 64 && D != 128 && D != 256)) return 0;
+    return 1024 + wr_eval_scratch_bytes(R, n_items, D, 2) + LongScratch::bytes(exact_blocking_long(R, n_items));
+}
+
+// precision-1 / precision-2 body of wr_eval_rank_topk (eval_kernels.cu dispatches here) and precision 2 of
+// wr_eval_rank_topk_long (long_lists: k <= 256, `scratch` past the long call's header)
 int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, const int64_t *pos, int64_t R,
                     int64_t n_users, int64_t n_items, int D, const int64_t *hist_ptr, const int32_t *hist_idx,
                     int32_t *rank, float *target, const float *target_in, float *scores_out, int k, int32_t *topk_idx,
-                    float *topk_val, void *scratch, WrWorkspace *ws, cudaStream_t st, int precision) {
+                    float *topk_val, void *scratch, WrWorkspace *ws, cudaStream_t st, int precision, bool long_lists) {
     if (D != 64 && D != 128 && D != 256) return WR_E_DIM;
     if (!scratch) return WR_E_NULL;
     if ((reinterpret_cast<uintptr_t>(scratch) & 1023u) != 0) return WR_E_ALIGN;
@@ -1278,11 +1311,13 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
     uint2 *cand = reinterpret_cast<uint2 *>(base);
     int64_t rb;
     unsigned long long cap;
-    exact_blocking_topk(R, n_items, topk_idx ? k : 0, &rb, &cap);
-    // top-k: per-row candidate counts and segments behind the list (wr_eval_scratch_bytes_topk)
+    exact_blocking_topk(R, n_items, topk_idx && !long_lists ? k : 0, &rb, &cap);
+    if (long_lists) rb = exact_blocking_long(R, n_items);
+    // top-k: per-row candidate counts and segments behind the list (wr_eval_scratch_bytes_topk); long lists: LongScratch
     const size_t seg_at = align_up((size_t)(base - static_cast<uint8_t *>(scratch)) + (size_t)cap * 8, 1024);
     int32_t *seg_cnt = reinterpret_cast<int32_t *>(static_cast<uint8_t *>(scratch) + seg_at);
     int32_t *seg = reinterpret_cast<int32_t *>(static_cast<uint8_t *>(scratch) + seg_at + align_up((size_t)rb * 4, 1024));
+    const LongScratch lg(static_cast<uint8_t *>(scratch) + seg_at, rb);
     cudaError_t e = cudaMemsetAsync(bmax_bits, 0, 64, st);
     if (e != cudaSuccess) return (int)e;
     pack_items_split_kernel<<<(int)min((int64_t)16 * kSMs, (n_items + 7) / 8), 256, 0, st>>>(Iemb, n_items, D, Bm, bmax_bits);
@@ -1321,9 +1356,43 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
             fill_rank_kernel<<<(int)min((int64_t)kSMs * 4, (rn + 255) / 256), 256, 0, st>>>(q.rank, rn, 1);
             WR_CHECK_LAUNCH();
         }
+        int ranges = 0, need = 1;
+        if (long_lists) {
+            // bound pass: the k'-th best t of each item range (its ranks land in the segment counts and are not used)
+            int tpr = 0, kp = 0;
+            ranges = long_ranges(q.n_tiles, k, &tpr, &kp, &need);
+            if (ranges > 0) {
+                TcParams b = q;
+                b.k = kp;
+                b.splits = ranges;
+                b.tiles_per_split = tpr;
+                b.rank = lg.seg_cnt;
+                b.bound = lg.bound;
+                e = cudaMemsetAsync(cand_cnt, 0, sizeof(unsigned long long), st);
+                if (e != cudaSuccess) return (int)e;
+                switch (D) {
+                    case 64: rc = launch_tc_v<192, 1, 2, 1, 1, 1>(ma, mb, b, row_tiles, st); break;
+                    case 128: rc = launch_tc_v<384, 1, 2, 1, 1, 1>(ma, mb, b, row_tiles, st); break;
+                    default: rc = launch_tc_v<768, 1, 2, 1, 1, 1>(ma, mb, b, row_tiles, st); break;
+                }
+                if (rc) return rc;
+            }
+        }
         e = cudaMemsetAsync(cand_cnt, 0, sizeof(unsigned long long), st);
         if (e != cudaSuccess) return (int)e;
-        if (topk_idx) {              // the ranks as below, plus the drain warps' candidate segments
+        if (long_lists) {            // collect pass: the ranks, and every item at or above the row's fixed threshold
+            q.k = 1;
+            q.seg = lg.seg;
+            q.seg_cnt = lg.seg_cnt;
+            q.bound = lg.bound;
+            q.n_bounds = ranges;
+            q.bound_need = need;
+            switch (D) {
+                case 64: rc = launch_tc_v<192, 1, 2, 1, 1, 2>(ma, mb, q, row_tiles, st); break;
+                case 128: rc = launch_tc_v<384, 1, 2, 1, 1, 2>(ma, mb, q, row_tiles, st); break;
+                default: rc = launch_tc_v<768, 1, 2, 1, 1, 2>(ma, mb, q, row_tiles, st); break;
+            }
+        } else if (topk_idx) {       // the ranks as below, plus the drain warps' candidate segments
             switch (D) {
                 case 64: rc = launch_tc_v<192, 1, 2, 1, 1>(ma, mb, q, row_tiles, st); break;
                 case 128: rc = launch_tc_v<384, 1, 2, 1, 1>(ma, mb, q, row_tiles, st); break;
@@ -1341,7 +1410,13 @@ int wr_eval_rank_tc(const float *Uemb, const float *Iemb, const int64_t *user, c
         eval_recheck_kernel<<<8 * kSMs, 256, 0, st>>>(cand, cand_cnt, cap, Ublk, q.user, target_in ? 1 : 0, Iemb, D,
                                                        q.target, q.rank);
         WR_CHECK_LAUNCH();
-        if (topk_idx) {
+        if (long_lists) {
+            uint32_t *fallback = reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(scratch) - 1024);     // header word 0
+            LongSelect sel{lg.seg, lg.seg_cnt, rn, Ublk, q.user, target_in ? 1 : 0, Iemb, D, n_items, hist_ptr, hist_idx, k,
+                           topk_idx + r0 * k, topk_val + r0 * k, fallback, &ws->status};
+            rc = long_select(sel, st);
+            if (rc) return rc;
+        } else if (topk_idx) {
             eval_topk_select_kernel<<<(int)min((int64_t)16 * kSMs, (rn + 7) / 8), 256, 0, st>>>(
                 seg, seg_cnt, rn, Ublk, q.user, target_in ? 1 : 0, Iemb, D, k, q.topk_idx, q.topk_val, &ws->status);
             WR_CHECK_LAUNCH();

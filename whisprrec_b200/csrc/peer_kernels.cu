@@ -282,3 +282,16 @@ extern "C" int wr_topk_merge(const float *val, const int32_t *idx, int world, in
     WR_CHECK_LAUNCH();
     return WR_OK;
 }
+
+// the same merge for lists of up to WR_LONG_KMAX entries (the kernel is per row and k-agnostic)
+extern "C" int wr_topk_merge_long(const float *val, const int32_t *idx, int world, int64_t R, int k, float *out_val,
+                                  int32_t *out_idx, void *stream) {
+    if (!val || !idx || !out_val || !out_idx) return WR_E_NULL;
+    if (world < 1 || world > WR_MAX_WORLD || R <= 0) return WR_E_SIZE;
+    if (k < 1 || k > WR_LONG_KMAX) return WR_E_TOPK;
+    int64_t g = (R + 127) / 128;
+    if (g > 8 * kSMs) g = 8 * kSMs;
+    topk_merge_kernel<<<(int)g, 128, 0, (cudaStream_t)stream>>>(val, idx, world, R, k, out_val, out_idx);
+    WR_CHECK_LAUNCH();
+    return WR_OK;
+}

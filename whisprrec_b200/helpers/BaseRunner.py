@@ -306,8 +306,11 @@ class BaseRunner(object):
         """Top-k recommendation lists for each row of `dataset`: (items int64 [n, k], scores float32 [n, k]) as host
         NumPy arrays, best first, in the corpus's item codes.  The user's history is masked as in evaluation; rows with
         fewer than k candidates are padded with (-1, -inf).  k defaults to max(self.topk).  At the default precision 2
-        the lists equal precision 0's.  On a sharded model every rank returns the same lists."""
+        the lists equal precision 0's.  On a sharded model every rank returns the same lists.  k is at most 256 (lists
+        of more than 32 items at precision 0 or 2)."""
         k = max(self.topk) if k is None else int(k)
+        if not 1 <= k <= _lib.TOPK_LONG_KMAX:
+            raise ValueError(f'recommend: k must be in 1..{_lib.TOPK_LONG_KMAX}, got {k}')
         _, _, tki, tkv, _ = self.rank_topk(dataset, k=k)
         dataset.model.tables.ws.raise_on_status()
         return tki.to(torch.int64).cpu().numpy(), tkv.cpu().numpy()
