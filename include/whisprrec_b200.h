@@ -200,9 +200,11 @@ int wr_bprmf_ctx_destroy(wr_bprmf_ctx *ctx);
  *     a_b = normalize(T1[idx_b]), t_j = normalize(T2[j]) (F.normalize, eps 1e-12), z_b = sum_j exp(a_b . t_j / tau)
  *     loss_out[0] += weight * sum_b (log z_b - a_b . t_{idx_b} / tau)
  *     dT1[idx_b] += grad_scale * dL/dT1[idx_b] (RED per occurrence), dT2[j] += grad_scale * dL/dT2[j] for every j
- *   T1 / T2 / dT1 / dT2: [N, D] fp32 blocks of the pooled view tables and their gradients; the [B, N] contraction runs as
- *   fp32 FMA tiles over a materialised softmax weight matrix (B x N x 4 bytes <= 512 MB).
- *   scratch: wr_infonce_scratch_bytes(B, N, D) bytes of device memory.
+ *   T1 / T2 / dT1 / dT2: [N, D] fp32 blocks of the pooled view tables and their gradients; D <= 256 (WR_E_DIM above).
+ *   The [B, N] contraction is streamed as fp32 FMA tiles in two passes over the table (row sums, then the weights
+ *   recomputed for both gradient products); no buffer grows with B x N, so any catalogue size runs.  The loss is the
+ *   same bits from call to call; the gradients are summed with REDs.
+ *   scratch: wr_infonce_scratch_bytes(B, N, D) bytes of device memory, O((B + N) D) (0 for arguments the call refuses).
  */
 int wr_bpr_logsig_sum_fwd_bwd(const float *U, const float *I, const int64_t *user, const int64_t *pos, const int64_t *neg,
                               int64_t B, int D, int64_t n_users, int64_t n_items, float grad_scale, float *gU, float *gI,
