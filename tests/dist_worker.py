@@ -6,7 +6,8 @@
 
 `gpu`: one B200 per rank.  The sharded BPRMF step, LightGCN step and item-sharded evaluation must reproduce the
 single-GPU kernels run by the same rank on the whole batch / whole tables (SURVEY.md section 8e: "G in {2,4,8}
-results equal G = 1").
+results equal G = 1").  The per-rank body, check_sharded_paths, also runs on one GPU with emulated ranks in threads
+(tests/test_sharded_emulated.py).
 """
 import os
 import sys
@@ -128,16 +129,27 @@ def run_cpu():
 # NCCL / one B200 per rank
 # --------------------------------------------------------------------------------------------------------------
 def run_gpu():
-    from oracle import whispr_oracle as O
-    from whisprrec_b200 import _lib
     from whisprrec_b200 import sharded as S
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
     dev = torch.device('cuda', local_rank)
     torch.cuda.set_device(dev)
     dist.init_process_group('nccl', device_id=dev)
-    rank, world = dist.get_rank(), dist.get_world_size()
-    assert torch.cuda.device_count() >= world, 'one GPU per rank (never share a GPU between spinning ranks)'
+    assert torch.cuda.device_count() >= dist.get_world_size(), \
+        'one GPU per rank (never share a GPU between spinning ranks)'
     peers = S.PeerGroup(dev)
+    check_sharded_paths(peers)
+    peers.close()
+    dist.destroy_process_group()
+
+
+def check_sharded_paths(peers):
+    """The per-rank body of the `gpu` mode on one rank of `peers` (a PeerGroup, or anything with its interface: world,
+    rank, device, ws, dist, group, alloc, alloc_bytes, host_sync, barrier).  Prints five `dist_worker gpu ok` lines on
+    rank 0."""
+    from oracle import whispr_oracle as O
+    from whisprrec_b200 import _lib
+    from whisprrec_b200 import sharded as S
+    rank, world, dev = peers.rank, peers.world, peers.device
     d = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
     host = lambda t: t.detach().cpu().numpy()
 
@@ -167,7 +179,7 @@ def run_gpu():
 
         # ---------------- the multi-launch form with the staged (inbox) gradient scatter: large batches ----------------
         if D == 128:
-            Bs = 16384
+            Bs = 8192 * world                               # 8,192 rows per rank: the staged protocol
             tabs3 = S.ShardedTables(peers, lay, D)
             tabs3.load_full(d(U), d(I))
             tabs3.single_launch = False                     # what shards too large for the cooperative step take
@@ -205,6 +217,11 @@ def run_gpu():
         assert (host(got[1]) == host(want[1])).all(), 'sharded targets'
         assert (host(got[2]) == host(want[2])).all(), 'sharded top-k ids'
         assert (host(got[3]) == host(want[3])).all(), 'sharded top-k values'
+        # lists longer than 32 items: the long-list kernels per shard and the long merge
+        want = _lib.eval_rank_topk(gu.contiguous(), gi.contiguous(), d(eu), d(ep), d(hp), d(hi_), ws, k=100)
+        got = S.sharded_eval(tabs, tabs.T, tabs.item_rows(tabs.P), d(eu), d(ep), lh, k=100)
+        for g_, w_, what in zip(got, want, ('ranks', 'targets', 'top-100 ids', 'top-100 values')):
+            assert (host(g_) == host(w_)).all(), 'sharded ' + what
         if D in (64, 128):
             want_tc = _lib.eval_rank_topk(gu.contiguous(), gi.contiguous(), d(eu), d(ep), d(hp), d(hi_), ws, precision=1)
             got_tc = S.sharded_eval(tabs, tabs.T, tabs.item_rows(tabs.P), d(eu), d(ep), lh, precision=1)
@@ -316,8 +333,6 @@ def run_gpu():
         peers.host_sync()
         if rank == 0:
             print(f'dist_worker gpu ok: world {world} {cls.__name__} ml-100k epoch, dev', res)
-    peers.close()
-    dist.destroy_process_group()
 
 
 if __name__ == '__main__':

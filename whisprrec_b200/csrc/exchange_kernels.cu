@@ -34,8 +34,11 @@ __global__ void __launch_bounds__(256) xchg_request_kernel(const int64_t *user, 
     for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < total; s += (int64_t)gridDim.x * blockDim.x) {
         const int64_t b = s / 3;
         const int which = (int)(s - 3 * b);
-        const int64_t id = which == 0 ? user[b] : (which == 1 ? pos[b] : neg[b]);
-        const bool ok = (uint64_t)id < (uint64_t)(which == 0 ? n_users : n_items);
+        const int64_t u = user[b], i = pos[b], j = neg[b];
+        const int64_t id = which == 0 ? u : (which == 1 ? i : j);
+        // an entry with any id out of range is skipped whole, as the batch kernels skip it: none of its rows is requested
+        // (the owners' EmbLoss reads the request lists, so a requested row would count in the norms)
+        const bool ok = (uint64_t)u < (uint64_t)n_users && (uint64_t)i < (uint64_t)n_items && (uint64_t)j < (uint64_t)n_items;
         if (!ok) {
             atomicOr(&ws->status, WR_STATUS_INDEX_OUT_OF_RANGE);
             where[s] = 0;                 // a valid slot (the compute kernel skips the entry by its id check)
@@ -247,7 +250,8 @@ extern "C" int wr_xchg_serve(const float *T_local, int D, int world, int rank, c
     RecvPtrs pr;
     for (int g = 0; g < WR_MAX_WORLD; ++g) {
         pr.recv[g] = g < world ? host_recv[g] : nullptr;
-        if (g < world && (!pr.recv[g] || !wr_aligned16(pr.recv[g]))) return WR_E_NULL;
+        if (g < world && !pr.recv[g]) return WR_E_NULL;
+        if (g < world && !wr_aligned16(pr.recv[g])) return WR_E_ALIGN;
     }
     xchg_serve_kernel<<<16 * kSMs, 256, 0, (cudaStream_t)stream>>>(T_local, D, world, rank, req_local, req_cnt_local, cap, pr);
     WR_CHECK_LAUNCH();
