@@ -423,6 +423,45 @@ int wr_bpr_fwd_bwd_sharded(const wr_shards *host_T, const wr_shards *host_Gd, co
                            const int64_t *pos, const int64_t *neg, int64_t B, int64_t B_global, int D, float gamma,
                            float grad_scale, float *loss_out, void *ws, void *stream);
 
+/* wr_bpr_logsig_sum_fwd_bwd_sharded: wr_bpr_logsig_sum_fwd_bwd (SGL's sum-form BPR) on this rank's slice, with the tables
+ * of wr_bpr_fwd_bwd_sharded.  loss_out[0] = this rank's share, sum_b -logsigmoid(s+ - s-) over the slice; the gradient is
+ * scaled by grad_scale alone (no 1 / B_global). */
+int wr_bpr_logsig_sum_fwd_bwd_sharded(const wr_shards *host_T, const wr_shards *host_Gd, const int64_t *user,
+                                      const int64_t *pos, const int64_t *neg, int64_t B, int64_t B_global, int D,
+                                      float grad_scale, float *loss_out, void *ws, void *stream);
+
+/* wr_infonce_sharded_*: wr_infonce_fwd_bwd for one block (which = 0: the batch's users against all users, 1: the
+ * positive items against all items) of row-sharded view tables.  Every rank runs the GLOBAL batch (idx: its B ids, the
+ * same on every rank) against ITS OWN rows of the block; the table is never gathered.  Three phases, each rank's calls in
+ * this order on its stream, with a wr_peer_barrier between consecutive phases:
+ *   partials: gather T1[idx_b] and T2[idx_b] from their owners and normalise them; normalise this rank's real rows of the
+ *             block of T2 (padding rows stay out of z); pass 1 against them; this rank's partial z_b is stored into
+ *             slot [rank][b] of every rank's z array (host_z[g]: rank g's [world][B] fp32).
+ *   weights:  z_b = the world partials summed in rank order (the same bits on every rank); loss_out[0] +=
+ *             weight * sum_b (log z_b - a_b . t_{idx_b} / tau) -- the InfoNCE loss of the whole batch, identical on
+ *             every rank (add it once, do not sum it over ranks); pass 2 against the local rows, the positive pull by the
+ *             owner of idx_b, the table-side chain rule into this rank's rows of dT2; this rank's partial Ga_b ([B, D])
+ *             is stored into slot [rank][b] of the owner of idx_b (host_ga[g]: rank g's [world][B][D] fp32, 16-byte
+ *             aligned).
+ *   batch:    the owner of idx_b sums Ga_b over the ranks in rank order and applies the chain rule through the
+ *             normalisation of a_b into its local row of dT1 (RED per occurrence).  No remote loads, no remote REDs.
+ * Traffic per block: O(world B D) bytes.  A rank that owns no rows of the block (world > n_users is allowed) takes part in
+ * every phase and contributes nothing to z.  D a multiple of 4, at most 256.  scratch: this rank's
+ * wr_infonce_sharded_scratch_bytes(B, N_local, D) bytes (N_local: its real rows of the block), the same buffer for the
+ * three phases of one block.  Ids outside the block raise WR_STATUS_INDEX_OUT_OF_RANGE and are skipped.
+ */
+size_t wr_infonce_sharded_scratch_bytes(int64_t B, int64_t N_local, int D);
+int wr_infonce_sharded_partials(const wr_shards *host_T1, const wr_shards *host_T2, int which, const int64_t *idx,
+                                int64_t B, int D, float tau, float *const host_z[WR_MAX_WORLD], void *scratch,
+                                size_t scratch_bytes, void *ws, void *stream);
+int wr_infonce_sharded_weights(const wr_shards *host_dT2, int which, const int64_t *idx, int64_t B, int D, float tau,
+                               float weight, float grad_scale, float *const host_z[WR_MAX_WORLD],
+                               float *const host_ga[WR_MAX_WORLD], float *loss_out, void *scratch, size_t scratch_bytes,
+                               void *stream);
+int wr_infonce_sharded_batch(const wr_shards *host_dT1, int which, const int64_t *idx, int64_t B, int D, float tau,
+                             float weight, float grad_scale, float *const host_ga[WR_MAX_WORLD], void *scratch,
+                             size_t scratch_bytes, void *stream);
+
 /* wr_bpr_fwd_bwd_sharded_staged + wr_inbox_scatter: the same for LARGE batches.  16-byte reductions over NVLink do not
  * scale with the number of GPUs (each is its own fabric transaction; measured: 65,536 rows per GPU on 8 GPUs spend
  * 4.5 ms in them), so remote gradient rows are written -- plain coalesced stores -- into the owner's inbox instead, slot

@@ -21,6 +21,9 @@ sharded()    { # sharded 8 [bprmf|lightgcn|both]      (WR_SPMM_PUSH=dma selects 
 push_overlap() { # push_overlap 8
   timeout 600 python -m torch.distributed.run --nnodes=1 --nproc-per-node "$1" --master-addr 127.0.0.1 --master-port 29518 \
       scripts/prof_push_overlap.py "gpurun_out/prof_push_overlap_n$1.json" 1.0 4 2>&1 | tail -20; }
+sgl_sharded() { # sgl_sharded 8      (merges into profiles/r08_bench_sgl_sharded.json; run 1, 2, 4 and 8)
+  timeout 2400 python -m torch.distributed.run --nnodes=1 --nproc-per-node "$1" --master-addr 127.0.0.1 --master-port 29533 \
+      scripts/bench_sgl_sharded.py --out profiles/r08_bench_sgl_sharded.json 2>&1 | tail -8; }
 ncu_all()    { bash scripts/_ncu1.sh; bash scripts/_ncu2.sh; }                                            # `ncu --set full` captures -> profiles/ via scripts/ncu_summary.py
 
 "$@"

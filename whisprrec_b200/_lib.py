@@ -70,6 +70,11 @@ SIGNATURES = {
     'wr_peer_close': (_int, [_p]),
     'wr_peer_barrier': (_int, [_p, _int, _int, _c.c_uint32, _p, _p, _int, _p, _p, _p]),
     'wr_bpr_fwd_bwd_sharded': (_int, [_p, _p, _p, _p, _p, _i64, _i64, _int, _f32, _f32, _p, _p, _p]),
+    'wr_bpr_logsig_sum_fwd_bwd_sharded': (_int, [_p, _p, _p, _p, _p, _i64, _i64, _int, _f32, _p, _p, _p]),
+    'wr_infonce_sharded_scratch_bytes': (_sz, [_i64, _i64, _int]),
+    'wr_infonce_sharded_partials': (_int, [_p, _p, _int, _p, _i64, _int, _f32, _p, _p, _sz, _p, _p]),
+    'wr_infonce_sharded_weights': (_int, [_p, _int, _p, _i64, _int, _f32, _f32, _f32, _p, _p, _p, _p, _sz, _p]),
+    'wr_infonce_sharded_batch': (_int, [_p, _int, _p, _i64, _int, _f32, _f32, _f32, _p, _p, _sz, _p]),
     'wr_bpr_fwd_bwd_sharded_staged': (_int, [_p, _p, _p, _p, _i64, _p, _p, _p, _i64, _i64, _int, _f32, _f32, _p, _p, _p]),
     'wr_xchg_request': (_int, [_p, _p, _p, _i64, _i64, _i64, _int, _int, _p, _p, _i64, _p, _p, _p, _p]),
     'wr_xchg_serve': (_int, [_p, _int, _int, _int, _p, _p, _i64, _p, _p]),
@@ -831,6 +836,44 @@ def bpr_fwd_bwd_sharded(T, Gd, user, pos, neg, B_global, D, loss_out, ws, gamma=
     check(load().wr_bpr_fwd_bwd_sharded(ctypes.addressof(T), ctypes.addressof(Gd), ptr(user, I64), ptr(pos, I64),
                                         ptr(neg, I64), user.numel(), B_global, D, gamma, grad_scale,
                                         ptr(loss_out, F32), ws.ptr, stream_ptr()))
+
+
+def bpr_logsig_sum_fwd_bwd_sharded(T, Gd, user, pos, neg, B_global, D, loss_out, ws, grad_scale=1.0):
+    """SGL's sum-form BPR term on this rank's slice (loss_out[0] = the slice's sum)."""
+    check(load().wr_bpr_logsig_sum_fwd_bwd_sharded(ctypes.addressof(T), ctypes.addressof(Gd), ptr(user, I64),
+                                                   ptr(pos, I64), ptr(neg, I64), user.numel(), B_global, D, grad_scale,
+                                                   ptr(loss_out, F32), ws.ptr, stream_ptr()))
+
+
+def infonce_sharded_scratch(B, N_local, D, device, scratch=None):
+    """Scratch of one rank for the three wr_infonce_sharded_* phases of one block (reused when large enough)."""
+    nbytes = load().wr_infonce_sharded_scratch_bytes(B, N_local, D)
+    if nbytes == 0:
+        raise WhisprError('wr_infonce_sharded: B = %d, D = %d not supported' % (B, D))
+    if scratch is None or scratch.numel() < nbytes:
+        scratch = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    return scratch
+
+
+def infonce_sharded_partials(T1, T2, which, idx, D, tau, z_ptrs, scratch, ws):
+    za = _ptr_array(z_ptrs, T2.world)
+    check(load().wr_infonce_sharded_partials(ctypes.addressof(T1), ctypes.addressof(T2), which, ptr(idx, I64), idx.numel(),
+                                             D, tau, ctypes.addressof(za), scratch.data_ptr(), scratch.numel(), ws.ptr,
+                                             stream_ptr()))
+
+
+def infonce_sharded_weights(dT2, which, idx, D, tau, weight, grad_scale, z_ptrs, ga_ptrs, loss_out, scratch):
+    za, ga = _ptr_array(z_ptrs, dT2.world), _ptr_array(ga_ptrs, dT2.world)
+    check(load().wr_infonce_sharded_weights(ctypes.addressof(dT2), which, ptr(idx, I64), idx.numel(), D, tau, weight,
+                                            grad_scale, ctypes.addressof(za), ctypes.addressof(ga), ptr(loss_out, F32),
+                                            scratch.data_ptr(), scratch.numel(), stream_ptr()))
+
+
+def infonce_sharded_batch(dT1, which, idx, D, tau, weight, grad_scale, ga_ptrs, scratch):
+    ga = _ptr_array(ga_ptrs, dT1.world)
+    check(load().wr_infonce_sharded_batch(ctypes.addressof(dT1), which, ptr(idx, I64), idx.numel(), D, tau, weight,
+                                          grad_scale, ctypes.addressof(ga), scratch.data_ptr(), scratch.numel(),
+                                          stream_ptr()))
 
 
 def bpr_fwd_bwd_sharded_staged(T, Gd, inbox_row_ptrs, inbox_idx_ptrs, cap, user, pos, neg, B_global, D, loss_out, ws,

@@ -390,20 +390,23 @@ static InfoncePlan infonce_plan(int64_t B, int64_t N, int D) {
 }
 
 template <int DT>
-static int infonce_passes(const InfoncePlan &pl, const float *An, const float *Tn, int64_t B, int64_t N, int D,
-                          float inv_tau, float *part1, const int64_t *idx, float *iz, float *part, float *Ga, float *Gt,
-                          float *Gtp, cudaStream_t st) {
-    const size_t s1 = infonce_pass1_smem<DT>(), s2 = infonce_pass2_smem<DT>();
+static int infonce_pass1_launch(const InfoncePlan &pl, const float *An, const float *Tn, int64_t B, int64_t N, int D,
+                                float inv_tau, float *part1, cudaStream_t st) {
+    const size_t s1 = infonce_pass1_smem<DT>();
     cudaError_t e = cudaFuncSetAttribute(infonce_pass1_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s1);
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(infonce_pass2_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s2);
     if (e != cudaSuccess) return (int)e;
     infonce_pass1_kernel<DT><<<dim3((unsigned)pl.n_btiles, (unsigned)pl.n_ranges1), 256, s1, st>>>(
         An, Tn, B, N, D, inv_tau, (int)pl.tiles_per_range1, part1);
     WR_CHECK_LAUNCH();
-    infonce_rows_kernel<<<(int)std::min((int64_t)8 * kSMs, (B + 7) / 8), 256, 0, st>>>(part1, (int)pl.n_ranges1, B, N, An, Tn,
-                                                                                     idx, D, inv_tau, iz, part);
-    WR_CHECK_LAUNCH();
+    return WR_OK;
+}
+
+template <int DT>
+static int infonce_pass2_launch(const InfoncePlan &pl, const float *An, const float *Tn, const float *iz, int64_t B,
+                                int64_t N, int D, float inv_tau, float *Ga, float *Gt, float *Gtp, cudaStream_t st) {
+    const size_t s2 = infonce_pass2_smem<DT>();
+    cudaError_t e = cudaFuncSetAttribute(infonce_pass2_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s2);
+    if (e != cudaSuccess) return (int)e;
     infonce_pass2_kernel<DT><<<dim3((unsigned)pl.n_ttiles, (unsigned)pl.n_ranges2), 256, s2, st>>>(
         An, Tn, iz, B, N, D, inv_tau, (int)pl.tiles_per_range2, Ga, Gt, Gtp);
     WR_CHECK_LAUNCH();
@@ -413,6 +416,128 @@ static int infonce_passes(const InfoncePlan &pl, const float *An, const float *T
         WR_CHECK_LAUNCH();
     }
     return WR_OK;
+}
+
+static int infonce_pass1(const InfoncePlan &pl, const float *An, const float *Tn, int64_t B, int64_t N, int D,
+                         float inv_tau, float *part1, cudaStream_t st) {
+    switch (pl.DT) {
+        case 16: return infonce_pass1_launch<16>(pl, An, Tn, B, N, D, inv_tau, part1, st);
+        case 32: return infonce_pass1_launch<32>(pl, An, Tn, B, N, D, inv_tau, part1, st);
+        case 64: return infonce_pass1_launch<64>(pl, An, Tn, B, N, D, inv_tau, part1, st);
+        case 128: return infonce_pass1_launch<128>(pl, An, Tn, B, N, D, inv_tau, part1, st);
+        default: return infonce_pass1_launch<256>(pl, An, Tn, B, N, D, inv_tau, part1, st);
+    }
+}
+
+static int infonce_pass2(const InfoncePlan &pl, const float *An, const float *Tn, const float *iz, int64_t B, int64_t N,
+                         int D, float inv_tau, float *Ga, float *Gt, float *Gtp, cudaStream_t st) {
+    switch (pl.DT) {
+        case 16: return infonce_pass2_launch<16>(pl, An, Tn, iz, B, N, D, inv_tau, Ga, Gt, Gtp, st);
+        case 32: return infonce_pass2_launch<32>(pl, An, Tn, iz, B, N, D, inv_tau, Ga, Gt, Gtp, st);
+        case 64: return infonce_pass2_launch<64>(pl, An, Tn, iz, B, N, D, inv_tau, Ga, Gt, Gtp, st);
+        case 128: return infonce_pass2_launch<128>(pl, An, Tn, iz, B, N, D, inv_tau, Ga, Gt, Gtp, st);
+        default: return infonce_pass2_launch<256>(pl, An, Tn, iz, B, N, D, inv_tau, Ga, Gt, Gtp, st);
+    }
+}
+
+// ---- InfoNCE split by table shard (wr_infonce_sharded_*): every rank runs the global batch against its own rows ----
+struct PeerSlots {
+    float *p[WR_MAX_WORLD];    // p[g]: rank g's slot array as mapped here
+    int world;
+};
+
+// z_b of this rank's rows = sum_r part1[r][b] (r ascending), posted into slot [rank][b] of every rank's [world][B] array
+// (plain stores: the wr_peer_barrier that follows orders them before any reader)
+__global__ void __launch_bounds__(256) infonce_post_partials_kernel(const float *__restrict__ part1, int n_ranges, int64_t B,
+                                                                     PeerSlots z, int world, int rank) {
+    for (int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += (int64_t)gridDim.x * blockDim.x) {
+        float s = 0.f;
+        for (int r = 0; r < n_ranges; ++r) s += part1[r * B + b];
+        for (int g = 0; g < world; ++g) z.p[g][rank * B + b] = s;
+    }
+}
+
+// the positive pair's pull, applied by the owner of idx_b only: Gt[local(idx_b)] -= a_b (RED: duplicate ids)
+__global__ void __launch_bounds__(256) infonce_owner_pull_kernel(const float *__restrict__ An, const int64_t *idx, int64_t Bn,
+                                                                  int64_t n_rows, int D, int world, int rank, float *Gt) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t b = warp; b < Bn; b += nwarps) {
+        const int64_t t = idx[b];
+        if ((uint64_t)t >= (uint64_t)n_rows || t % world != rank) continue;
+        const int64_t l = t / world;
+        for (int d = lane; d < D; d += 32) atomicAdd(Gt + l * D + d, -An[b * D + d]);
+    }
+}
+
+// this rank's partial Ga_b, stored into slot [rank][b] of the owner of idx_b ([world][B][D] per rank)
+__global__ void __launch_bounds__(256) infonce_post_ga_kernel(const float *__restrict__ Ga, const int64_t *idx, int64_t Bn,
+                                                               int64_t n_rows, int D, PeerSlots ga, int rank) {
+    const int D4 = D >> 2;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < Bn * D4; e += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t b = e / D4;
+        const int v = (int)(e - b * D4);
+        const int64_t t = idx[b];
+        if ((uint64_t)t >= (uint64_t)n_rows) continue;
+        float *dst = ga.p[t % ga.world] + ((int64_t)rank * Bn + b) * D + 4 * v;
+        *reinterpret_cast<float4 *>(dst) = reinterpret_cast<const float4 *>(Ga + b * D)[v];
+    }
+}
+
+// owner side of the batch: Ga_b = sum over ranks r (ascending) of slot [r][b]; then infonce_batch_kernel's chain rule
+// through the normalisation of a_b into the local row of dT1 (RED: duplicate ids)
+__global__ void __launch_bounds__(256) infonce_owner_batch_kernel(const float *__restrict__ ga_local, int world, int rank,
+                                                                   const float *__restrict__ An, const float *__restrict__ inv1,
+                                                                   const float *__restrict__ Pn, const int64_t *idx,
+                                                                   int64_t Bn, int64_t n_rows, int D, float c, float *dT1) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t b = warp; b < Bn; b += nwarps) {
+        const int64_t t = idx[b];
+        if ((uint64_t)t >= (uint64_t)n_rows || t % world != rank) continue;
+        const int64_t l = t / world;
+        auto g_at = [&](int d) {
+            float s = 0.f;
+            for (int r = 0; r < world; ++r) s += ga_local[((int64_t)r * Bn + b) * D + d];
+            return s - Pn[b * D + d];
+        };
+        float dot = 0.f;
+        for (int d = lane; d < D; d += 32) dot = fmaf(g_at(d), An[b * D + d], dot);
+        dot = warp_sum(dot);
+        const float k = c * inv1[b];
+        for (int d = lane; d < D; d += 32) atomicAdd(dT1 + l * D + d, k * (g_at(d) - dot * An[b * D + d]));
+    }
+}
+
+__global__ void iota_kernel(int64_t *out, int64_t n) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = i;
+}
+
+// Scratch of one rank, carried from phase to phase: its table rows (Tn, Gt, inv2, Gtp) and the whole batch's rows.
+struct InfonceShardScratch {
+    InfoncePlan pl;
+    float *Tn, *Gt, *inv2, *An, *Pn, *Ga, *inv1, *iz, *part, *part1, *Gtp;
+    int64_t *iota;
+};
+
+static size_t infonce_shard_layout(int64_t B, int64_t N_local, int D, void *scratch, InfonceShardScratch *s) {
+    // an empty shard plans as one row (never launched), so the layout is defined for every rank
+    const int64_t N = std::max<int64_t>(N_local, 1);
+    InfonceShardScratch t;
+    t.pl = infonce_plan(B, N, D);
+    char *p = (char *)(((uintptr_t)scratch + 255) & ~(uintptr_t)255);
+    char *const p0 = p;
+    auto take = [&](size_t bytes) { char *q = p; p += sgl_align(bytes); return q; };
+    t.Tn = (float *)take((size_t)N * D * 4), t.Gt = (float *)take((size_t)N * D * 4), t.inv2 = (float *)take((size_t)N * 4);
+    t.An = (float *)take((size_t)B * D * 4), t.Pn = (float *)take((size_t)B * D * 4), t.Ga = (float *)take((size_t)B * D * 4);
+    t.inv1 = (float *)take((size_t)B * 4), t.iz = (float *)take((size_t)B * 4), t.part = (float *)take((size_t)B * 4);
+    t.iota = (int64_t *)take((size_t)B * 8);
+    t.part1 = (float *)take((size_t)t.pl.n_ranges1 * B * 4);
+    t.Gtp = (float *)take((size_t)(t.pl.n_ranges2 - 1) * N * D * 4);
+    if (s) *s = t;
+    return (size_t)(p - p0) + 256;
 }
 
 }  // namespace wr
@@ -452,14 +577,12 @@ extern "C" int wr_infonce_fwd_bwd(const float *T1, const float *T2, const int64_
     WR_CHECK_LAUNCH();
     cudaError_t e = cudaMemsetAsync(Ga, 0, (size_t)B * D * 4, st);
     if (e != cudaSuccess) return (int)e;
-    int rc;
-    switch (pl.DT) {
-        case 16: rc = infonce_passes<16>(pl, An, Tn, B, N, D, inv_tau, part1, idx, iz, part, Ga, Gt, Gtp, st); break;
-        case 32: rc = infonce_passes<32>(pl, An, Tn, B, N, D, inv_tau, part1, idx, iz, part, Ga, Gt, Gtp, st); break;
-        case 64: rc = infonce_passes<64>(pl, An, Tn, B, N, D, inv_tau, part1, idx, iz, part, Ga, Gt, Gtp, st); break;
-        case 128: rc = infonce_passes<128>(pl, An, Tn, B, N, D, inv_tau, part1, idx, iz, part, Ga, Gt, Gtp, st); break;
-        default: rc = infonce_passes<256>(pl, An, Tn, B, N, D, inv_tau, part1, idx, iz, part, Ga, Gt, Gtp, st); break;
-    }
+    int rc = infonce_pass1(pl, An, Tn, B, N, D, inv_tau, part1, st);
+    if (rc != WR_OK) return rc;
+    infonce_rows_kernel<<<(int)std::min((int64_t)8 * kSMs, (B + 7) / 8), 256, 0, st>>>(part1, (int)pl.n_ranges1, B, N, An, Tn,
+                                                                                     idx, D, inv_tau, iz, part);
+    WR_CHECK_LAUNCH();
+    rc = infonce_pass2(pl, An, Tn, iz, B, N, D, inv_tau, Ga, Gt, Gtp, st);
     if (rc != WR_OK) return rc;
     scaled_sum_kernel<<<1, 256, 0, st>>>(part, B, weight, loss_out);
     WR_CHECK_LAUNCH();
@@ -467,6 +590,141 @@ extern "C" int wr_infonce_fwd_bwd(const float *T1, const float *T2, const int64_
     infonce_batch_kernel<<<(int)min((int64_t)gw, (B + 7) / 8), 256, 0, st>>>(Ga, An, inv1, Tn, idx, B, N, D, c, dT1, Gt);
     WR_CHECK_LAUNCH();
     infonce_table_kernel<<<(int)min((int64_t)gw, (N + 7) / 8), 256, 0, st>>>(Gt, Tn, inv2, N, D, c, dT2);
+    WR_CHECK_LAUNCH();
+    return WR_OK;
+}
+
+// ---- InfoNCE split by table shard -------------------------------------------------------------------------------------
+// Block `which` (0: users, 1: items) of the pooled view tables; this rank's block rows are local rows off .. off + N_local
+// of its shard (global id = l * world + rank), the rest of the block's rows (padding) never enter z.
+struct InfonceShardArgs {
+    int64_t n_rows, N_local, off;
+};
+
+static int infonce_shard_args(const wr_shards *s, int which, int64_t B, int D, float tau, float *const host_slots[WR_MAX_WORLD],
+                              bool need16, InfonceShardArgs *a) {
+    const int rc = wr_check_shards(s);
+    if (rc) return rc;
+    if (which != 0 && which != 1) return WR_E_SIZE;
+    if (B <= 0 || !(tau > 0.f)) return WR_E_SIZE;
+    if (D <= 0 || (D & 3) || D > WR_INFONCE_DMAX) return WR_E_DIM;
+    for (int g = 0; g < s->world; ++g) {
+        if (!host_slots[g]) return WR_E_NULL;
+        if (need16 && !wr_aligned16(host_slots[g])) return WR_E_ALIGN;
+    }
+    a->n_rows = which == 0 ? s->n_users : s->n_items;
+    a->N_local = s->rank < a->n_rows ? (a->n_rows - s->rank + s->world - 1) / s->world : 0;
+    a->off = which == 0 ? 0 : s->rows_u_local;
+    return WR_OK;
+}
+
+static PeerSlots peer_slots(float *const host_slots[WR_MAX_WORLD], int world) {
+    PeerSlots p{};
+    for (int g = 0; g < world; ++g) p.p[g] = host_slots[g];
+    p.world = world;
+    return p;
+}
+
+extern "C" size_t wr_infonce_sharded_scratch_bytes(int64_t B, int64_t N_local, int D) {
+    if (B <= 0 || N_local < 0 || D <= 0 || (D & 3) || D > WR_INFONCE_DMAX) return 0;
+    return infonce_shard_layout(B, N_local, D, nullptr, nullptr);
+}
+
+extern "C" int wr_infonce_sharded_partials(const wr_shards *host_T1, const wr_shards *host_T2, int which, const int64_t *idx,
+                                           int64_t B, int D, float tau, float *const host_z[WR_MAX_WORLD], void *scratch,
+                                           size_t scratch_bytes, void *ws, void *stream) {
+    if (!host_T1 || !host_T2 || !idx || !host_z || !scratch || !ws) return WR_E_NULL;
+    InfonceShardArgs a;
+    int rc = wr_check_shards(host_T1);
+    if (rc) return rc;
+    rc = infonce_shard_args(host_T2, which, B, D, tau, host_z, false, &a);
+    if (rc) return rc;
+    if (host_T1->world != host_T2->world || host_T1->rank != host_T2->rank) return WR_E_SIZE;
+    if (scratch_bytes < wr_infonce_sharded_scratch_bytes(B, a.N_local, D)) return WR_E_SIZE;
+    InfonceShardScratch s;
+    infonce_shard_layout(B, a.N_local, D, scratch, &s);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int gw = 8 * kSMs;
+    const float inv_tau = 1.0f / tau;
+    iota_kernel<<<(int)min((int64_t)gw, (B + 255) / 256), 256, 0, st>>>(s.iota, B);
+    WR_CHECK_LAUNCH();
+    // the batch's rows of both views from their owners (Ga holds the raw rows until phase 2 clears it)
+    rc = wr_gather_rows_sharded(host_T1, which, idx, B, D, s.Ga, ws, stream);
+    if (rc) return rc;
+    rows_normalize_kernel<<<(int)min((int64_t)gw, (B + 7) / 8), 256, 0, st>>>(s.Ga, nullptr, B, B, D, s.An, s.inv1, (WrWorkspace *)ws);
+    WR_CHECK_LAUNCH();
+    rc = wr_gather_rows_sharded(host_T2, which, idx, B, D, s.Ga, ws, stream);
+    if (rc) return rc;
+    rows_normalize_kernel<<<(int)min((int64_t)gw, (B + 7) / 8), 256, 0, st>>>(s.Ga, nullptr, B, B, D, s.Pn, s.iz, (WrWorkspace *)ws);
+    WR_CHECK_LAUNCH();
+    if (a.N_local > 0) {
+        const float *T2l = host_T2->base[host_T2->rank] + a.off * D;
+        rows_normalize_kernel<<<(int)min((int64_t)gw, (a.N_local + 7) / 8), 256, 0, st>>>(T2l, nullptr, a.N_local, a.N_local, D,
+                                                                                         s.Tn, s.inv2, (WrWorkspace *)ws);
+        WR_CHECK_LAUNCH();
+        rc = infonce_pass1(s.pl, s.An, s.Tn, B, a.N_local, D, inv_tau, s.part1, st);
+        if (rc) return rc;
+    }
+    infonce_post_partials_kernel<<<(int)min((int64_t)gw, (B + 255) / 256), 256, 0, st>>>(
+        s.part1, a.N_local > 0 ? (int)s.pl.n_ranges1 : 0, B, peer_slots(host_z, host_T2->world), host_T2->world, host_T2->rank);
+    WR_CHECK_LAUNCH();
+    return WR_OK;
+}
+
+extern "C" int wr_infonce_sharded_weights(const wr_shards *host_dT2, int which, const int64_t *idx, int64_t B, int D,
+                                          float tau, float weight, float grad_scale, float *const host_z[WR_MAX_WORLD],
+                                          float *const host_ga[WR_MAX_WORLD], float *loss_out, void *scratch,
+                                          size_t scratch_bytes, void *stream) {
+    if (!host_dT2 || !idx || !host_z || !host_ga || !loss_out || !scratch) return WR_E_NULL;
+    InfonceShardArgs a;
+    int rc = infonce_shard_args(host_dT2, which, B, D, tau, host_z, false, &a);
+    if (rc) return rc;
+    rc = infonce_shard_args(host_dT2, which, B, D, tau, host_ga, true, &a);
+    if (rc) return rc;
+    if (scratch_bytes < wr_infonce_sharded_scratch_bytes(B, a.N_local, D)) return WR_E_SIZE;
+    InfonceShardScratch s;
+    infonce_shard_layout(B, a.N_local, D, scratch, &s);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int gw = 8 * kSMs, world = host_dT2->world, rank = host_dT2->rank;
+    const float inv_tau = 1.0f / tau;
+    // z_b from the world partials (the same bits on every rank), the loss rows against the gathered positives
+    infonce_rows_kernel<<<(int)std::min((int64_t)gw, (B + 7) / 8), 256, 0, st>>>(host_z[rank], world, B, B, s.An, s.Pn, s.iota,
+                                                                                D, inv_tau, s.iz, s.part);
+    WR_CHECK_LAUNCH();
+    scaled_sum_kernel<<<1, 256, 0, st>>>(s.part, B, weight, loss_out);
+    WR_CHECK_LAUNCH();
+    cudaError_t e = cudaMemsetAsync(s.Ga, 0, (size_t)B * D * 4, st);
+    if (e != cudaSuccess) return (int)e;
+    if (a.N_local > 0) {
+        rc = infonce_pass2(s.pl, s.An, s.Tn, s.iz, B, a.N_local, D, inv_tau, s.Ga, s.Gt, s.Gtp, st);
+        if (rc) return rc;
+        infonce_owner_pull_kernel<<<(int)min((int64_t)gw, (B + 7) / 8), 256, 0, st>>>(s.An, idx, B, a.n_rows, D, world, rank, s.Gt);
+        WR_CHECK_LAUNCH();
+        const float c = weight * inv_tau * grad_scale;
+        infonce_table_kernel<<<(int)min((int64_t)gw, (a.N_local + 7) / 8), 256, 0, st>>>(
+            s.Gt, s.Tn, s.inv2, a.N_local, D, c, host_dT2->base[rank] + a.off * D);
+        WR_CHECK_LAUNCH();
+    }
+    infonce_post_ga_kernel<<<(int)min((int64_t)gw, (B * (D / 4) + 255) / 256), 256, 0, st>>>(s.Ga, idx, B, a.n_rows, D,
+                                                                                           peer_slots(host_ga, world), rank);
+    WR_CHECK_LAUNCH();
+    return WR_OK;
+}
+
+extern "C" int wr_infonce_sharded_batch(const wr_shards *host_dT1, int which, const int64_t *idx, int64_t B, int D,
+                                        float tau, float weight, float grad_scale, float *const host_ga[WR_MAX_WORLD],
+                                        void *scratch, size_t scratch_bytes, void *stream) {
+    if (!host_dT1 || !idx || !host_ga || !scratch) return WR_E_NULL;
+    InfonceShardArgs a;
+    int rc = infonce_shard_args(host_dT1, which, B, D, tau, host_ga, true, &a);
+    if (rc) return rc;
+    if (scratch_bytes < wr_infonce_sharded_scratch_bytes(B, a.N_local, D)) return WR_E_SIZE;
+    InfonceShardScratch s;
+    infonce_shard_layout(B, a.N_local, D, scratch, &s);
+    const int world = host_dT1->world, rank = host_dT1->rank;
+    const float c = weight * (1.0f / tau) * grad_scale;
+    infonce_owner_batch_kernel<<<(int)min((int64_t)8 * kSMs, (B + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
+        host_ga[rank], world, rank, s.An, s.inv1, s.Pn, idx, B, a.n_rows, D, c, host_dT1->base[rank] + a.off * D);
     WR_CHECK_LAUNCH();
     return WR_OK;
 }

@@ -797,6 +797,22 @@ extern "C" int wr_bpr_fwd_bwd_sharded(const wr_shards *host_T, const wr_shards *
     return launch_bpr(p, D, (cudaStream_t)stream);
 }
 
+// SGL's sum-form BPR term on shards: wr_bpr_logsig_sum_fwd_bwd's parameters on wr_bpr_fwd_bwd_sharded's tables
+extern "C" int wr_bpr_logsig_sum_fwd_bwd_sharded(const wr_shards *host_T, const wr_shards *host_Gd, const int64_t *user,
+                                                 const int64_t *pos, const int64_t *neg, int64_t B, int64_t B_global, int D,
+                                                 float grad_scale, float *loss_out, void *ws, void *stream) {
+    if (!host_T || !host_Gd || !user || !pos || !neg || !loss_out || !ws) return WR_E_NULL;
+    int rc = wr_check_shards(host_T);
+    if (rc) return rc;
+    rc = wr_check_shards(host_Gd);
+    if (rc) return rc;
+    if (B <= 0 || B_global < B) return WR_E_SIZE;
+    if (D <= 0 || (D & 3)) return WR_E_DIM;
+    BprParamsT<ShardTabs> p{{*host_T, *host_Gd}, user, pos, neg, B, host_T->n_users, host_T->n_items,
+                            -1.0f /* logsigmoid form */, grad_scale, 1.0f, loss_out, 0, (WrWorkspace *)ws};
+    return launch_bpr(p, D, (cudaStream_t)stream);
+}
+
 extern "C" int wr_embloss_fwd_bwd(const float *U0, const float *I0, const int64_t *user, const int64_t *pos,
                                   const int64_t *neg, int64_t B, int D, int64_t n_users, int64_t n_items,
                                   float reg_weight, float *gU0, float *gI0, float *loss_out, void *ws,

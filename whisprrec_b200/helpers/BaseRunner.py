@@ -247,7 +247,8 @@ class BaseRunner(object):
                                           'that does not leave such a remainder' % (hi - lo, st.layout.world))
             a, b = st.layout.batch_slice(hi - lo)
             loss = model.sharded_train_step(batches[0, lo + a:lo + b], batches[1, lo + a:lo + b],
-                                            batches[2, lo + a:lo + b], hi - lo, self.learning_rate, self.l2)
+                                            batches[2, lo + a:lo + b], hi - lo, self.learning_rate, self.l2,
+                                            batch=batches[:, lo:hi])
             losses[s:s + 1].copy_(loss[:1])
         if model.optimizer is not None:
             model.optimizer.step_count = st.step_count

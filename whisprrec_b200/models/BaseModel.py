@@ -252,8 +252,10 @@ class GeneralModel(BaseModel):
     def _on_sharded(self):
         pass
 
-    def sharded_train_step(self, user, pos, neg, B_global, lr, l2):
-        """This rank's slice of one global batch; returns the batch loss (device view, same on every rank)."""
+    def sharded_train_step(self, user, pos, neg, B_global, lr, l2, batch=None):
+        """This rank's slice of one global batch; returns the batch loss (device view, same on every rank).  batch: the
+        whole global batch ([3, B_global] ids, the same on every rank), for models whose step needs more than the
+        slice (SGL); the others ignore it."""
         raise NotImplementedError
 
     def sharded_eval_tables(self):

@@ -115,7 +115,7 @@ class BPRMF(GeneralModel):
         """Loss of the k-th train_step_host call of this model (0-based), for calls made with wait=0."""
         return self._host_ctx.wait(k, wait)
 
-    def sharded_train_step(self, user, pos, neg, B_global, lr, l2):
+    def sharded_train_step(self, user, pos, neg, B_global, lr, l2, batch=None):
         from ... import sharded as S
         return S.bprmf_step(self.sharded, user, pos, neg, B_global, lr, l2)
 

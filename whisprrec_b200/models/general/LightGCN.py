@@ -209,7 +209,7 @@ class LightGCN(GeneralModel):
         rowptr, col, dinv = self._adj_host
         self.sharded_gcn = S.ShardedLightGCN(self.sharded, rowptr, col, dinv, self.gcn_layers, self.reg_weight)
 
-    def sharded_train_step(self, user, pos, neg, B_global, lr, l2):
+    def sharded_train_step(self, user, pos, neg, B_global, lr, l2, batch=None):
         return self.sharded_gcn.step(user, pos, neg, B_global, lr, l2)
 
     def sharded_eval_tables(self):

@@ -87,13 +87,17 @@ class SGL(GeneralModel):
         self.sub_graphs = None
 
     def graph_construction(self):
-        """SGL.py:67-79: the two augmented views of this epoch (edge dropout on Python's global random stream)."""
+        """SGL.py:67-79: the two augmented views of this epoch (edge dropout on Python's global random stream).  Sharded,
+        every rank draws the same two views (its Python stream is seeded as every other rank's) and keeps its rows."""
         t = self.fuse()
         g = self.train_graph
         views = []
         for _ in range(2):
             fwd, tr = graph_views.edge_dropout_view_device(g.rowptr, g.col, self.drop_ratio, t.ws)
-            views.append(_Graph(*fwd, D=t.D, transpose=tr))
+            views.append((fwd, tr) if self.sharded is not None else _Graph(*fwd, D=t.D, transpose=tr))
+        if self.sharded is not None:
+            self.sharded_sgl.set_views(views)
+            return
         self.sub_graphs = views
 
     # ---- propagation -----------------------------------------------------------------------------------------------
@@ -172,8 +176,26 @@ class SGL(GeneralModel):
                              torch.zeros(1, dtype=torch.int32, device=dev))
         return _lib.eval_rank_topk(ue, ie, user, pos, self._no_hist[0], self._no_hist[1], self.tables.ws, scores=True)[4]
 
-    def shard(self, peers):
-        raise NotImplementedError('SGL runs on one GPU')
+    def _on_sharded(self):
+        from ... import sharded as S
+        rowptr, col, dinv = self._adj_host
+        self.sharded_sgl = S.ShardedSGL(self.sharded, rowptr, col, dinv, self.gcn_layers, self.reg_weight, self.ssl_tau,
+                                        self.ssl_weight)
+
+    def sharded_train_step(self, user, pos, neg, B_global, lr, l2, batch=None):
+        """batch: the global batch ([3, B_global] user / positive / negative ids, the same on every rank) -- the sharded
+        InfoNCE runs every rank's table rows against all of it."""
+        if batch is None:
+            raise ValueError('the sharded SGL step needs the global batch (batch=[3, B_global] ids)')
+        g = self.sharded_sgl
+        if g.views is None:
+            self.graph_construction()
+        return g.step(user, pos, neg, B_global, lr, l2, batch[0], batch[1])
+
+    def sharded_eval_tables(self):
+        g, st = self.sharded_sgl, self.sharded
+        g.propagate()
+        return g.pool_T, st.item_rows(g.pool)
 
     class Dataset(GeneralModel.Dataset):
         def actions_before_epoch(self):

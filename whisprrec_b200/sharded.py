@@ -354,6 +354,48 @@ def bprmf_step(tabs, user, pos, neg, B_global, lr, l2):
     return loss
 
 
+def local_rows(lay, rowptr, col):
+    """This rank's rows of a GLOBAL node CSR (int64 rowptr / int32 col tensors, on any device), in local row order:
+    (rowptr_local [n_local + 1], col_local (global node ids), src: position of every local edge in `col`,
+    rows: local row of every local edge, nodes: global node of every local row, -1 on padding rows)."""
+    dev = rowptr.device
+    nodes = torch.from_numpy(lay.local_nodes()).to(dev)
+    safe = nodes.clamp(min=0)
+    deg = torch.where(nodes >= 0, rowptr[safe + 1] - rowptr[safe], torch.zeros_like(safe))
+    lptr = torch.zeros(lay.n_local + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(deg, 0, out=lptr[1:])
+    total = int(lptr[-1].item())
+    rows = torch.repeat_interleave(torch.arange(lay.n_local, device=dev), deg)
+    src = rowptr[safe][rows] + (torch.arange(total, device=dev) - lptr[:-1][rows])
+    return lptr, col[src], src, rows, nodes
+
+
+class LocalGraph(object):
+    """This rank's rows of a GLOBAL node CSR (every rank passes the same; NumPy arrays or device tensors), cut out on the
+    device by local_rows; column ids stay global node ids.  Weights: `val` (global, one per edge) sliced, or LightGCN's
+    fl32(fl32(dinv[row] * 1) * dinv[col]) from `dinv` (LightGCN.py:89-97)."""
+
+    def __init__(self, tabs, rowptr, col, dinv=None, val=None):
+        lay, dev = tabs.layout, tabs.peers.device
+        as_dev = lambda a, dt: (a if torch.is_tensor(a) else torch.from_numpy(np.ascontiguousarray(a))).to(dev).to(dt)
+        lptr, col_local, src, rows, nodes = local_rows(lay, as_dev(rowptr, torch.int64), as_dev(col, torch.int32))
+        safe = nodes.clamp(min=0)
+        total = int(lptr[-1].item())
+        self.rowptr = lptr
+        self.col = col_local.contiguous() if total else torch.zeros(1, dtype=torch.int32, device=dev)
+        if not total:
+            self.val = torch.zeros(1, dtype=torch.float32, device=dev)
+        elif val is not None:
+            self.val = as_dev(val, torch.float32)[src].contiguous()
+        else:
+            dinv_d = as_dev(dinv, torch.float32)
+            d_row = torch.where(nodes >= 0, dinv_d[safe], torch.zeros_like(dinv_d[safe]))
+            self.val = ((d_row[rows] * 1.0) * dinv_d[self.col[:total].long()]).contiguous()
+        del rows, src
+        self.plan = _lib.SpmmPlan(lptr.cpu().numpy(), tabs.D, dev)
+        self.nnz = total
+
+
 class ShardedLightGCN(object):
     """LightGCN propagation state of one rank: its rows of the adjacency and the symmetric layer / pool buffers."""
 
@@ -362,25 +404,10 @@ class ShardedLightGCN(object):
         passes the same).  The rank's rows are cut out on the device."""
         self.tabs, self.L, self.reg_weight = tabs, int(n_layers), float(reg_weight)
         lay, dev = tabs.layout, tabs.peers.device
-        as_dev = lambda a, dt: (a if torch.is_tensor(a) else torch.from_numpy(np.ascontiguousarray(a))).to(dev).to(dt)
-        rowptr_d, col_d, dinv_d = as_dev(rowptr, torch.int64), as_dev(col, torch.int32), as_dev(dinv, torch.float32)
-        nodes = torch.from_numpy(lay.local_nodes()).to(dev)                  # -1 on padding rows
-        safe = nodes.clamp(min=0)
-        deg = torch.where(nodes >= 0, rowptr_d[safe + 1] - rowptr_d[safe], torch.zeros_like(safe))
-        lptr = torch.zeros(lay.n_local + 1, dtype=torch.int64, device=dev)
-        torch.cumsum(deg, 0, out=lptr[1:])
-        total = int(lptr[-1].item())
-        rows = torch.repeat_interleave(torch.arange(lay.n_local, device=dev), deg)
-        src = rowptr_d[safe][rows] + (torch.arange(total, device=dev) - lptr[:-1][rows])
-        self.rowptr = lptr
-        self.col = col_d[src].contiguous() if total else torch.zeros(1, dtype=torch.int32, device=dev)
-        # weights: fl32(fl32(dinv[row] * 1) * dinv[col]) -- LightGCN.py:89-97
-        d_row = torch.where(nodes >= 0, dinv_d[safe], torch.zeros_like(dinv_d[safe]))
-        self.val = ((d_row[rows] * 1.0) * dinv_d[self.col[:total].long()]).contiguous() if total else \
-            torch.zeros(1, dtype=torch.float32, device=dev)
-        del rows, src
-        self.plan = _lib.SpmmPlan(lptr.cpu().numpy(), tabs.D, dev)
-        self.nnz = total
+        self.graph = LocalGraph(tabs, rowptr, col, dinv=dinv)
+        self.rowptr, self.col, self.val = self.graph.rowptr, self.graph.col, self.graph.val
+        self.plan, self.nnz = self.graph.plan, self.graph.nnz
+        total = self.nnz
         self.pool, self.pool_T = tabs.symmetric()
         self.pool_grad, self.pool_Gd = tabs.symmetric()
         self.layer = [tabs.symmetric(), tabs.symmetric()]
@@ -432,11 +459,12 @@ class ShardedLightGCN(object):
             self._local_views[key] = v
         return v
 
-    def _spmm(self, X, push=False, **kw):
-        """One propagation.  push=True: the output Y is the next SpMM's input -- its rows go into every peer's other
-        gathered copy while the kernel runs (copy engines; store-push epilogue where that is not available), and that
-        SpMM skips its all-gather."""
+    def _spmm(self, X, push=False, graph=None, **kw):
+        """One propagation over `graph` (a LocalGraph; default: this object's adjacency).  push=True: the output Y is the
+        next SpMM's input -- its rows go into every peer's other gathered copy while the kernel runs (copy engines;
+        store-push epilogue where that is not available), and that SpMM skips its all-gather."""
         t = self.tabs
+        g = self.graph if graph is None else graph
         lay = t.layout
         push_ptrs = None
         if self.gather_first:
@@ -460,35 +488,40 @@ class ShardedLightGCN(object):
                 self._cur = 1 - cur
         if push_ptrs is not None and self.dma and self.dma_spmm:
             self._epoch += 1
-            _lib.csr_spmm_sharded_dma(self.rowptr, self.col, self.val, lay.n_local, t.D, X, kw.pop('Y'), push_ptrs,
-                                      self._progress, self._block_rows, self._epoch, self._side, nnz=self.nnz,
-                                      plan=self.plan, **kw)
+            _lib.csr_spmm_sharded_dma(g.rowptr, g.col, g.val, lay.n_local, t.D, X, kw.pop('Y'), push_ptrs,
+                                      self._progress, self._block_rows, self._epoch, self._side, nnz=g.nnz,
+                                      plan=g.plan, **kw)
         else:
-            _lib.csr_spmm_sharded(self.rowptr, self.col, self.val, lay.n_local, t.D, X, plan=self.plan,
+            _lib.csr_spmm_sharded(g.rowptr, g.col, g.val, lay.n_local, t.D, X, plan=g.plan,
                                   push_ptrs=push_ptrs, **kw)
         t.peers.barrier()          # every rank's rows of the output exist (everywhere) before anyone reads them
 
     def _shard_tensor(self, X):
         """The local tensor behind a wr_shards struct of this object (P, the pooled gradient or a layer buffer)."""
         base = X.base[X.rank]
-        for cand in (self.tabs.P, self.pool_grad, self.pool, self.layer[0][0], self.layer[1][0], self.tabs.G):
+        for cand in self._shard_tensors():
             if cand.data_ptr() == base:
                 return cand
         raise _lib.WhisprError('unknown shard')
 
-    def propagate(self):
-        """LightGCN.py:134-148 on row shards: layer k+1 reads its neighbours' layer-k rows from their owners."""
+    def _shard_tensors(self):
+        return (self.tabs.P, self.pool_grad, self.pool, self.layer[0][0], self.layer[1][0], self.tabs.G)
+
+    def propagate(self, graph=None, pool=None):
+        """LightGCN.py:134-148 on row shards: layer k+1 reads its neighbours' layer-k rows from their owners.
+        graph / pool: a LocalGraph and the local pool tensor it fills (default: this object's adjacency and pool)."""
         t, L = self.tabs, self.L
+        pool = self.pool if pool is None else pool
         t.settle()
         if L == 0:
-            self.pool.copy_(t.P)
+            pool.copy_(t.P)
             t.peers.barrier()
             return
         x = t.T
         for k in range(1, L + 1):
             y, ys = self.layer[(k - 1) & 1]
-            self._spmm(x, push=k < L, Y=y if k < L else None, acc_in=t.P if k == 1 else self.pool, acc_out=self.pool,
-                       acc_div=float(L + 1) if k == L else 1.0)
+            self._spmm(x, push=k < L, graph=graph, Y=y if k < L else None, acc_in=t.P if k == 1 else pool,
+                       acc_out=pool, acc_div=float(L + 1) if k == L else 1.0)
             x = ys
 
     def step(self, user, pos, neg, B_global, lr, l2):
@@ -586,6 +619,123 @@ def _node_map(self):
 
 ShardedLightGCN._node_map = _node_map
 ShardedLightGCN._step_exchanged = _step_exchanged
+
+
+class ShardedSGL(ShardedLightGCN):
+    """SGL (models/general/SGL.py) on row shards: three pooled tables -- the main graph's and the two edge-dropout
+    views' -- propagated from the same ego table, their pooled gradients, and this rank's rows of the views and of their
+    transposes (set_views, every epoch).  The main graph, the layer buffers and the SpMM are ShardedLightGCN's.
+
+    InfoNCE is split by table shard (wr_infonce_sharded_*): every rank runs the global batch against its own rows of
+    the view tables, so it needs the global batch's user and positive ids.  One protocol at every batch size: the
+    peer-load form.  The row exchange that BPRMF / LightGCN switch to at >= 8,192 rows per rank is not implemented for
+    SGL."""
+
+    def __init__(self, tabs, rowptr, col, dinv, n_layers, reg_weight, ssl_tau, ssl_weight, gather_first=None):
+        super().__init__(tabs, rowptr, col, dinv, n_layers, reg_weight, gather_first=gather_first)
+        if self.L < 1:
+            raise NotImplementedError('SGL needs at least one propagation layer')
+        self.ssl_tau, self.ssl_weight = float(ssl_tau), float(ssl_weight)
+        self.view_pool = [tabs.symmetric(), tabs.symmetric()]       # (local tensor, wr_shards) of view 1 / view 2
+        self.view_grad = [tabs.symmetric(), tabs.symmetric()]
+        self.views = None               # [(LocalGraph of the view, LocalGraph of its transpose)] x 2
+        self._slots = None
+        self._scratch = [None, None]
+        tabs.peers.host_sync()
+
+    def _shard_tensors(self):
+        return super()._shard_tensors() + tuple(p for p, _ in self.view_pool + self.view_grad)
+
+    def set_views(self, views):
+        """views: the epoch's two views as edge_dropout_view_device returns them (GLOBAL device CSRs, the same on every
+        rank); keeps this rank's rows of each view and of its transpose."""
+        t = self.tabs
+        self.views = [(LocalGraph(t, *fwd[:2], val=fwd[2]), LocalGraph(t, *tr[:2], val=tr[2])) for fwd, tr in views]
+
+    def slots(self, B):
+        """Symmetric z / Ga slot arrays of the sharded InfoNCE for a global batch of up to B rows (collective)."""
+        lay = self.tabs.layout
+        if self._slots is None or self._slots['cap'] < B:
+            z, z_ptrs = self.tabs.peers.alloc((lay.world, B))
+            ga, ga_ptrs = self.tabs.peers.alloc((lay.world, B, self.tabs.D))
+            self._slots = {'cap': B, 'z': z, 'z_ptrs': z_ptrs, 'ga': ga, 'ga_ptrs': ga_ptrs}
+            self.tabs.peers.host_sync()
+        return self._slots
+
+    def _infonce(self, which, ids, scale):
+        """InfoNCE of one block (0: the batch's users, 1: its positive items): three phases, two barriers."""
+        t, lay = self.tabs, self.tabs.layout
+        B = ids.numel()
+        sl = self.slots(B)
+        n = lay.n_users if which == 0 else lay.n_items
+        n_local = (n - lay.rank + lay.world - 1) // lay.world          # rows u % world == rank of the block
+        sc = self._scratch[which] = _lib.infonce_sharded_scratch(B, n_local, t.D, t.peers.device, self._scratch[which])
+        (_, p1), (_, p2) = self.view_pool
+        (_, g1), (_, g2) = self.view_grad
+        _lib.infonce_sharded_partials(p1, p2, which, ids, t.D, self.ssl_tau, sl['z_ptrs'], sc, t.ws)
+        t.peers.barrier()               # every rank's partial z has landed
+        _lib.infonce_sharded_weights(g2, which, ids, t.D, self.ssl_tau, self.ssl_weight, scale, sl['z_ptrs'],
+                                     sl['ga_ptrs'], t.loss, sc)
+        t.peers.barrier()               # every rank's partial Ga has landed at the owners
+        _lib.infonce_sharded_batch(g1, which, ids, t.D, self.ssl_tau, self.ssl_weight, scale, sl['ga_ptrs'], sc)
+
+    def _adjoint(self, gt, grad, first):
+        """SGL._adjoint on shards: dE0 += H_0 with H_L = grad, H_{k-1} = grad + A^T H_k; gt: the transpose's LocalGraph,
+        grad: (local tensor, wr_shards) of a pooled gradient."""
+        t, L = self.tabs, self.L
+        g_local, h = grad
+        for k in range(1, L + 1):
+            last = k == L
+            kw = dict(graph=gt, add=g_local, zero_add=last and L > 1)
+            if not last:
+                y, ys = self.layer[(k - 1) & 1]
+                self._spmm(h, push=True, Y=y, **kw)
+                h = ys
+            elif first:
+                self._spmm(h, Y=t.G, **kw)                                  # tabs.G is zero: overwrite
+            else:
+                self._spmm(h, acc_in=t.G, acc_out=t.G, acc_div=1.0, **kw)
+        if L == 1:
+            g_local.zero_()
+
+    def step(self, user, pos, neg, B_global, lr, l2, batch_user, batch_pos, mark=None):
+        """SGL.py:233-246 + backward + Adam on this rank's slice (user, pos, neg) of a global batch whose user and
+        positive ids are batch_user / batch_pos (the same on every rank).  mark (optional): called with the name of
+        each phase as it is issued (scripts/bench_sgl_sharded.py records an event there)."""
+        t, L = self.tabs, self.L
+        mark = mark or (lambda name: None)
+        if self.views is None:
+            raise _lib.WhisprError('ShardedSGL.step before set_views')
+        pools = [(self.graph, (self.pool, self.pool_T))] + [(v[0], p) for v, p in zip(self.views, self.view_pool)]
+        for g, (p, _) in pools:
+            self.propagate(g, p)
+        mark('propagate_x3')
+        scale = 1.0 / (L + 1)
+        _lib.bpr_logsig_sum_fwd_bwd_sharded(self.pool_T, self.pool_Gd, user, pos, neg, B_global, t.D, t.loss_part, t.ws,
+                                            grad_scale=scale)
+        _lib.embloss_sumsq_sharded(t.T, user, pos, neg, t.D, t.loss_part[1:], t.ws)
+        sums = t.peers.barrier(t.loss_part)          # BPR sums and the three norms reduced
+        t.loss.copy_(sums[:1])
+        self.sumsq[:3].copy_(sums[1:4])
+        mark('bpr_embloss_norms')
+        self._infonce(0, batch_user, scale)          # adds the batch's InfoNCE loss to t.loss once, on every rank
+        mark('infonce_users')
+        self._infonce(1, batch_pos, scale)
+        t.peers.barrier()                            # every pooled gradient row has landed
+        mark('infonce_items')
+        graphs_t = [self.graph] + [v[1] for v in self.views]
+        grads = [(self.pool_grad, self.pool_Gd)] + self.view_grad
+        for n, (gt, grad) in enumerate(zip(graphs_t, grads)):
+            self._adjoint(gt, grad, first=n == 0)
+        mark('adjoint_x3')
+        _lib.embloss_scatter_sharded(t.T, t.Gd, user, pos, neg, B_global, t.D, self.reg_weight, self.sumsq, t.loss,
+                                     t.ws)
+        t.peers.barrier()                            # every gradient row has landed
+        mark('embloss_scatter')
+        t.adam(lr, l2)
+        t.peers.barrier()
+        mark('adam')
+        return t.loss
 
 
 def sharded_eval(tabs, shards, item_table_local, user, pos, hist_local, k=0, precision=0):
