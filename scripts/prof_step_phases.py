@@ -8,7 +8,8 @@ library (default: the in-tree build) it reports
   * the event-timed step beside the event floor (a 4-element Adam sweep timed the same way, after the same flush);
   * from the traced instantiation (wr_debug_step_trace: %globaltimer stamps of thread 0 of every CTA), per phase, the
     median over steps of the median over CTAs (`median_cta`) and the critical path (`critical`: the latest CTA at each
-    stamp, measured from the earliest entry).
+    stamp, measured from the earliest entry).  Stamp 1 (`ids_mv_prefetch`) is thread 0's first ids landed, with the
+    G / M / V prefetch that waits for them issued.
 Several --lib arguments compare builds in one process (each is loaded in a child process of its own).
 """
 import argparse
@@ -21,7 +22,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-STAMPS = ['entry', 'ids', 'rows', 'reds_issued', 'arrived', 'passed', 'adam_operands', 'exit']
+STAMPS = ['entry', 'ids_mv_prefetch', 'rows', 'reds_issued', 'arrived', 'passed', 'adam_operands', 'exit']
 PHASES = [('launch_to_ids', 0, 1), ('ids_to_rows', 1, 2), ('rows_to_reds', 2, 3), ('fence_and_arrive', 3, 4),
           ('barrier_wait', 4, 5), ('adam_operands', 5, 6), ('adam_to_exit', 6, 7)]
 

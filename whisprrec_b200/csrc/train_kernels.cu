@@ -410,10 +410,10 @@ __global__ void __launch_bounds__(256) scatter_add_rows_kernel(float *G, const i
 
 // ------------------------------------------------------------------------------------------------------
 // One launch for a whole BPRMF step (BaseRunner.py:196-199) when the tables are cache-sized and the step is
-// latency-bound rather than bandwidth-bound: every warp first issues its ids, then the CTA pulls its spans of
-// P / M / V / G towards L2 (they do not depend on the batch), the grid does the BPR forward+backward (ids -> rows ->
-// REDs into G) while those streams are in flight, meets at a grid barrier (cooperative launch: all CTAs are
-// resident), and finishes with the Adam+L2 update of its spans, which come back as L2 hits.
+// latency-bound rather than bandwidth-bound: every warp first issues its ids, then the CTA pulls its spans of P towards
+// L2 (they do not depend on the batch) and, once its ids have landed, those of G, M and V; the grid does the BPR
+// forward+backward (ids -> rows -> REDs into G) while those streams are in flight, meets at a grid barrier (cooperative
+// launch: all CTAs are resident), and finishes with the Adam+L2 update of its spans, which come back as L2 hits.
 // ------------------------------------------------------------------------------------------------------
 // Cross-GPU synchronisation state of the single-launch step on row-sharded tables (world > 1).
 struct StepSync {
@@ -425,9 +425,9 @@ struct StepSync {
 };
 
 // wr_debug_step_trace: [CTA][8] %globaltimer stamps of thread 0 of every CTA, written by the TRACE instantiation only
-// (the production instantiation never names it).  Slots: 0 entry, 1 ids landed, 2 rows landed, 3 REDs issued,
-// 4 arrived (fence + arrival done), 5 barrier passed, 6 Adam operands landed, 7 exit.  Slots 1 / 2 / 6 are thread 0's
-// last batch group and last Adam iteration.
+// (the production instantiation never names it).  Slots: 0 entry, 1 ids landed and the G / M / V prefetch issued
+// (thread 0's first batch group), 2 rows landed, 3 REDs issued, 4 arrived (fence + arrival done), 5 barrier passed,
+// 6 Adam operands landed, 7 exit.  Slots 2 / 6 are thread 0's last batch group and last Adam iteration.
 __device__ uint64_t *g_step_trace;
 
 __device__ __forceinline__ void wait_for(int64_t x) { asm volatile("" ::"l"(x)); }
@@ -441,6 +441,14 @@ __device__ __forceinline__ void step_stamp(int slot, T... deps) {
             (wait_for(deps), ...);
             g_step_trace[8 * blockIdx.x + slot] = global_timer_ns();
         }
+    }
+}
+
+// One bulk L2 prefetch per span of blockDim float4 of `arr` that this CTA's Adam phase updates.
+__device__ __forceinline__ void prefetch_spans(const float4 *arr, int64_t n4) {
+    for (int64_t c = (int64_t)blockIdx.x * blockDim.x; c < n4; c += (int64_t)gridDim.x * blockDim.x) {
+        const uint32_t bytes = (uint32_t)min((int64_t)blockDim.x, n4 - c) * 16u;
+        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(arr + c), "r"(bytes) : "memory");
     }
 }
 
@@ -490,14 +498,15 @@ __global__ void __launch_bounds__(1024, 1) bprmf_step_kernel(BprParamsT<TABS> p,
         i = p.pos[first + grp];
         j = p.neg[first + grp];
     }
-    // ---- phase 0: pull this CTA's spans of P / M / V / G towards L2 (one bulk prefetch per span) ----
-    if (threadIdx.x < 4) {      // G too: the gradient REDs then meet lines that are already on their way
-        const float4 *arr = threadIdx.x == 0 ? P : (threadIdx.x == 1 ? M : (threadIdx.x == 2 ? V : G));
-        for (int64_t c = (int64_t)blockIdx.x * blockDim.x; c < n4; c += stride) {
-            const uint32_t bytes = (uint32_t)min((int64_t)blockDim.x, n4 - c) * 16u;
-            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(arr + c), "r"(bytes) : "memory");
-        }
-    }
+    // ---- phase 0: pull this CTA's spans of the four arrays towards L2, in the order the step needs them.  P, the
+    //      gathers' source, goes now.  G (the REDs' target) and M / V (read only by Adam, after the barrier) go once this
+    //      thread's ids have landed -- the test of j is what waits for them (an out-of-range j is reported below): their
+    //      fills, each evicting a dirty line, then queue in DRAM behind the first ids and gathers instead of ahead of
+    //      them.  (G at entry with P measured slower on the bench: the REDs are issued later.) ----
+    if (threadIdx.x == 2) prefetch_spans(P, n4);
+    if ((threadIdx.x < 2 || threadIdx.x == 3) && (uint64_t)j < (uint64_t)p.n_items)
+        prefetch_spans(threadIdx.x == 0 ? M : (threadIdx.x == 1 ? V : G), n4);
+    step_stamp<TRACE>(1, j);
     if (sy.world > 1) {
         // remote rows may be gathered only once their owners have finished the previous step's Adam
         if (threadIdx.x < sy.world) {
@@ -526,7 +535,6 @@ __global__ void __launch_bounds__(1024, 1) bprmf_step_kernel(BprParamsT<TABS> p,
         }
         const bool ok = valid && (uint64_t)u < (uint64_t)p.n_users && (uint64_t)i < (uint64_t)p.n_items &&
                         (uint64_t)j < (uint64_t)p.n_items;
-        step_stamp<TRACE>(1, j);                   // (the last of the three id loads)
         if (valid && !ok && sub == 0) atomicOr(&p.ws->status, WR_STATUS_INDEX_OUT_OF_RANGE);
         float4 ue[VPL], pe[VPL], ne[VPL];
         if (ok) {     // P is rewritten by phase 2 (and by the peers' Adam phases): coherent loads, not ld.global.nc
