@@ -136,6 +136,13 @@ int wr_bprmf_step_marked(float *P, float *M, float *V, float *G, uint32_t *touch
  * evaluated in double on the host as torch does); NULL forces the per-step form.  Launches only; nothing is synchronised.
  */
 size_t wr_bprmf_epoch_scratch_bytes(int64_t N, int64_t batch);
+/* Which form trains BPRMF on a table of n_users + n_items rows of size D with batches of at most batch_cap rows:
+ * 2 = the owner-computes resident kernel (one grid barrier per step), 1 = the two-barrier resident kernel, 0 = one
+ * wr_bprmf_step launch per batch; a negative error otherwise (WR_E_SIZE / WR_E_DIM for bad arguments, -1000 - the CUDA
+ * error when the device cannot be queried).  host_fed = 0 answers for wr_bprmf_epoch (with its scratch given),
+ * host_fed != 0 for a step of batch_cap rows on a fresh wr_bprmf_ctx (which sizes the kernel for >= 2,048 rows, in
+ * steps of 1,024).  The same decision the calls make, WR_EPOCH_KERNEL and WR_CTX_KERNEL included. */
+int wr_bprmf_epoch_form(int64_t n_users, int64_t n_items, int D, int64_t batch_cap, int host_fed);
 /* Profiling aid: with a DEVICE buffer of 8 x uint64 per step set here (NULL switches it off), every later launch of the
  * resident kernel records %globaltimer stamps per step: [0] step start, [1] BPR phase done, [2] past grid barrier 1,
  * [3] Adam phase done, [4] past grid barrier 2 (CTA 0), [5] descriptor seen by the poller, [6] ids staged (CTA 0),
@@ -177,8 +184,9 @@ int wr_bprmf_step_host(const int64_t *host_ids, int64_t *dev_ids, float *host_lo
  * the step is complete; anything else is first copied into the context's own pinned ring (the collate copy).
  * The kernel writes M / V back and leaves when wr_bprmf_ctx_sync / wr_bprmf_ctx_destroy close it, or by itself after 5 ms
  * without a new batch (the next step relaunches it).  WHILE IT IS RESIDENT THE ADAM MOMENTS LIVE IN SHARED MEMORY: call
- * wr_bprmf_ctx_sync before anything else reads M / V or writes the tables.  Tables that do not qualify for the resident
- * kernel fall back to one launch per step (ids must then be mapped pinned memory: WR_E_ALIGN otherwise).
+ * wr_bprmf_ctx_sync before anything else reads M / V or writes the tables.  Tables and batches that do not qualify for
+ * the resident kernel (wr_bprmf_epoch_form with host_fed = 1 returns 0) run as one launch per step on `stream`; such a
+ * step takes the next step number like any other, so wr_bprmf_ctx_wait works after any mix of the two routes.
  */
 typedef struct wr_bprmf_ctx wr_bprmf_ctx;
 int wr_bprmf_ctx_create(float *P, float *M, float *V, float *G, int64_t n_users, int64_t n_items, int D, float gamma,

@@ -67,6 +67,9 @@ def test_argument_errors_need_no_gpu():
     assert lib.wr_bprmf_epoch(16, 16, 16, 16, None, 100, 10, 8, 4, 4, 1e-10, 1e-3, 0.0, 0.9, 0.999, 1e-8, 0, 16, None, 0, 16, None) == -1
     assert lib.wr_bprmf_epoch(16, 16, 16, 16, 16, 100, 0, 8, 4, 4, 1e-10, 1e-3, 0.0, 0.9, 0.999, 1e-8, 0, 16, None, 0, 16, None) == -2
     assert lib.wr_bprmf_epoch_scratch_bytes(100, 10) == 10 * 32 and lib.wr_bprmf_epoch_scratch_bytes(0, 10) == 0
+    assert lib.wr_bprmf_epoch_form(0, 900, 64, 2048, 0) == -2 and lib.wr_bprmf_epoch_form(700, 0, 64, 2048, 1) == -2
+    assert lib.wr_bprmf_epoch_form(700, 900, 64, 0, 0) == -2 and lib.wr_bprmf_epoch_form(700, 900, 64, -5, 1) == -2
+    assert lib.wr_bprmf_epoch_form(700, 900, 6, 2048, 0) == -3 and lib.wr_bprmf_epoch_form(700, 900, 0, 2048, 1) == -3
     assert lib.wr_csr_build(None, 16, 5, 3, 3, 16, 16, 16, 16, 1 << 30, 16, None) == -1
     assert lib.wr_csr_build(16, 16, 0, 3, 3, 16, 16, 16, 16, 1 << 30, 16, None) == -2
     assert lib.wr_csr_build(16, 16, 5, 3, 3, 16, 16, 16, 16, 8, 16, None) == -2          # scratch too small

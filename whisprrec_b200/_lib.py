@@ -34,6 +34,7 @@ SIGNATURES = {
     'wr_bprmf_step': (_int, [_p, _p, _p, _p, _p, _p, _p, _i64, _int, _i64, _i64, _f32, _f32, _f64, _f64, _f32, _f32,
                              _f32, _p, _p, _p, _p]),
     'wr_bprmf_epoch_scratch_bytes': (_sz, [_i64, _i64]),
+    'wr_bprmf_epoch_form': (_int, [_i64, _i64, _int, _i64, _int]),
     'wr_debug_epoch_trace': (_int, [_p, _p]),
     'wr_debug_step_trace': (_int, [_p]),
     'wr_bprmf_epoch': (_int, [_p, _p, _p, _p, _p, _i64, _i64, _int, _i64, _i64, _f32, _f64, _f32, _f64, _f64, _f32, _i64,
@@ -312,6 +313,18 @@ def bprmf_epoch(P, M, V, G, ids, batch, n_users, adam_t0, lr, l2, losses, ws, be
                              ptr(losses, F32), None if scratch is None else scratch.data_ptr(), nbytes, ws.ptr,
                              stream_ptr()))
     return (N + batch - 1) // batch
+
+
+EPOCH_PER_STEP, EPOCH_TWO_BARRIER, EPOCH_OWNER = 0, 1, 2      # wr_bprmf_epoch_form
+
+
+def bprmf_epoch_form(n_users, n_items, D, batch_cap, host_fed=False):
+    """The form that trains this table: EPOCH_OWNER / EPOCH_TWO_BARRIER (one resident launch) or EPOCH_PER_STEP.
+    host_fed: for a step of `batch_cap` rows through a fresh BprmfContext instead of bprmf_epoch."""
+    rc = load().wr_bprmf_epoch_form(n_users, n_items, D, batch_cap, int(host_fed))
+    if rc < 0:
+        check(rc)
+    return rc
 
 
 def bprmf_step_host(host_ids, dev_ids, host_loss, P, M, V, G, n_users, step, lr, l2, loss_out, ws, beta1=0.9,

@@ -994,8 +994,8 @@ static bool epoch_owner_enabled() {
 }
 
 // 0 = eligible (cfg filled), -1000 = not eligible (use the per-step path), anything else = error
-// WR_CTX_KERNEL=owner puts the host-fed context on the one-barrier kernel too (its streaming path is complete and passes the
-// same tests; see epoch_config for why it is not the default there)
+// WR_CTX_KERNEL=owner puts the host-fed context on the one-barrier kernel too (its streaming path is complete and tested,
+// tests/test_resident_epoch.py::test_host_fed_owner_every_dim; see epoch_config for why it is not the default there)
 static bool ctx_owner_ok() {
     static int v = -1;
     if (v < 0) {
@@ -1056,6 +1056,13 @@ static void epoch_fill(EpochParams &p, const EpochConfig &cfg, float *P, float *
     p.cta_trace = g_epoch_cta_trace;
 }
 
+// The host-fed context launches the resident kernel for the largest batch seen so far, at least 2,048 rows, in steps of
+// 1,024 (so a stream of ragged batches does not relaunch it); `cur` is the capacity it runs with now (0: none yet).
+static inline int64_t ctx_batch_cap(int64_t cur, int64_t B) {
+    if (B <= cur) return cur;
+    return B < 2048 ? 2048 : (B + 1023) & ~(int64_t)1023;
+}
+
 // torch/optim/adam.py evaluates these in Python floats (C doubles, libm pow): the same calls here
 static inline void adam_step_scalars(double lr, double beta1, double beta2, double t, float *step_size, float *bc2_sqrt) {
     *step_size = (float)(lr / (1.0 - pow(beta1, t)));
@@ -1070,6 +1077,18 @@ extern "C" int wr_debug_epoch_trace(uint64_t *dev_trace, uint64_t *dev_cta_trace
     g_epoch_trace = dev_trace;
     g_epoch_cta_trace = dev_cta_trace;
     return WR_OK;
+}
+
+extern "C" int wr_bprmf_epoch_form(int64_t n_users, int64_t n_items, int D, int64_t batch_cap, int host_fed) {
+    if (n_users <= 0 || n_items <= 0 || batch_cap <= 0) return WR_E_SIZE;
+    if (D <= 0 || (D & 3)) return WR_E_DIM;
+    EpochConfig cfg;
+    const int64_t bcap = host_fed ? ctx_batch_cap(0, batch_cap) : batch_cap;
+    const int rc = epoch_config((n_users + n_items) * D, D, bcap, &cfg, host_fed ? ctx_owner_ok() : true);
+    if (rc == -1000) return 0;
+    if (rc > 0) return -1000 - rc;      // a CUDA error (no device): kept apart from the forms
+    if (rc < 0) return rc;
+    return cfg.owner ? 2 : 1;
 }
 
 extern "C" size_t wr_bprmf_epoch_scratch_bytes(int64_t N, int64_t batch) {
@@ -1141,10 +1160,17 @@ struct HostRing {                      // one mapped pinned allocation
     StepDesc desc[CTX_RING];
     uint32_t lossq[2 * CTX_RING];      // {step + 1, loss bits} written by the kernel as one 8-byte store
     uint32_t done[CTX_RING];
-    float loss0;                       // per-step-launch fallback: the loss by copy
     uint32_t exit_word;
     uint32_t pad[15];
 };
+
+// A step of the context that ran as per-step launches (large tables / batches) signals like a resident step: after the
+// step on the same stream, one thread stores its loss word pair, then its completion word, into the mapped ring.
+__global__ void ctx_signal_kernel(const float *loss, uint32_t *lossq, uint32_t *done, uint32_t seq) {
+    asm volatile("st.relaxed.sys.global.v2.b32 [%0], {%1, %2};" ::"l"(lossq), "r"(seq), "r"(__float_as_uint(*loss)) : "memory");
+    __threadfence_system();
+    asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(done), "r"(seq) : "memory");
+}
 
 struct wr_bprmf_ctx {
     float *P, *M, *V, *G;
@@ -1163,9 +1189,10 @@ struct wr_bprmf_ctx {
     int64_t *dev_ids;                  // device [CTX_RING][3 * dev_cap]: where the helper warps put the ids they pull over PCIe
     int64_t dev_cap;
     int64_t bcap;                      // batch capacity the resident kernel is configured for
-    float *dev_loss;                   // large tables: per-step launches, loss by copy
-    uint32_t pushed;                   // steps handed over so far
-    uint32_t first_live;               // first step the resident kernel (or the next launch) is responsible for
+    float *dev_loss;                   // per-step launches: the step's loss before ctx_signal_kernel forwards it
+    uint32_t pushed;                   // steps handed over so far (on either route)
+    uint32_t first_live;               // first step the resident kernel (or the next launch) is responsible for; steps
+                                       // below it are complete or queued on `stream` as per-step launches
     bool resident;
     uint64_t idle_ns;
     const void *checked[4];
@@ -1282,7 +1309,13 @@ static int ctx_wait_word(wr_bprmf_ctx *c, const EpochConfig &cfg, volatile uint3
             if (rc) return rc;
             if (!c->resident) {
                 if (__atomic_load_n(word, __ATOMIC_ACQUIRE) == step + 1u) break;
-                if (step < c->first_live) return (int)cudaErrorUnknown;       // finished, yet never signalled
+                if (step < c->first_live) {
+                    // not the resident kernel's: a per-step launch, whose words the caller's stream writes
+                    const cudaError_t e = cudaStreamSynchronize(c->stream);
+                    if (e != cudaSuccess) return (int)e;
+                    if (__atomic_load_n(word, __ATOMIC_ACQUIRE) == step + 1u) break;
+                    return (int)cudaErrorUnknown;                              // finished, yet never signalled
+                }
                 rc = ctx_launch(c, cfg);
                 if (rc) return rc;
             } else if ((spins & 0xfffffu) == 0xfffffu) {
@@ -1345,11 +1378,35 @@ extern "C" int wr_bprmf_ctx_wait(wr_bprmf_ctx *c, int64_t step, int wait, float 
         return WR_E_SIZE;
     EpochConfig cfg;
     int rc = epoch_config((c->n_users + c->n_items) * c->D, c->D, c->bcap > 0 ? c->bcap : 1, &cfg, ctx_owner_ok());
-    if (rc) return rc == -1000 ? WR_E_SIZE : rc;
+    // -1000: the context never ran resident, so every step is below first_live and cfg is never launched
+    if (rc && rc != -1000) return rc;
     const uint32_t s = (uint32_t)step;
     rc = ctx_wait_word(c, cfg, wait == 2 ? &c->hr->lossq[2 * (s % CTX_RING)] : &c->hr->done[s % CTX_RING], s);
     if (rc) return rc;
     if (host_loss_out) memcpy(host_loss_out, (const void *)&c->hr->lossq[2 * (s % CTX_RING) + 1], sizeof(float));
+    return WR_OK;
+}
+
+// Pageable (or unmapped) ids go into slot s of the context's own pinned ring -- the host half of the H2D transfer; *ids
+// is what the kernels read.  The slot's previous tenant is complete (the caller has waited for it).
+static int ctx_stage_ids(wr_bprmf_ctx *c, const int64_t *host_ids, int64_t B, uint32_t s, const int64_t **ids) {
+    *ids = host_ids;
+    if (wr_aligned16(host_ids) && ctx_ids_are_mapped(c, host_ids)) return WR_OK;
+    if (B > c->stage_cap) {
+        int rc = wr_bprmf_ctx_sync(c);
+        if (rc) return rc;
+        const cudaError_t q = cudaStreamSynchronize(c->stream);     // per-step launches may still read the old ring
+        if (q != cudaSuccess) return (int)q;
+        if (c->stage_ids) cudaFreeHost(c->stage_ids);
+        c->stage_ids = nullptr;
+        c->stage_cap = ((B < 4096 ? 4096 : B) + 15) & ~(int64_t)15;
+        const cudaError_t e = cudaHostAlloc((void **)&c->stage_ids, (size_t)CTX_RING * 3 * c->stage_cap * sizeof(int64_t),
+                                            cudaHostAllocMapped | cudaHostAllocPortable);
+        if (e != cudaSuccess) { c->stage_cap = 0; return (int)e; }
+    }
+    int64_t *slot = c->stage_ids + (size_t)(s % CTX_RING) * 3 * c->stage_cap;
+    memcpy(slot, host_ids, (size_t)(3 * B) * sizeof(int64_t));
+    *ids = slot;
     return WR_OK;
 }
 
@@ -1362,41 +1419,33 @@ extern "C" int wr_bprmf_ctx_step(wr_bprmf_ctx *c, const int64_t *host_ids, int64
     const int64_t n_elems = (c->n_users + c->n_items) * c->D;
     const int D = c->D;
     EpochConfig cfg;
-    // the resident kernel stages whole batches in shared memory: it is launched for the largest batch seen so far (at least
-    // 2,048 rows, in steps of 1,024) and relaunched when a larger one arrives
-    int64_t bcap = c->bcap;
-    if (B > bcap) bcap = B < 2048 ? 2048 : (B + 1023) & ~(int64_t)1023;
+    // the resident kernel stages whole batches in shared memory: it is launched for the largest batch seen so far and
+    // relaunched when a larger one arrives
+    const int64_t bcap = ctx_batch_cap(c->bcap, B);
     int rc = epoch_config(n_elems, D, bcap, &cfg, ctx_owner_ok());
     if (rc == 0 && bcap != c->bcap) {
         rc = wr_bprmf_ctx_sync(c);        // (still configured for the old size: closes the running kernel, if any)
         if (rc) return rc;
         c->bcap = bcap;
     }
-    if (rc == -1000) {
-        // large tables / batches: per-step launches that read the ids straight from the mapped buffer; the loss comes back by copy
-        if (!ctx_ids_are_mapped(c, host_ids)) return WR_E_ALIGN;
+    if (rc != 0 && rc != -1000) return rc;
+    const bool per_step = rc == -1000;
+    if (per_step) {
+        // large tables / batches: per-step launches on the caller's stream.  The step still takes the next step number
+        // and ring slot, so wr_bprmf_ctx_wait finds it like any other step.
         rc = wr_bprmf_ctx_sync(c);
         if (rc) return rc;
-        rc = wr_bprmf_step_impl(c->P, c->M, c->V, c->G, host_ids, host_ids + B, host_ids + 2 * B, B, D, c->n_users,
-                                c->n_items, c->gamma, c->l2, c->beta1, c->beta2, c->eps, step_size, bc2_sqrt, nullptr,
-                                c->dev_loss, c->ws, c->stream);
+    } else {
+        rc = ctx_check_exit(c);
         if (rc) return rc;
-        cudaError_t e = cudaMemcpyAsync(&c->hr->loss0, c->dev_loss, sizeof(float), cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess && wait) e = cudaStreamSynchronize(c->stream);
-        if (e != cudaSuccess) return (int)e;
-        if (wait && host_loss_out) *host_loss_out = c->hr->loss0;
-        return WR_OK;
     }
-    if (rc) return rc;
-    rc = ctx_check_exit(c);
-    if (rc) return rc;
     const uint32_t s = c->pushed;
     if (s >= EP_COUNT_MASK - 1u) return WR_E_SIZE;
     if (s >= CTX_RING) {                 // the slot's previous tenant (step s - CTX_RING) must be complete
         rc = ctx_wait_word(c, cfg, &c->hr->done[s % CTX_RING], s - CTX_RING);
         if (rc) return rc;
     }
-    if (B > c->dev_cap) {                // (re)size the device-side id ring; the kernel must not be running on the old one
+    if (!per_step && B > c->dev_cap) {   // (re)size the device-side id ring; the kernel must not be running on the old one
         rc = wr_bprmf_ctx_sync(c);
         if (rc) return rc;
         if (c->dev_ids) cudaFree(c->dev_ids);
@@ -1406,21 +1455,27 @@ extern "C" int wr_bprmf_ctx_step(wr_bprmf_ctx *c, const int64_t *host_ids, int64
         if (e != cudaSuccess) { c->dev_cap = 0; return (int)e; }
     }
     const int64_t *ids = host_ids;
-    if (!wr_aligned16(host_ids) || !ctx_ids_are_mapped(c, host_ids)) {
-        // pageable (or unmapped) ids: collate into the context's own pinned ring -- the host half of the H2D transfer
-        if (B > c->stage_cap) {
-            rc = wr_bprmf_ctx_sync(c);
-            if (rc) return rc;
-            if (c->stage_ids) cudaFreeHost(c->stage_ids);
-            c->stage_ids = nullptr;
-            c->stage_cap = ((B < 4096 ? 4096 : B) + 15) & ~(int64_t)15;
-            const cudaError_t e = cudaHostAlloc((void **)&c->stage_ids, (size_t)CTX_RING * 3 * c->stage_cap * sizeof(int64_t),
-                                                cudaHostAllocMapped | cudaHostAllocPortable);
-            if (e != cudaSuccess) { c->stage_cap = 0; return (int)e; }
-        }
-        int64_t *slot = c->stage_ids + (size_t)(s % CTX_RING) * 3 * c->stage_cap;
-        memcpy(slot, host_ids, (size_t)(3 * B) * sizeof(int64_t));
-        ids = slot;
+    rc = ctx_stage_ids(c, host_ids, B, s, &ids);
+    if (rc) return rc;
+    if (per_step) {
+        // the kernels read the ids straight from mapped pinned memory; the loss and completion words reach the same
+        // slots the resident kernel writes
+        rc = wr_bprmf_step_impl(c->P, c->M, c->V, c->G, ids, ids + B, ids + 2 * B, B, D, c->n_users, c->n_items,
+                                c->gamma, c->l2, c->beta1, c->beta2, c->eps, step_size, bc2_sqrt, nullptr, c->dev_loss,
+                                c->ws, c->stream);
+        if (rc) return rc;
+        ctx_signal_kernel<<<1, 1, 0, c->stream>>>(c->dev_loss, &c->hr->lossq[2 * (s % CTX_RING)],
+                                                   &c->hr->done[s % CTX_RING], s + 1u);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return (int)e;
+        c->pushed = s + 1u;
+        c->first_live = s + 1u;
+        if (!wait) return WR_OK;
+        e = cudaStreamSynchronize(c->stream);
+        if (e != cudaSuccess) return (int)e;
+        if (__atomic_load_n(&c->hr->done[s % CTX_RING], __ATOMIC_ACQUIRE) != s + 1u) return (int)cudaErrorUnknown;
+        if (host_loss_out) memcpy(host_loss_out, (const void *)&c->hr->lossq[2 * (s % CTX_RING) + 1], sizeof(float));
+        return WR_OK;
     }
     StepDesc *d = &c->hr->desc[s % CTX_RING];
     d->ids = ids; d->stride = B; d->B = (int32_t)B; d->step_size = step_size; d->bc2_sqrt = bc2_sqrt;
